@@ -4,7 +4,7 @@ nprobe=32, 1024-query batches, k=10) on N B200s, with recall@10, the HBM rooflin
 posting-list scan kernel, an end-to-end number through the host-buffer C-ABI call and the CPU
 baseline (the oracle port of the Rust reference) timed on this box's host cores.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 N > 1 (torchrun, one rank per GPU): weak scaling — every GPU holds 1M rows / 1024 lists of an
 N-times larger index (list l on rank l % N), the batch is 1024*N queries, each rank scans the
@@ -261,6 +261,19 @@ def recall_of(found_ids, found_cnt, truth_ids, truth_cnt, k):
         f = set(found_ids[i, :found_cnt[i]].tolist())
         acc += len(t & f) / max(1, len(t))
     return acc / found_ids.shape[0]
+
+
+def dump_outputs(out_dir, ids, dist, cnt):
+    """--dump-outputs: the results of the last timed step as a caller of the search receives them (ids and
+    distances [nq x k], counts [nq]), one DIR/<name>.npy each, so that two builds can be compared output for
+    output.  Ids and counts are stored as float64 (every u32, the 0xFFFFFFFF of an empty slot included, is
+    exact), distances in their own float32.  At most 10 K queries x k = 10: well under 64 MB, no sampling."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"ids": ids.cpu().numpy().view(np.uint32).astype(np.float64),
+              "distances": dist.cpu().numpy().astype(np.float32),
+              "counts": cnt.cpu().numpy().view(np.uint32).astype(np.float64)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 # ---------------------------------------------------------------------------------------------
@@ -547,7 +560,15 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--mode", default=os.environ.get("FVDB_BENCH_MODE", "auto"), choices=["auto", "exact", "tc"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step (ids, distances, counts) to DIR/<name>.npy; "
+                         "the inputs are seeded, so runs with the same arguments compare output for output "
+                         "(cfg2 / cfg5)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.config in ("cfg3", "cfg4")):
+        ap.error("--dump-outputs covers the IVF search of cfg2 / cfg5 (--impl b200)")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", 0))
@@ -653,12 +674,12 @@ def main():
     ev0.record()
     for s in range(args.steps):
         if pipe > 1:
-            sh.submit(qsets[s % N_QUERY_SETS], K, NPROBE, tiers=L.TIER_HISTORICAL, slot=s % pipe)
+            last = sh.submit(qsets[s % N_QUERY_SETS], K, NPROBE, tiers=L.TIER_HISTORICAL, slot=s % pipe)
             if (s + 1) % pipe and s + 1 != args.steps:
                 continue
             sh.finish()
         else:
-            step(s)
+            last = step(s)
         st = eng.stats()
         scan_ms.append(st.last_scan_ms)
         n_in_group = ((s % pipe) + 1) if pipe > 1 else 1
@@ -671,6 +692,10 @@ def main():
         torch.cuda.profiler.stop()
     elapsed_ms = ev0.elapsed_time(ev1)
     clocks = sampler.stop()
+    # before the end-to-end leg, which reuses the pipeline slots' result buffers (N > 1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last)
+        log(f"wrote the last timed step's results to {args.dump_outputs}")
     if world > 1:
         t = torch.tensor([elapsed_ms], dtype=torch.float64, device="cuda")
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

@@ -1,11 +1,13 @@
 """CPU checks of bench.py's host-side logic (no GPU, no timing): the training-sample layout both arms share, the
-k-means seeding rule, the reference arm's host-built index on a tiny workload, and that the committed scan-traffic
-stamp belongs to the committed kernel sources (otherwise the bench line would carry no `roofline.traffic`)."""
+k-means seeding rule, the reference arm's host-built index on a tiny workload, the --dump-outputs writer and the
+argument checks, and that the committed scan-traffic stamp belongs to the committed kernel sources (otherwise the
+bench line would carry no `roofline.traffic`)."""
 import json
 import os
 import sys
 
 import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -51,6 +53,31 @@ def test_reference_arm_host_index_small(monkeypatch):
     ids, dist, cnt = O.hybrid_batch_search(ivf, None, None, q, 5, nlist, tiers=2)
     base = synth.query_base_rows(0, 8, n_total, bench.SEED_Q)
     assert (cnt == 5).all() and ids[:, 0].tolist() == base.tolist()
+
+
+def test_dump_outputs_writes_float_arrays(tmp_path):
+    """--dump-outputs: ids / distances / counts of a step as .npy in float64 / float32; the id of an empty slot
+    (0xFFFFFFFF) survives exactly."""
+    import torch
+    ids = torch.tensor([[3, 7], [999_999, -1]], dtype=torch.int32)
+    dist = torch.tensor([[0.5, 1.25], [0.75, float("inf")]], dtype=torch.float32)
+    cnt = torch.tensor([2, 1], dtype=torch.int32)
+    out = tmp_path / "out"
+    bench.dump_outputs(str(out), ids, dist, cnt)
+    assert sorted(os.listdir(out)) == ["counts.npy", "distances.npy", "ids.npy"]
+    got = {n: np.load(out / f"{n}.npy") for n in ("ids", "distances", "counts")}
+    assert got["ids"].dtype == np.float64 and got["ids"].tolist() == [[3, 7], [999_999, 0xFFFFFFFF]]
+    assert got["distances"].dtype == np.float32 and np.array_equal(got["distances"], dist.numpy())
+    assert got["counts"].dtype == np.float64 and got["counts"].tolist() == [2, 1]
+
+
+def test_bench_arguments_are_checked_before_any_work(monkeypatch):
+    for argv in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "x"],
+                 ["--config", "cfg3", "--dump-outputs", "x"]):
+        monkeypatch.setattr(sys, "argv", ["bench.py", *argv])
+        with pytest.raises(SystemExit) as e:
+            bench.main()
+        assert e.value.code == 2
 
 
 def test_committed_scan_traffic_stamp_matches_the_kernel_sources():
