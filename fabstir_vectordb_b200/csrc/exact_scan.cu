@@ -740,8 +740,9 @@ cudaError_t launch_finalize(const uint64_t* recent, const uint64_t* ivf, uint32_
 }
 
 // Cross-GPU merge after the all-gather (fvdb_merge_topk_device): parts x [nq][k] (ids, dist,
-// count) -> [nq][k].  Order: (distance, part, position) — each part is already sorted, lower
-// part first on ties.  One thread per query (k and parts are small).
+// count) -> [nq][k].  Order: (distance, row id), the ABI's tie rule — each part is already sorted
+// that way and the parts hold disjoint rows, so the head of every part is compared by distance and,
+// on equal distances, by id.  One thread per query (k and parts are small).
 // part p's block starts at p * stride_kv (ids, dist; elements) and p * stride_c (counts).
 __global__ void merge_parts_kernel(const uint32_t* __restrict__ ids, const float* __restrict__ dist,
                                    const uint32_t* __restrict__ cnt, uint32_t parts, uint32_t nq,
@@ -755,16 +756,19 @@ __global__ void merge_parts_kernel(const uint32_t* __restrict__ ids, const float
     uint32_t o = 0;
     for (; o < k; ++o) {
         float best = 0.f;
+        uint32_t best_id = 0;
         int bp = -1;
         for (uint32_t p = 0; p < parts; ++p) {
             const uint32_t c = min(cnt[(size_t)p * stride_c + q], k);
             if (pos[p] < c) {
-                const float d = dist[(size_t)p * stride_kv + (size_t)q * k + pos[p]];
-                if (bp < 0 || d < best) { best = d; bp = (int)p; }
+                const size_t at = (size_t)p * stride_kv + (size_t)q * k + pos[p];
+                const float d = dist[at];
+                const uint32_t id = ids[at];
+                if (bp < 0 || d < best || (d == best && id < best_id)) { best = d; best_id = id; bp = (int)p; }
             }
         }
         if (bp < 0) break;
-        out_ids[(size_t)q * k + o] = ids[(size_t)bp * stride_kv + (size_t)q * k + pos[bp]];
+        out_ids[(size_t)q * k + o] = best_id;
         out_dist[(size_t)q * k + o] = best;
         pos[bp]++;
     }

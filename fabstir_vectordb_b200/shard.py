@@ -2,7 +2,9 @@
 plumbing.  IVF list l lives on rank (l % world); centroids are replicated, so every rank runs
 the same coarse step, scans only the probed lists it owns (the others are empty in its arena)
 and emits a local top-k.  One exchange step: all-gather of the packed per-rank results (ids | dist | count), then
-the k-way merge of src/hybrid/core.rs:482-483 (`fvdb_merge_topk_device`).
+the k-way merge of src/hybrid/core.rs:482-483 (`fvdb_merge_topk_device`) in (distance, row id) order, the tie
+rule of the unsharded search.  The merge does not know the tier of a row, so sharded search serves one tier
+at a time (the IVF tier, or the recent tier in slabs), not FVDB_TIER_BOTH.
 
 The collective is torch.distributed (NCCL on GPUs; gloo in the CPU tests of the layout logic).
 """
@@ -66,8 +68,11 @@ def pack_layout(nq: int, k: int) -> Tuple[int, int, int, int]:
 
 
 def merge_parts_reference(ids: np.ndarray, dist: np.ndarray, cnt: np.ndarray, k: int):
-    """Host statement of the merge rule (distance, then part, then position) used by the CPU
-    gloo tests to validate the gather layout; the product path merges on the GPU."""
+    """Host statement of the merge rule of fvdb_merge_topk_device, used by the CPU gloo tests to validate
+    the gather layout; the product path merges on the GPU.  Order: (distance, row id), the ABI's tie rule,
+    so that the merged result equals the unsharded search whichever rank holds which of two rows at the
+    same distance.  The parts hold disjoint rows of one tier (an IVF-only sharded search, or recent-tier
+    slabs); the first min(count, k) entries of each part count."""
     parts, nq, _ = ids.shape
     out_ids = np.full((nq, k), 0xFFFFFFFF, dtype=np.uint32)
     out_dist = np.full((nq, k), np.inf, dtype=np.float32)
@@ -76,12 +81,12 @@ def merge_parts_reference(ids: np.ndarray, dist: np.ndarray, cnt: np.ndarray, k:
         cand = []
         for p in range(parts):
             for j in range(min(int(cnt[p, q]), k)):
-                cand.append((float(dist[p, q, j]), p, j, int(ids[p, q, j])))
-        cand.sort(key=lambda t: (t[0], t[1], t[2]))
+                cand.append((float(dist[p, q, j]), int(ids[p, q, j])))
+        cand.sort()
         cand = cand[:k]
         out_cnt[q] = len(cand)
         for o, c in enumerate(cand):
-            out_ids[q, o] = c[3]
+            out_ids[q, o] = c[1]
             out_dist[q, o] = c[0]
     return out_ids, out_dist, out_cnt
 

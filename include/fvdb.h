@@ -354,15 +354,20 @@ int fvdb_bounds_begin_batch(fvdb_index *h, uint32_t nq, void *stream);
 /* The same merge over ONE packed buffer per part — [ids nq*k | dist nq*k | count nq] 32-bit words,
  * parts back to back — so that the exchange step is a single all-gather: a rank lets
  * fvdb_search_device write its results into the three sections of its own chunk and gathers the
- * chunks.  Device pointers. */
+ * chunks.  Order and preconditions as for fvdb_merge_topk_device below.  Device pointers. */
 int fvdb_merge_topk_packed_device(fvdb_index *h, const uint32_t *d_pack, uint32_t parts, uint32_t nq,
                                   uint32_t k, uint32_t *d_out_ids, float *d_out_dist,
                                   uint32_t *d_out_count, void *stream);
 
 /* K-way merge of `parts` per-query partial results laid out [parts][nq][k] (ids, dist) with
  * counts [parts][nq] into [nq][k]: the `sort_by(distance); truncate(k)` of
- * src/hybrid/core.rs:482-483 applied across GPUs after the all-gather.  Ties: lower part first,
- * then lower id.  Device pointers. */
+ * src/hybrid/core.rs:482-483 applied across GPUs after the all-gather.  Order: (distance, row id),
+ * the ABI's tie rule, so the merged result equals one unsharded search however the rows are split.
+ * The parts must hold disjoint rows of ONE tier, each part sorted by (distance, row id) — as the
+ * list-sharded IVF search (FVDB_TIER_HISTORICAL) and a recent-tier scan split into slabs produce them.
+ * A FVDB_TIER_BOTH search orders recent-tier rows first on equal distances; a part does not carry
+ * the tier of its rows, so merging such parts is unsupported (ties would be ordered by id alone).
+ * Counts above k are clamped to k; parts must be in 1..64.  Device pointers. */
 int fvdb_merge_topk_device(fvdb_index *h, const uint32_t *d_ids, const float *d_dist,
                            const uint32_t *d_count, uint32_t parts, uint32_t nq, uint32_t k,
                            uint32_t *d_out_ids, float *d_out_dist, uint32_t *d_out_count,

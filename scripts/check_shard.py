@@ -117,6 +117,35 @@ print(f"rank {rank}/{world}: near-duplicate shell (proof fails somewhere): sync 
 ok = ok and bool(same3) and bool(same3p)
 eng.close()
 
+# ---- exact distance ties across ranks: binary rows (d 64) make every distance exact and give each query tie
+# groups of dozens of rows spread over the lists of all ranks; the merge must order them by row id, as the
+# unsharded search does, not by rank -------------------------------------------------------------------------------
+rng4 = np.random.default_rng(77)
+x4 = rng4.integers(0, 2, size=(20_000, 64)).astype(np.float32)
+q4 = rng4.integers(0, 2, size=(70, 64)).astype(np.float32)
+c4 = (0.5 + 0.3 * rng4.standard_normal((16, 64))).astype(np.float32)
+ivf4 = O.IVF(c4, x4, np.arange(x4.shape[0], dtype=np.uint32))
+w4 = O.hybrid_batch_search(ivf4, None, None, q4, K, 6, tiers=2)
+rank_of_row = (ivf4.assign % world).astype(np.int64)
+ties4 = sum(int(np.unique(rank_of_row[w4[0][i][w4[1][i] == v]]).size > 1)
+            for i in range(q4.shape[0]) for v in np.unique(w4[1][i]))
+same4 = ties4 > 0
+for mode in (L.SCAN_EXACT, L.SCAN_TC):
+    eng = Engine(64, k_max=16, device=local)
+    eng.set_option(L.OPT_SCAN_MODE, mode)
+    eng.set_centroids(c4)
+    sh = ShardedIndex(eng, rank, world)
+    sh.add_rows_device(torch.from_numpy(x4).to(dev), torch.arange(x4.shape[0], dtype=torch.int32, device=dev))
+    g4 = sh.search(torch.from_numpy(q4).to(dev), K, 6, tiers=L.TIER_HISTORICAL)
+    torch.cuda.synchronize()
+    same4 = same4 and (g4[0].cpu().numpy().view(np.uint32) == w4[0]).all() \
+        and (g4[1].cpu().numpy().view(np.uint32) == w4[1].view(np.uint32)).all() \
+        and (g4[2].cpu().numpy().view(np.uint32) == w4[2]).all()
+    eng.close()
+print(f"rank {rank}/{world}: lattice rows with {ties4} cross-rank tie groups in the top-{K}: exact and tc paths identical "
+      f"to the oracle: {bool(same4)}", flush=True)
+ok = ok and bool(same4)
+
 # ---- sharded k-means (points split over the ranks, one all-reduce per iteration) against the single-GPU
 # order-faithful training from the same initial centroids ------------------------------------------------
 eng = Engine(D, k_max=16, device=local)

@@ -34,12 +34,31 @@ def _case():
     return x, q, cents
 
 
-def _worker(rank, world, port, out_dir):
+def _lattice_case():
+    """Exact distance ties across ranks: integer rows, d 8, four lists on two ranks (l % 2).  Row 0 sits in
+    list 1 (rank 1), row 1 in list 0 (rank 0), both at distance 1.0 from q = 0: the unsharded search returns
+    row 0 first, a merge that breaks ties by rank returns row 1."""
+    d, nlist = 8, 4
+    cents = np.zeros((nlist, d), dtype=np.float32)
+    cents[np.arange(nlist), np.arange(nlist)] = 10
+    x = np.zeros((6, d), dtype=np.float32)
+    x[0, 1] = 1; x[1, 0] = 1; x[2, 2] = 3; x[3, 3] = 3; x[4, 0] = 5; x[5, 1] = 5
+    q = np.zeros((2, d), dtype=np.float32)
+    q[1, :2] = 0.5                    # rows 0 and 1 tie again, at sqrt(0.5)
+    return x, q, cents
+
+
+CASES = {"synth": (_case, K, NPROBE), "lattice": (_lattice_case, 4, 4)}
+
+
+def _worker(rank, world, port, out_dir, case="synth"):
     os.environ["MASTER_ADDR"] = "127.0.0.1"
     os.environ["MASTER_PORT"] = str(port)
     dist.init_process_group("gloo", rank=rank, world_size=world)
     try:
-        x, q, cents = _case()
+        make, K, NPROBE = CASES[case]
+        x, q, cents = make()
+        N, NQ = x.shape[0], q.shape[0]
         full = O.IVF(cents, x, np.arange(N, dtype=np.uint32))
         # this rank's shard: rows of the lists it owns, same centroids (replicated)
         mine = np.array([owner_of_list(int(l), world) == rank for l in full.assign])
@@ -64,19 +83,33 @@ def _worker(rank, world, port, out_dir):
         dist.destroy_process_group()
 
 
-def test_list_sharded_search_world2(tmp_path):
+def _check_sharded_search(tmp_path, case):
     world = 2
-    mp.spawn(_worker, args=(world, _free_port(), str(tmp_path)), nprocs=world, join=True)
-    x, q, cents = _case()
-    full = O.IVF(cents, x, np.arange(N, dtype=np.uint32))
+    mp.spawn(_worker, args=(world, _free_port(), str(tmp_path), case), nprocs=world, join=True)
+    make, K, NPROBE = CASES[case]
+    x, q, cents = make()
+    full = O.IVF(cents, x, np.arange(x.shape[0], dtype=np.uint32))
     w_ids, w_dst, w_cnt = O.hybrid_batch_search(full, None, None, q, K, NPROBE, tiers=2)
     for r in range(world):
         got = np.load(tmp_path / f"rank{r}.npz")
         assert got["cnt"].tolist() == w_cnt.tolist()
-        for i in range(NQ):
+        for i in range(q.shape[0]):
             c = int(w_cnt[i])
             assert got["ids"][i, :c].tolist() == w_ids[i, :c].tolist()
             assert got["dst"][i, :c].view(np.uint32).tolist() == w_dst[i, :c].view(np.uint32).tolist()
+    return full, w_ids
+
+
+def test_list_sharded_search_world2(tmp_path):
+    _check_sharded_search(tmp_path, "synth")
+
+
+def test_list_sharded_search_cross_rank_ties_world2(tmp_path):
+    """Two rows at exactly the same distance in lists of different ranks, the higher id on the lower rank:
+    the merge must order them by row id, as the unsharded search does, not by rank."""
+    full, w_ids = _check_sharded_search(tmp_path, "lattice")
+    assert full.assign[:2].tolist() == [1, 0]             # row 0 on rank 1, row 1 on rank 0
+    assert w_ids[0].tolist() == [0, 1, 2, 3] and w_ids[1, :2].tolist() == [0, 1]
 
 
 def test_owner_rule_partitions_lists():
