@@ -112,6 +112,12 @@ SIGNATURES = {
     "fvdb_search_device_coarse_submit": (C.c_int, [_vp, _vp, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, _vp,
                                                    C.c_uint64, _vp, _vp, _vp, _vp, _vp]),
     "fvdb_search_device_wait": (C.c_int, [_vp, C.c_uint32, _vp]),
+    "fvdb_search_device_tiers": (C.c_int, [_vp, _vp, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, _vp,
+                                           C.c_uint64, _vp, _vp, _vp]),
+    "fvdb_search_device_tiers_submit": (C.c_int, [_vp, _vp, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, _vp,
+                                                  C.c_uint64, _vp, _vp, _vp]),
+    "fvdb_merge_topk_tiers_packed_device": (C.c_int, [_vp, _vp, C.c_uint32, C.c_uint32, C.c_uint32, _vp, _vp, _vp,
+                                                      _vp]),
     "fvdb_merge_topk_device": (C.c_int, [_vp, _vp, _vp, _vp, C.c_uint32, C.c_uint32, C.c_uint32,
                                          _vp, _vp, _vp, _vp]),
     "fvdb_ivf_max_sqnorm": (C.c_int, [_vp, _f32p]),

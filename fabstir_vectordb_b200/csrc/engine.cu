@@ -225,6 +225,7 @@ struct fvdb_index {
         void *ho_ids, *ho_dist, *ho_cnt;   // fvdb_search_submit: the caller's page-locked result buffers (else NULL)
         int slot;             // pipeline slot the batch ran in (-1: the handle's own stream and scratch)
         cudaStream_t user_stream;
+        bool split;           // fvdb_search_device_tiers_submit: the outputs are a two-part packed chunk
     };
     // fvdb_search_submit: device-side query / result buffers of the batches in flight and the copy stream
     // their uploads run on (so that batch i + 1 uploads while batch i is scanned)
@@ -947,7 +948,8 @@ int search_device_impl(fvdb_index* h, const float* d_q, uint32_t nq, uint32_t k,
                        uint32_t tiers, const uint64_t* d_filter, uint64_t filter_bits,
                        uint32_t* d_out_ids, float* d_out_dist, uint32_t* d_out_count,
                        cudaStream_t st, const uint64_t* ext_coarse = nullptr, const HostOut* ho = nullptr,
-                       bool defer = false, bool want_pipe = false, cudaEvent_t wait_first = nullptr) {
+                       bool defer = false, bool want_pipe = false, cudaEvent_t wait_first = nullptr,
+                       bool split = false) {
     if (k == 0) return h->fail(FVDB_ERR_INVALID_ARG, "k must be >= 1");
     if (k > h->k_max) return h->fail(FVDB_ERR_K_TOO_LARGE, "k exceeds k_max given at fvdb_create");
     h->stats.last_nq = nq;
@@ -1019,6 +1021,12 @@ int search_device_impl(fvdb_index* h, const float* d_q, uint32_t nq, uint32_t k,
 
     uint64_t* ivf_keys = nullptr;
     uint64_t* flat_keys = nullptr;
+    // split (fvdb_search_device_tiers): the result arrays are the recent-tier part of a packed chunk
+    // [ids nq*k | dist nq*k | count nq]; the IVF tier's part follows it, one part length further on
+    const size_t part_words = (size_t)2 * nq * k + nq;
+    uint32_t* const ivf_out_ids = split ? d_out_ids + part_words : nullptr;
+    float* const ivf_out_dist = split ? d_out_dist + part_words : nullptr;
+    uint32_t* const ivf_out_count = split ? d_out_count + part_words : nullptr;
     bool scan_timed = false, used_tc = false, fused_finalize = false;
     uint32_t np = 0;
 
@@ -1059,7 +1067,7 @@ int search_device_impl(fvdb_index* h, const float* d_q, uint32_t nq, uint32_t k,
             ta.xmax_floor_sq = h->proof_xmax_sq;
             ta.scan_sms = sl ? h->scan_sms : 0;   // only pipelined batches have neighbours to leave room for
             ta.d_nan = d_nan;
-            if (!use_flat) {   // the only tier: the re-rank writes the result arrays itself
+            if (!use_flat && !split) {   // the only tier: the re-rank writes the result arrays itself
                 ta.fin_ids = d_out_ids; ta.fin_dist = d_out_dist; ta.fin_count = d_out_count;
                 fused_finalize = true;
             }
@@ -1117,7 +1125,8 @@ int search_device_impl(fvdb_index* h, const float* d_q, uint32_t nq, uint32_t k,
         }
     }
     if (!fused_finalize) {
-        CK(launch_finalize(flat_keys, ivf_keys, nq, k, d_out_ids, d_out_dist, d_out_count, st, h->metric));
+        CK(launch_finalize(flat_keys, ivf_keys, nq, k, d_out_ids, d_out_dist, d_out_count, st, h->metric,
+                           ivf_out_ids, ivf_out_dist, ivf_out_count));
         h->stats.last_launches += 1;
     }
     CK(cudaEventRecord(e_b, st));
@@ -1130,7 +1139,8 @@ int search_device_impl(fvdb_index* h, const float* d_q, uint32_t nq, uint32_t k,
         const size_t words = 16 + (size_t)4 * nq;
         fvdb_index::Pending pb{d_q, nq, k, nprobe, tiers, d_filter, filter_bits, d_out_ids, d_out_dist, d_out_count,
                                used_tc, flat_tc, use_ivf, use_flat, (tomb ? 1u : 0u) + (filt ? 1u : 0u), nullptr, 0,
-                               ho ? ho->ids : nullptr, ho ? ho->dist : nullptr, ho ? ho->cnt : nullptr, slot, user_st};
+                               ho ? ho->ids : nullptr, ho ? ho->dist : nullptr, ho ? ho->cnt : nullptr, slot, user_st,
+                               split};
         for (size_t i = 0; i < h->pending_pool.size(); ++i)
             if (h->pending_pool[i].second >= words) {
                 pb.host = h->pending_pool[i].first; pb.host_words = h->pending_pool[i].second;
@@ -1173,7 +1183,8 @@ int search_device_impl(fvdb_index* h, const float* d_q, uint32_t nq, uint32_t k,
         RET(scan_all_exact(h, h->flat_rows.p, h->flat_ids.p, h->flat_n, h->s_fb_q.p, n_fb_flat, k, tomb, h->tomb_bits,
                            filt, filter_bits, h->s_fb_keys.p, st, h->metric));
         CK(launch_scatter_keys(h->s_fb_keys.p, h->s_fb_idx_flat.p, n_fb_flat, k, flat_keys, st));
-        CK(launch_finalize(flat_keys, ivf_keys, nq, k, d_out_ids, d_out_dist, d_out_count, st, h->metric));
+        CK(launch_finalize(flat_keys, ivf_keys, nq, k, d_out_ids, d_out_dist, d_out_count, st, h->metric,
+                           ivf_out_ids, ivf_out_dist, ivf_out_count));
         if (ho) CK(copy_out(ho, d_out_ids, d_out_dist, d_out_count, st));
         CK(cudaStreamSynchronize(st));
         h->stats.last_launches += 3;
@@ -1192,7 +1203,8 @@ int search_device_impl(fvdb_index* h, const float* d_q, uint32_t nq, uint32_t k,
         RET(ivf_scan_exact(h, h->s_fb_q.p, n_fb, k, np, h->s_fb_coarse.p, tomb, filt, filter_bits,
                            h->s_fb_keys.p, nullptr, false, st));
         CK(launch_scatter_keys(h->s_fb_keys.p, h->s_fb_idx.p, n_fb, k, ivf_keys, st));
-        CK(launch_finalize(flat_keys, ivf_keys, nq, k, d_out_ids, d_out_dist, d_out_count, st, h->metric));
+        CK(launch_finalize(flat_keys, ivf_keys, nq, k, d_out_ids, d_out_dist, d_out_count, st, h->metric,
+                           ivf_out_ids, ivf_out_dist, ivf_out_count));
         if (ho) CK(copy_out(ho, d_out_ids, d_out_dist, d_out_count, st));
         CK(cudaStreamSynchronize(st));
         h->stats.last_launches += 3;
@@ -1847,12 +1859,20 @@ static int finish_pending(fvdb_index* h, cudaStream_t st) {
                 CK(cudaStreamSynchronize(st));   // idx (host vector) has been consumed
                 const uint32_t mode = h->scan_mode;
                 h->scan_mode = FVDB_SCAN_EXACT;
+                // (a split batch: t_ids / t_dist / t_cnt are the packed layout, its IVF part follows; the
+                // buffer holds 4 m k + 2 m words, two such parts)
                 const int r3 = search_device_impl(h, h->s_fb_q.p, m, pb.k, pb.nprobe, pb.tiers, pb.d_filter, pb.filter_bits,
-                                                  t_ids, t_dist, t_cnt, st);
+                                                  t_ids, t_dist, t_cnt, st, nullptr, nullptr, false, false, nullptr, pb.split);
                 h->scan_mode = mode;
                 if (r3 != FVDB_OK) return r3;
-                CK(launch_scatter_result_rows(t_ids, t_dist, t_cnt, reinterpret_cast<const uint32_t*>(h->s_fb_coarse.p), m,
-                                              pb.k, pb.d_out_ids, pb.d_out_dist, pb.d_out_count, st));
+                const uint32_t* fb_rows = reinterpret_cast<const uint32_t*>(h->s_fb_coarse.p);
+                CK(launch_scatter_result_rows(t_ids, t_dist, t_cnt, fb_rows, m, pb.k, pb.d_out_ids, pb.d_out_dist,
+                                              pb.d_out_count, st));
+                if (pb.split) {
+                    const size_t tp = (size_t)2 * m * pb.k + m, bp = (size_t)2 * pb.nq * pb.k + pb.nq;
+                    CK(launch_scatter_result_rows(t_ids + tp, t_dist + tp, t_cnt + tp, fb_rows, m, pb.k, pb.d_out_ids + bp,
+                                                  pb.d_out_dist + bp, pb.d_out_count + bp, st));
+                }
                 if (pb.ho_ids) {
                     const HostOut ho2{pb.ho_ids, pb.ho_dist, pb.ho_cnt, (size_t)pb.nq * pb.k * 4, (size_t)pb.nq * 4};
                     CK(copy_out(&ho2, pb.d_out_ids, pb.d_out_dist, pb.d_out_count, st));
@@ -1944,6 +1964,41 @@ int fvdb_search_device_coarse(fvdb_index* h, const float* d_q, uint32_t nq, uint
     cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
     return search_device_impl(h, d_q, nq, k, nprobe, tiers, d_filter_bits, filter_nbits, d_out_ids,
                               d_out_dist, d_out_count, st, d_coarse_keys);
+}
+
+// fvdb_search_device_coarse / _coarse_submit with the tiers kept apart: one flag through search_device_impl,
+// whose final merge then writes the recent tier to the first part of d_out_pack and the IVF tier to the second.
+static int search_device_tiers_common(fvdb_index* h, const float* d_q, uint32_t nq, uint32_t k, uint32_t nprobe,
+                                      uint32_t tiers, const uint64_t* d_filter_bits, uint64_t filter_nbits,
+                                      const uint64_t* d_coarse_keys, uint32_t* d_out_pack, void* stream, bool submit) {
+    if (h->metric != FVDB_METRIC_L2)
+        return h->fail(FVDB_ERR_INVALID_CONFIG, "fvdb_search_device_tiers serves L2 handles only");
+    if (!d_out_pack) return h->fail(FVDB_ERR_INVALID_ARG, "d_out_pack is NULL");
+    if (d_coarse_keys && nprobe > h->nlist)
+        return h->fail(FVDB_ERR_INVALID_ARG, "coarse keys are [nq x nprobe]: nprobe must not exceed nlist");
+    if (submit && h->pending.size() >= 64)
+        return h->fail(FVDB_ERR_INVALID_ARG, "64 batches are pending: call fvdb_search_device_finish");
+    cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
+    const size_t nk = (size_t)nq * k;
+    return search_device_impl(h, d_q, nq, k, nprobe, tiers, d_filter_bits, filter_nbits, d_out_pack,
+                              reinterpret_cast<float*>(d_out_pack + nk), d_out_pack + 2 * nk, st, d_coarse_keys,
+                              nullptr, submit, submit, nullptr, true);
+}
+
+int fvdb_search_device_tiers(fvdb_index* h, const float* d_q, uint32_t nq, uint32_t k, uint32_t nprobe,
+                             uint32_t tiers, const uint64_t* d_filter_bits, uint64_t filter_nbits,
+                             const uint64_t* d_coarse_keys, uint32_t* d_out_pack, void* stream) {
+    ENTER(h);
+    return search_device_tiers_common(h, d_q, nq, k, nprobe, tiers, d_filter_bits, filter_nbits, d_coarse_keys,
+                                      d_out_pack, stream, false);
+}
+
+int fvdb_search_device_tiers_submit(fvdb_index* h, const float* d_q, uint32_t nq, uint32_t k, uint32_t nprobe,
+                                    uint32_t tiers, const uint64_t* d_filter_bits, uint64_t filter_nbits,
+                                    const uint64_t* d_coarse_keys, uint32_t* d_out_pack, void* stream) {
+    ENTER_PIPE(h);
+    return search_device_tiers_common(h, d_q, nq, k, nprobe, tiers, d_filter_bits, filter_nbits, d_coarse_keys,
+                                      d_out_pack, stream, true);
 }
 
 namespace {
@@ -2263,6 +2318,21 @@ int fvdb_merge_topk_packed_device(fvdb_index* h, const uint32_t* d_pack, uint32_
     const size_t nk = (size_t)nq * k, chunk = 2 * nk + nq;
     CK(launch_merge_parts(d_pack, reinterpret_cast<const float*>(d_pack + nk), d_pack + 2 * nk, parts, nq, k,
                           d_out_ids, d_out_dist, d_out_count, st, chunk, chunk));
+    return FVDB_OK;
+}
+
+int fvdb_merge_topk_tiers_packed_device(fvdb_index* h, const uint32_t* d_pack, uint32_t ranks, uint32_t nq,
+                                        uint32_t k, uint32_t* d_out_ids, float* d_out_dist, uint32_t* d_out_count,
+                                        void* stream) {
+    ENTER_PIPE(h);   // touches nothing a batch in a pipeline slot reads: no drain
+    if (h->metric != FVDB_METRIC_L2)
+        return h->fail(FVDB_ERR_INVALID_CONFIG, "the tiered merge is ascending L2: L2 handles only");
+    if (ranks == 0 || ranks > 32) return h->fail(FVDB_ERR_INVALID_ARG, "ranks must be in 1..32");
+    cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
+    // a rank's chunk is two packed parts (recent, IVF) back to back: 2 * ranks parts of one part length each
+    const size_t nk = (size_t)nq * k, part = 2 * nk + nq;
+    CK(launch_merge_parts(d_pack, reinterpret_cast<const float*>(d_pack + nk), d_pack + 2 * nk, 2 * ranks, nq, k,
+                          d_out_ids, d_out_dist, d_out_count, st, part, part, true));
     return FVDB_OK;
 }
 

@@ -703,13 +703,9 @@ cudaError_t launch_merge_partials(const uint64_t* in, uint32_t nq, uint32_t P, u
 // Final hybrid merge (src/hybrid/core.rs:482-483): recent-tier keys and IVF keys, each sorted,
 // two-pointer merged by distance with the recent tier first on ties, truncated to k, split
 // into ids / distances / count.  Either input may be null.
-__global__ void finalize_kernel(const uint64_t* __restrict__ recent, const uint64_t* __restrict__ ivf,
-                                uint32_t nq, uint32_t k, uint32_t* __restrict__ out_ids,
-                                float* __restrict__ out_dist, uint32_t* __restrict__ out_count, int metric) {
-    const uint32_t q = blockIdx.x * blockDim.x + threadIdx.x;
-    if (q >= nq) return;
-    const uint64_t* a = recent ? recent + (size_t)q * k : nullptr;
-    const uint64_t* b = ivf ? ivf + (size_t)q * k : nullptr;
+__device__ __forceinline__ void finalize_row(const uint64_t* a, const uint64_t* b, uint32_t q, uint32_t k,
+                                             uint32_t* __restrict__ out_ids, float* __restrict__ out_dist,
+                                             uint32_t* __restrict__ out_count, int metric) {
     uint32_t ia = 0, ib = 0, o = 0;
     while (o < k) {
         const uint64_t ka = (a && ia < k) ? a[ia] : KEY_NONE;
@@ -730,20 +726,43 @@ __global__ void finalize_kernel(const uint64_t* __restrict__ recent, const uint6
     }
 }
 
+// Without a second output set the two tiers are merged into the first; with one (fvdb_search_device_tiers)
+// the recent tier goes to the first set and the IVF tier to the second, each as finalize writes a lone tier.
+__global__ void finalize_kernel(const uint64_t* __restrict__ recent, const uint64_t* __restrict__ ivf,
+                                uint32_t nq, uint32_t k, uint32_t* __restrict__ out_ids,
+                                float* __restrict__ out_dist, uint32_t* __restrict__ out_count, int metric,
+                                uint32_t* __restrict__ ivf_ids, float* __restrict__ ivf_dist,
+                                uint32_t* __restrict__ ivf_count) {
+    const uint32_t q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= nq) return;
+    const uint64_t* a = recent ? recent + (size_t)q * k : nullptr;
+    const uint64_t* b = ivf ? ivf + (size_t)q * k : nullptr;
+    if (ivf_ids) {
+        finalize_row(a, nullptr, q, k, out_ids, out_dist, out_count, metric);
+        finalize_row(nullptr, b, q, k, ivf_ids, ivf_dist, ivf_count, metric);
+    } else {
+        finalize_row(a, b, q, k, out_ids, out_dist, out_count, metric);
+    }
+}
+
 cudaError_t launch_finalize(const uint64_t* recent, const uint64_t* ivf, uint32_t nq, uint32_t k,
                             uint32_t* out_ids, float* out_dist, uint32_t* out_count,
-                            cudaStream_t stream, int metric) {
+                            cudaStream_t stream, int metric, uint32_t* ivf_ids, float* ivf_dist,
+                            uint32_t* ivf_count) {
     if (nq == 0) return cudaSuccess;
     finalize_kernel<<<(nq + 127) / 128, 128, 0, stream>>>(recent, ivf, nq, k, out_ids, out_dist,
-                                                         out_count, metric);
+                                                         out_count, metric, ivf_ids, ivf_dist, ivf_count);
     return cudaGetLastError();
 }
 
 // Cross-GPU merge after the all-gather (fvdb_merge_topk_device): parts x [nq][k] (ids, dist,
 // count) -> [nq][k].  Order: (distance, row id), the ABI's tie rule — each part is already sorted
 // that way and the parts hold disjoint rows, so the head of every part is compared by distance and,
-// on equal distances, by id.  One thread per query (k and parts are small).
+// on equal distances, by id.  TIERED (fvdb_merge_topk_tiers_packed_device): part p holds rows of tier
+// p & 1 (0 = recent, 1 = IVF) and the order is (distance, tier, row id), the recent-first rule of
+// finalize_kernel.  One thread per query (k and parts are small).
 // part p's block starts at p * stride_kv (ids, dist; elements) and p * stride_c (counts).
+template <bool TIERED>
 __global__ void merge_parts_kernel(const uint32_t* __restrict__ ids, const float* __restrict__ dist,
                                    const uint32_t* __restrict__ cnt, uint32_t parts, uint32_t nq,
                                    uint32_t k, size_t stride_kv, size_t stride_c, uint32_t* __restrict__ out_ids,
@@ -764,7 +783,12 @@ __global__ void merge_parts_kernel(const uint32_t* __restrict__ ids, const float
                 const size_t at = (size_t)p * stride_kv + (size_t)q * k + pos[p];
                 const float d = dist[at];
                 const uint32_t id = ids[at];
-                if (bp < 0 || d < best || (d == best && id < best_id)) { best = d; best_id = id; bp = (int)p; }
+                bool take = bp < 0 || d < best;
+                if (!take && d == best) {
+                    const uint32_t tp = TIERED ? (p & 1u) : 0u, tb = TIERED ? ((uint32_t)bp & 1u) : 0u;
+                    take = tp < tb || (tp == tb && id < best_id);
+                }
+                if (take) { best = d; best_id = id; bp = (int)p; }
             }
         }
         if (bp < 0) break;
@@ -782,13 +806,17 @@ __global__ void merge_parts_kernel(const uint32_t* __restrict__ ids, const float
 cudaError_t launch_merge_parts(const uint32_t* ids, const float* dist, const uint32_t* cnt,
                                uint32_t parts, uint32_t nq, uint32_t k, uint32_t* out_ids,
                                float* out_dist, uint32_t* out_count, cudaStream_t stream,
-                               size_t stride_kv, size_t stride_c) {
+                               size_t stride_kv, size_t stride_c, bool tiered) {
     if (nq == 0) return cudaSuccess;
     if (parts > 64) return cudaErrorInvalidValue;
     if (stride_kv == 0) stride_kv = (size_t)nq * k;
     if (stride_c == 0) stride_c = nq;
-    merge_parts_kernel<<<(nq + 127) / 128, 128, 0, stream>>>(ids, dist, cnt, parts, nq, k, stride_kv, stride_c,
-                                                            out_ids, out_dist, out_count);
+    if (tiered)
+        merge_parts_kernel<true><<<(nq + 127) / 128, 128, 0, stream>>>(ids, dist, cnt, parts, nq, k, stride_kv, stride_c,
+                                                                      out_ids, out_dist, out_count);
+    else
+        merge_parts_kernel<false><<<(nq + 127) / 128, 128, 0, stream>>>(ids, dist, cnt, parts, nq, k, stride_kv, stride_c,
+                                                                       out_ids, out_dist, out_count);
     return cudaGetLastError();
 }
 

@@ -56,13 +56,16 @@ cudaError_t launch_merge_partials(const uint64_t* in, uint32_t nq, uint32_t P, u
 // same for P rows of 32 keys each that may be unsorted or empty (tensor-core scan output)
 cudaError_t launch_merge_rows32(const uint64_t* in, uint32_t nq, uint32_t P, uint64_t* out,
                                 cudaStream_t stream, const uint32_t* row_stamp, uint32_t stamp);
+// ivf_ids / ivf_dist / ivf_count given: the tiers are not merged, the IVF tier goes to this second set
 cudaError_t launch_finalize(const uint64_t* recent, const uint64_t* ivf, uint32_t nq, uint32_t k,
                             uint32_t* out_ids, float* out_dist, uint32_t* out_count,
-                            cudaStream_t stream, int metric = 0);
+                            cudaStream_t stream, int metric = 0, uint32_t* ivf_ids = nullptr,
+                            float* ivf_dist = nullptr, uint32_t* ivf_count = nullptr);
+// tiered: part p holds rows of tier p & 1, order (distance, tier, row id)
 cudaError_t launch_merge_parts(const uint32_t* ids, const float* dist, const uint32_t* cnt,
                                uint32_t parts, uint32_t nq, uint32_t k, uint32_t* out_ids,
                                float* out_dist, uint32_t* out_count, cudaStream_t stream,
-                               size_t stride_kv = 0, size_t stride_c = 0);
+                               size_t stride_kv = 0, size_t stride_c = 0, bool tiered = false);
 // dst[idx[i]][0..k) = src[i][0..k)
 cudaError_t launch_scatter_result_rows(const uint32_t* ids, const float* dist, const uint32_t* cnt,
                                        const uint32_t* idx, uint32_t n, uint32_t k, uint32_t* out_ids,

@@ -363,6 +363,21 @@ class Engine:
     def search_device_wait(self, age: int = 0, stream: int = 0):
         self._ck(self._lib.fvdb_search_device_wait(self._h, age, _stream(stream)))
 
+    def search_device_tiers(self, d_q: int, nq: int, k: int, nprobe: int, tiers: int, d_filter: int,
+                            filter_nbits: int, d_coarse_keys: int, d_out_pack: int, stream: int = 0):
+        """search_device_coarse with the tiers kept apart: d_out_pack receives two packed parts, recent tier
+        then IVF tier (see shard.tiers_pack_layout)."""
+        self._ck(self._lib.fvdb_search_device_tiers(self._h, d_q, nq, k, nprobe, tiers, d_filter or None,
+                                                    filter_nbits, d_coarse_keys or None, d_out_pack,
+                                                    _stream(stream)))
+
+    def search_device_tiers_submit(self, d_q: int, nq: int, k: int, nprobe: int, tiers: int, d_filter: int,
+                                   filter_nbits: int, d_coarse_keys: int, d_out_pack: int, stream: int = 0):
+        """Stream-ordered search_device_tiers; the chunk is valid after search_device_finish."""
+        self._ck(self._lib.fvdb_search_device_tiers_submit(self._h, d_q, nq, k, nprobe, tiers, d_filter or None,
+                                                           filter_nbits, d_coarse_keys or None, d_out_pack,
+                                                           _stream(stream)))
+
     def merge_topk_device(self, d_ids: int, d_dist: int, d_count: int, parts: int, nq: int, k: int,
                           d_out_ids: int, d_out_dist: int, d_out_count: int, stream: int = 0):
         self._ck(self._lib.fvdb_merge_topk_device(self._h, d_ids, d_dist, d_count, parts, nq, k,
@@ -393,6 +408,12 @@ class Engine:
         """parts x [ids nq*k | dist nq*k | count nq] 32-bit words (see shard.pack_layout)."""
         self._ck(self._lib.fvdb_merge_topk_packed_device(self._h, d_pack, parts, nq, k, d_out_ids, d_out_dist,
                                                          d_out_count, _stream(stream)))
+
+    def merge_topk_tiers_packed_device(self, d_pack: int, ranks: int, nq: int, k: int, d_out_ids: int,
+                                       d_out_dist: int, d_out_count: int, stream: int = 0):
+        """ranks x search_device_tiers chunks -> the (distance, tier, row id) merge of both tiers."""
+        self._ck(self._lib.fvdb_merge_topk_tiers_packed_device(self._h, d_pack, ranks, nq, k, d_out_ids, d_out_dist,
+                                                               d_out_count, _stream(stream)))
 
     def ivf_add_device(self, d_x: int, d_ids: int, n: int, mod: int = 1, rem: int = 0) -> int:
         kept = C.c_uint64()

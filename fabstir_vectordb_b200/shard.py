@@ -1,10 +1,20 @@
-"""Multi-GPU list-sharded search (SURVEY §8e): one process per GPU, torch.distributed for the
-plumbing.  IVF list l lives on rank (l % world); centroids are replicated, so every rank runs
-the same coarse step, scans only the probed lists it owns (the others are empty in its arena)
-and emits a local top-k.  One exchange step: all-gather of the packed per-rank results (ids | dist | count), then
-the k-way merge of src/hybrid/core.rs:482-483 (`fvdb_merge_topk_device`) in (distance, row id) order, the tie
-rule of the unsharded search.  The merge does not know the tier of a row, so sharded search serves one tier
-at a time (the IVF tier, or the recent tier in slabs), not FVDB_TIER_BOTH.
+"""Multi-GPU sharded hybrid index (SURVEY §8e): one process per GPU, torch.distributed for the
+plumbing.  IVF list l lives on rank (l % world, or a place_lists table); centroids are replicated, so
+every rank runs the same coarse step, scans only the probed lists it owns (the others are empty in its
+arena) and emits a local top-k.  Recent-tier ("HNSW") rows live in slabs: row id r on rank r % world
+(owner_of_recent_row), scanned exhaustively by the rank that holds them.
+
+One exchange step: all-gather of the packed per-rank results, then the k-way merge of
+src/hybrid/core.rs:482-483.  A one-tier search (FVDB_TIER_HISTORICAL, or FVDB_TIER_RECENT) gathers one part
+per rank (ids | dist | count) and merges in (distance, row id) order (`fvdb_merge_topk_packed_device`).  A
+FVDB_TIER_BOTH search keeps the tiers apart on every rank (`fvdb_search_device_tiers`: a recent part and an
+IVF part per chunk) and merges the 2 * world parts in (distance, tier with recent first, row id) order
+(`fvdb_merge_topk_tiers_packed_device`): exactly one unsharded FVDB_TIER_BOTH search, however the rows of
+both tiers are split over the ranks.
+
+Mutations (delete, vacuum, migrate) are broadcast: every rank applies them to the rows it holds.  The
+tombstone and filter bitmaps are indexed by global row id, so a rank accepts ids it does not hold.  A
+migrated row joins its nearest list in the arena of the rank that held it, whichever rank owns that list.
 
 The collective is torch.distributed (NCCL on GPUs; gloo in the CPU tests of the layout logic).
 """
@@ -22,6 +32,12 @@ from .engine import Engine, NanInput
 def owner_of_list(list_id: int, world: int) -> int:
     """List -> rank placement rule; must match fvdb_ivf_add_device(list_filter_mod=world)."""
     return list_id % world
+
+
+def owner_of_recent_row(row_id: int, world: int) -> int:
+    """Recent-tier row -> rank placement rule (slabs by id): a pure function of the id, so every rank agrees
+    which rank holds a row without any table."""
+    return row_id % world
 
 
 def place_lists(sizes, world: int) -> np.ndarray:
@@ -67,12 +83,33 @@ def pack_layout(nq: int, k: int) -> Tuple[int, int, int, int]:
     return 0, nk, 2 * nk, 2 * nk + nq
 
 
+def tiers_pack_layout(nq: int, k: int) -> Tuple[int, int, int, int, int]:
+    """One rank's chunk of a FVDB_TIER_BOTH exchange (fvdb_search_device_tiers), in 32-bit words: two
+    pack_layout parts back to back, the recent tier then the IVF tier.  Returns (offset of ids, of dist, of
+    count inside a part, part length, chunk length); part t starts at t * part length.  Must match
+    fvdb_merge_topk_tiers_packed_device."""
+    o_ids, o_dist, o_cnt, part = pack_layout(nq, k)
+    return o_ids, o_dist, o_cnt, part, 2 * part
+
+
 def merge_parts_reference(ids: np.ndarray, dist: np.ndarray, cnt: np.ndarray, k: int):
     """Host statement of the merge rule of fvdb_merge_topk_device, used by the CPU gloo tests to validate
     the gather layout; the product path merges on the GPU.  Order: (distance, row id), the ABI's tie rule,
     so that the merged result equals the unsharded search whichever rank holds which of two rows at the
     same distance.  The parts hold disjoint rows of one tier (an IVF-only sharded search, or recent-tier
     slabs); the first min(count, k) entries of each part count."""
+    return _merge_reference(ids, dist, cnt, k, tiered=False)
+
+
+def merge_tiers_reference(ids: np.ndarray, dist: np.ndarray, cnt: np.ndarray, k: int):
+    """Host statement of fvdb_merge_topk_tiers_packed_device: ids / dist [2 * ranks][nq][k], cnt
+    [2 * ranks][nq], part 2r = recent tier of rank r, part 2r + 1 = IVF tier of rank r.  Order: (distance,
+    tier with recent first, row id), the order of one unsharded FVDB_TIER_BOTH search (the stable sort of
+    src/hybrid/core.rs:482-483 over recent-then-IVF results, each tier in (distance, row id) order)."""
+    return _merge_reference(ids, dist, cnt, k, tiered=True)
+
+
+def _merge_reference(ids, dist, cnt, k, tiered):
     parts, nq, _ = ids.shape
     out_ids = np.full((nq, k), 0xFFFFFFFF, dtype=np.uint32)
     out_dist = np.full((nq, k), np.inf, dtype=np.float32)
@@ -81,12 +118,12 @@ def merge_parts_reference(ids: np.ndarray, dist: np.ndarray, cnt: np.ndarray, k:
         cand = []
         for p in range(parts):
             for j in range(min(int(cnt[p, q]), k)):
-                cand.append((float(dist[p, q, j]), int(ids[p, q, j])))
+                cand.append((float(dist[p, q, j]), p & 1 if tiered else 0, int(ids[p, q, j])))
         cand.sort()
         cand = cand[:k]
         out_cnt[q] = len(cand)
         for o, c in enumerate(cand):
-            out_ids[q, o] = c[1]
+            out_ids[q, o] = c[2]
             out_dist[q, o] = c[0]
     return out_ids, out_dist, out_cnt
 
@@ -118,6 +155,9 @@ class ShardedIndex:
         self._group = []           # ... and every batch submitted since the last finish()
         self._nlist = None
         self._deferred_error = None
+        # an IVF-tier mutation can raise a rank's largest row norm: FVDB_OPT_PROOF_XMAX is max-reduced again
+        # before the next search (every rank mutates in the same order, so every rank sees the same flag)
+        self._xmax_dirty = False
         # the coarse step of a pipelined batch: stream-ordered until a proof failure shows up there (dense
         # centroid tables, e.g. nlist 16384), then the synchronous, self-repairing entry (see submit / finish)
         self.coarse_async = os.environ.get("FVDB_SHARD_COARSE_ASYNC", "1") == "1"
@@ -129,16 +169,35 @@ class ShardedIndex:
         # no rank may free its exported array while a peer still has it mapped
         self.eng.bounds_close_peers()
         dist.barrier(group=self.group)
-        # rows of this shard can be dropped by a bound a peer published: the tensor-core proof of every
-        # shard uses the largest row norm of ALL shards (FVDB_OPT_PROOF_XMAX)
-        xm = torch.tensor([self.eng.ivf_max_sqnorm()], dtype=torch.float32, device=device)
-        dist.all_reduce(xm, op=dist.ReduceOp.MAX, group=self.group)
-        self.eng.set_option(L.OPT_PROOF_XMAX, int(np.float32(xm.item()).view(np.uint32)))
+        self._reduce_xmax(device)
         mine = torch.frombuffer(bytearray(self.eng.bounds_export(nq)), dtype=torch.uint8).to(device)
         allh = torch.empty((self.world * 64,), dtype=torch.uint8, device=device)
         dist.all_gather_into_tensor(allh, mine, group=self.group)
         self.eng.bounds_import(bytes(allh.cpu().numpy().tobytes()), self.world, self.rank)
         self._bounds_cap = nq
+
+    def _reduce_xmax(self, device):
+        """Rows of this shard can be dropped by a bound a peer published: the tensor-core proof of every shard
+        uses the largest row norm of ALL shards (FVDB_OPT_PROOF_XMAX).  One all-reduce (max)."""
+        import torch
+        import torch.distributed as dist
+        xm = torch.tensor([self.eng.ivf_max_sqnorm()], dtype=torch.float32, device=device)
+        dist.all_reduce(xm, op=dist.ReduceOp.MAX, group=self.group)
+        self.eng.set_option(L.OPT_PROOF_XMAX, int(np.float32(xm.item()).view(np.uint32)))
+        self._xmax_dirty = False
+
+    def _begin_batch(self, q, nq: int, stream: int):
+        """NVLink bound sharing: reset this rank's bound array BEFORE the coarse all-gather (which orders the
+        reset before any peer's scan of this batch); the proof floor is re-reduced first after an IVF-tier
+        mutation."""
+        if not (self.share_bounds and self.world <= 8):
+            return
+        if q.is_cuda and nq > self._bounds_cap:
+            self._setup_bound_sharing(nq, q.device)
+        elif self._xmax_dirty:
+            self._reduce_xmax(q.device)
+        if q.is_cuda:
+            self.eng.bounds_begin_batch(nq, stream)
 
     def set_placement(self, owner):
         """Install a list -> rank table (place_lists) in place of the l % world rule; `owner` is a host
@@ -156,11 +215,57 @@ class ShardedIndex:
         hist += torch.bincount(a.long(), minlength=hist.shape[0])
 
     def add_rows_device(self, x, row_ids) -> int:
-        """Assign rows to lists and keep those this rank owns."""
+        """Assign rows to lists and keep those this rank owns (every rank calls this with the same rows)."""
+        self._xmax_dirty = True
         if getattr(self, "owner", None) is not None:
             return self.eng.ivf_add_device_owned(x.data_ptr(), row_ids.data_ptr(), x.shape[0], self.owner.data_ptr(),
                                                  self.rank)
         return self.eng.ivf_add_device(x.data_ptr(), row_ids.data_ptr(), x.shape[0], self.world, self.rank)
+
+    def add_recent_rows_device(self, x, row_ids) -> int:
+        """Recent-tier insert (HNSWIndex::insert, src/hnsw/core.rs:226): every rank is handed the same rows
+        (CUDA tensors x [n x dim], row_ids [n] int32) and keeps those it holds by owner_of_recent_row.
+        Returns the number of rows kept on this rank."""
+        if self.world > 1:
+            mine = (row_ids.long() & 0xFFFFFFFF) % self.world == self.rank
+            x, row_ids = x[mine].contiguous(), row_ids[mine].contiguous()
+        n = int(x.shape[0])
+        if n:
+            self.eng.flat_add_device(x.data_ptr(), row_ids.data_ptr(), n)
+        return n
+
+    def _sum_over_ranks(self, v: int) -> int:
+        if self.world == 1:
+            return int(v)
+        import torch
+        import torch.distributed as dist
+        dev = torch.device("cpu") if dist.get_backend(self.group) == "gloo" else \
+            torch.device("cuda", torch.cuda.current_device())
+        t = torch.tensor([int(v)], dtype=torch.int64, device=dev)
+        dist.all_reduce(t, op=dist.ReduceOp.SUM, group=self.group)
+        return int(t.item())
+
+    def delete(self, row_ids, deleted: bool = True):
+        """IVFIndex::mark_deleted / HNSWIndex::mark_deleted on every rank (fvdb_set_deleted): `row_ids` is a
+        host array, the same on every rank.  The tombstone bitmap is indexed by global row id, so every rank
+        takes the whole list; sharded handles (loaded through the device entries) do not track which ids they
+        hold, so ids held by other ranks, or by none, are accepted."""
+        self.eng.set_deleted(np.ascontiguousarray(row_ids, dtype=np.uint32), deleted)
+
+    def vacuum(self) -> int:
+        """fvdb_vacuum on every rank: drop the tombstoned rows each rank holds.  Returns the rows removed on
+        all ranks."""
+        self._xmax_dirty = True
+        return self._sum_over_ranks(self.eng.vacuum())
+
+    def migrate(self, row_ids) -> int:
+        """HybridIndex::migrate_with_threshold (fvdb_move_flat_to_ivf) on every rank: each rank moves those of
+        `row_ids` (host array, the same on every rank) that sit in its recent slab into its IVF arena.  A moved
+        row joins its nearest list on the rank that held it, even when another rank owns that list: results
+        do not change (every rank scans its own rows of every probed list), but the per-rank scan load drifts
+        from the placement's balance as rows migrate.  Returns the rows moved on all ranks."""
+        self._xmax_dirty = True
+        return self._sum_over_ranks(self.eng.move_flat_to_ivf(np.ascontiguousarray(row_ids, dtype=np.uint32)))
 
     def train(self, points, nlist: int, max_iterations: int, init_centroids):
         """IVFIndex::train (src/ivf/core.rs:240-334) with the points sharded over the ranks (SURVEY §8e):
@@ -209,11 +314,13 @@ class ShardedIndex:
         torch.cuda.synchronize()
         return dict(iterations=iterations, converged=converged, initial_error=initial, final_error=err)
 
-    def _buffers(self, nq: int, k: int, device, slot: int = 0):
+    def _buffers(self, nq: int, k: int, device, slot: int = 0, tiered: bool = False):
         import torch
-        key = (nq, k, slot)
+        key = (nq, k, slot, tiered)
         if key not in self._bufs:
             o_ids, o_dist, o_cnt, chunk = pack_layout(nq, k)
+            if tiered:     # two parts, recent tier then IVF tier (tiers_pack_layout); ids / dist / cnt: the first
+                chunk = tiers_pack_layout(nq, k)[4]
             # this rank's results are written straight into the three sections of its packed chunk
             pack = torch.empty((chunk,), dtype=torch.int32, device=device)
             self._bufs[key] = dict(
@@ -239,24 +346,27 @@ class ShardedIndex:
         i's result exchange (one all-gather of the packed chunks + merge) is enqueued only after batch
         i + 1's scan has been handed to the engine (fvdb_search_device_wait joins it on the device).  No
         host synchronisation per batch.  The NVLink bound arrays stay safe: a rank's reset for batch i + 2
-        is ordered behind its all-gather of batch i's results, which needs every peer's finished scan of i."""
+        is ordered behind its all-gather of batch i's results, which needs every peer's finished scan of i.
+
+        tiers: FVDB_TIER_HISTORICAL, or FVDB_TIER_BOTH (fvdb_search_device_tiers_submit + the tiered merge).
+        A rank that holds recent-tier rows runs a hybrid batch on the handle's own stream, not in a pipeline
+        slot: it is stream-ordered and correct but does not overlap its neighbours."""
         import torch
         import torch.distributed as dist
         nq = q.shape[0]
-        b = self._buffers(nq, k, q.device, slot)
+        tiered = self.world > 1 and tiers == L.TIER_BOTH
+        b = self._buffers(nq, k, q.device, slot, tiered)
         stream = _cur_stream(q)
         if self.world == 1:
             self.eng.search_device_submit(q.data_ptr(), nq, k, nprobe, tiers, 0, 0, b["ids"].data_ptr(),
                                           b["dist"].data_ptr(), b["cnt"].data_ptr(), stream)
             return b["ids"], b["dist"], b["cnt"]
-        assert (tiers & L.TIER_HISTORICAL) and nprobe > 0 and self.shard_coarse, "pipelined sharded search: IVF tier"
+        assert tiers in (L.TIER_HISTORICAL, L.TIER_BOTH) and nprobe > 0 and self.shard_coarse, \
+            "pipelined sharded search: the IVF tier, or both tiers"
         np_ = min(nprobe, self.eng.stats().nlist) if self._nlist is None else min(nprobe, self._nlist)
         if self._nlist is None:
             self._nlist = self.eng.stats().nlist
-        if self.share_bounds and q.is_cuda and self.world <= 8:
-            if nq > self._bounds_cap:
-                self._setup_bound_sharing(nq, q.device)
-            self.eng.bounds_begin_batch(nq, stream)
+        self._begin_batch(q, nq, stream)
         per = (nq + self.world - 1) // self.world
         key = ("coarse", nq, np_, slot)
         if key not in self._bufs:
@@ -281,11 +391,15 @@ class ShardedIndex:
                 mine.fill_(-1)
                 self._deferred_error = e
         dist.all_gather_into_tensor(allk, mine, group=self.group)
-        self.eng.search_device_coarse_submit(q.data_ptr(), nq, k, np_, tiers, 0, 0, allk.data_ptr(),
-                                             b["ids"].data_ptr(), b["dist"].data_ptr(), b["cnt"].data_ptr(), stream)
+        if tiered:
+            self.eng.search_device_tiers_submit(q.data_ptr(), nq, k, np_, tiers, 0, 0, allk.data_ptr(),
+                                                b["pack"].data_ptr(), stream)
+        else:
+            self.eng.search_device_coarse_submit(q.data_ptr(), nq, k, np_, tiers, 0, 0, allk.data_ptr(),
+                                                 b["ids"].data_ptr(), b["dist"].data_ptr(), b["cnt"].data_ptr(), stream)
         if self._inflight is not None:
             self._exchange(self._inflight, age=1)
-        self._inflight = (b, nq, k)
+        self._inflight = (b, nq, k, tiered)
         self._group.append((q, k, nprobe, tiers, slot))
         return b["o_ids"], b["o_dist"], b["o_cnt"]
 
@@ -293,12 +407,16 @@ class ShardedIndex:
         """Result exchange of a submitted batch: join its scan on the device, ONE all-gather, merge."""
         import torch
         import torch.distributed as dist
-        b, nq, k = rec
+        b, nq, k, tiered = rec
         stream = _cur_stream(b["pack"])
         self.eng.search_device_wait(age, stream)
         dist.all_gather_into_tensor(b["g_pack"].view(-1), b["pack"], group=self.group)
-        self.eng.merge_topk_packed_device(b["g_pack"].data_ptr(), self.world, nq, k, b["o_ids"].data_ptr(),
-                                          b["o_dist"].data_ptr(), b["o_cnt"].data_ptr(), stream)
+        self._merge(b, nq, k, tiered, stream)
+
+    def _merge(self, b, nq: int, k: int, tiered: bool, stream: int):
+        merge = self.eng.merge_topk_tiers_packed_device if tiered else self.eng.merge_topk_packed_device
+        merge(b["g_pack"].data_ptr(), self.world, nq, k, b["o_ids"].data_ptr(), b["o_dist"].data_ptr(),
+              b["o_cnt"].data_ptr(), stream)
 
     def finish(self):
         """Wait for every submitted batch.  Raises NanInput if one held a NaN query.  Several GPUs: if the
@@ -345,11 +463,14 @@ class ShardedIndex:
     def search(self, q, k: int, nprobe: int, tiers: int = L.TIER_HISTORICAL, filter_bits=None,
                filter_nbits: int = 0, slot: int = 0, _check: bool = True):
         """q: [nq x dim] CUDA tensor, identical on every rank.  Returns (ids, dist, cnt) CUDA
-        tensors holding the GLOBAL top-k on every rank."""
+        tensors holding the GLOBAL top-k on every rank.  tiers = FVDB_TIER_BOTH is HybridIndex::search over
+        both tiers (fvdb_search_device_tiers on every rank, the tiered merge); one tier alone merges by
+        (distance, row id)."""
         import torch
         import torch.distributed as dist
         nq = q.shape[0]
-        b = self._buffers(nq, k, q.device, slot)
+        tiered = self.world > 1 and tiers == L.TIER_BOTH
+        b = self._buffers(nq, k, q.device, slot, tiered)
         stream = _cur_stream(q)
         f_ptr = filter_bits.data_ptr() if filter_bits is not None else 0
         if self.world == 1:
@@ -361,12 +482,7 @@ class ShardedIndex:
             # the coarse step is sharded by QUERY: each rank ranks its slice of the batch against the
             # (replicated) centroid table, one small all-gather hands every rank the whole ranking
             np_ = min(nprobe, self.eng.stats().nlist)
-            if self.share_bounds and q.is_cuda and self.world <= 8:
-                # NVLink bound sharing: reset this rank's bound array BEFORE the coarse all-gather
-                # (which orders the reset before any peer's scan of this batch)
-                if nq > self._bounds_cap:
-                    self._setup_bound_sharing(nq, q.device)
-                self.eng.bounds_begin_batch(nq, stream)
+            self._begin_batch(q, nq, stream)
             per = (nq + self.world - 1) // self.world
             key = ("coarse", nq, np_)
             if key not in self._bufs:
@@ -381,12 +497,15 @@ class ShardedIndex:
                 self.eng.coarse_device(q[lo:lo + n_mine].data_ptr(), n_mine, np_, mine.data_ptr(), stream)
             dist.all_gather_into_tensor(allk, mine, group=self.group)
             coarse, nprobe = allk.data_ptr(), np_
-        self.eng.search_device_coarse(q.data_ptr(), nq, k, nprobe, tiers, f_ptr, filter_nbits, coarse,
-                                      b["ids"].data_ptr(), b["dist"].data_ptr(), b["cnt"].data_ptr(), stream)
+        if tiered:
+            self.eng.search_device_tiers(q.data_ptr(), nq, k, nprobe, tiers, f_ptr, filter_nbits, coarse,
+                                         b["pack"].data_ptr(), stream)
+        else:
+            self.eng.search_device_coarse(q.data_ptr(), nq, k, nprobe, tiers, f_ptr, filter_nbits, coarse,
+                                          b["ids"].data_ptr(), b["dist"].data_ptr(), b["cnt"].data_ptr(), stream)
         # ONE exchange step: all-gather of the packed per-rank chunks (ids | dist | count), then the merge
         dist.all_gather_into_tensor(b["g_pack"].view(-1), b["pack"], group=self.group)
-        self.eng.merge_topk_packed_device(b["g_pack"].data_ptr(), self.world, nq, k, b["o_ids"].data_ptr(),
-                                          b["o_dist"].data_ptr(), b["o_cnt"].data_ptr(), stream)
+        self._merge(b, nq, k, tiered, stream)
         if _check and filter_bits is None and self._tc_mode():
             # one more small collective on this (synchronous) path: did the proof fail anywhere?  (see _redo_exact)
             fb = torch.tensor([self.eng.stats().last_fallback_queries], dtype=torch.int32, device=q.device)
@@ -394,6 +513,31 @@ class ShardedIndex:
             if int(fb.item()) > 0:
                 self._redo_exact([(q, k, nprobe, tiers, slot)])
         return b["o_ids"], b["o_dist"], b["o_cnt"]
+
+    def search_postfilter(self, q, k: int, nprobe: int, keep_bits, tiers: int = L.TIER_BOTH):
+        """HybridIndex::search_with_filter (src/hybrid/core.rs:513-549), the reference's 3x post-filter, over
+        the sharded index: a sharded search of 3k, then — in order — the candidates whose row id has its bit
+        set in `keep_bits` (int64 tensor of u64 words over row ids, on q's device; ids beyond it fail), truncated
+        to k.  Like fvdb_search_postfilter it may return fewer than k rows although more match, and needs
+        3k <= k_max.  Returns (ids, dist, cnt) tensors."""
+        import torch
+        k3 = 3 * k
+        k_max = getattr(self.eng, "k_max", None)
+        if k_max is not None and k3 > k_max:
+            raise ValueError(f"search_postfilter needs 3k <= k_max ({k3} > {k_max})")
+        ids, dst, cnt = self.search(q, k3, nprobe, tiers=tiers)
+        nq = ids.shape[0]
+        rid = ids.long() & 0xFFFFFFFF
+        nwords = keep_bits.numel()
+        word = keep_bits[(rid >> 6).clamp(max=max(nwords - 1, 0))] if nwords else torch.zeros_like(rid)
+        ok = (torch.arange(k3, device=ids.device)[None, :] < cnt.long()[:, None]) & (rid < nwords * 64) & \
+             (((word >> (rid & 63)) & 1) != 0)
+        pos = torch.cumsum(ok.long(), dim=1) - 1
+        dest = torch.where(ok & (pos < k), pos, torch.full_like(pos, k))      # column k collects what is dropped
+        o_ids = torch.full((nq, k + 1), -1, dtype=torch.int32, device=ids.device).scatter_(1, dest, ids)
+        o_dst = torch.full((nq, k + 1), float("inf"), dtype=torch.float32, device=ids.device).scatter_(1, dest, dst)
+        o_cnt = ok.sum(dim=1).clamp(max=k).to(torch.int32)
+        return o_ids[:, :k].contiguous(), o_dst[:, :k].contiguous(), o_cnt
 
     def _tc_mode(self) -> bool:
         return os.environ.get("FVDB_SHARD_CHECK", "1") != "0" and self.share_bounds

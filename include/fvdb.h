@@ -328,6 +328,22 @@ int fvdb_search_device_coarse_submit(fvdb_index *h, const float *d_q, uint32_t n
                                      void *stream);
 int fvdb_search_device_wait(fvdb_index *h, uint32_t age, void *stream);
 
+/* fvdb_search_device_coarse, but the result of each tier is written separately into ONE packed chunk:
+ *   [recent ids nq*k | recent dist nq*k | recent count nq | IVF ids nq*k | IVF dist nq*k | IVF count nq]
+ * (two fvdb_merge_topk_packed_device parts back to back; 2 * (2 nq k + nq) 32-bit words).  Each part is what
+ * a search of that tier alone returns.  A tier not searched, or empty on this handle, has counts 0.
+ * d_coarse_keys may be NULL.  This is the per-rank step of a sharded FVDB_TIER_BOTH search: the chunks of
+ * all ranks are all-gathered and merged with fvdb_merge_topk_tiers_packed_device.  L2 handles only
+ * (FVDB_ERR_INVALID_CONFIG otherwise).  _submit is the stream-ordered twin (arguments and pipeline rules of
+ * fvdb_search_device_coarse_submit), finished by fvdb_search_device_finish, whose exact re-run of proof
+ * failures rewrites both parts. */
+int fvdb_search_device_tiers(fvdb_index *h, const float *d_q, uint32_t nq, uint32_t k, uint32_t nprobe,
+                             uint32_t tiers, const uint64_t *d_filter_bits, uint64_t filter_nbits,
+                             const uint64_t *d_coarse_keys, uint32_t *d_out_pack, void *stream);
+int fvdb_search_device_tiers_submit(fvdb_index *h, const float *d_q, uint32_t nq, uint32_t k, uint32_t nprobe,
+                                    uint32_t tiers, const uint64_t *d_filter_bits, uint64_t filter_nbits,
+                                    const uint64_t *d_coarse_keys, uint32_t *d_out_pack, void *stream);
+
 /* Multi-GPU bound sharing over NVLink peer memory (one process per GPU, lists sharded by
  * l % world as above).  During the posting-list scan every query carries a running upper bound of
  * its 32nd-nearest approximate distance; rows above it are dropped in the epilogue.  A shard that
@@ -365,13 +381,22 @@ int fvdb_merge_topk_packed_device(fvdb_index *h, const uint32_t *d_pack, uint32_
  * the ABI's tie rule, so the merged result equals one unsharded search however the rows are split.
  * The parts must hold disjoint rows of ONE tier, each part sorted by (distance, row id) — as the
  * list-sharded IVF search (FVDB_TIER_HISTORICAL) and a recent-tier scan split into slabs produce them.
- * A FVDB_TIER_BOTH search orders recent-tier rows first on equal distances; a part does not carry
- * the tier of its rows, so merging such parts is unsupported (ties would be ordered by id alone).
+ * A FVDB_TIER_BOTH search orders recent-tier rows first on equal distances; a part here does not carry
+ * the tier of its rows, so FVDB_TIER_BOTH results are merged with fvdb_merge_topk_tiers_packed_device.
  * Counts above k are clamped to k; parts must be in 1..64.  Device pointers. */
 int fvdb_merge_topk_device(fvdb_index *h, const uint32_t *d_ids, const float *d_dist,
                            const uint32_t *d_count, uint32_t parts, uint32_t nq, uint32_t k,
                            uint32_t *d_out_ids, float *d_out_dist, uint32_t *d_out_count,
                            void *stream);
+
+/* After the all-gather of the per-rank fvdb_search_device_tiers chunks: 2 * ranks parts, part 2r = recent
+ * tier of rank r, part 2r + 1 = IVF tier of rank r.  Order: (distance, tier with recent first, row id), i.e.
+ * the merge of src/hybrid/core.rs:482-483 applied across GPUs, equal to one unsharded FVDB_TIER_BOTH search
+ * however the rows of both tiers are split over the ranks.  Counts above k are clamped to k.  ranks 1..32;
+ * L2 handles only (FVDB_ERR_INVALID_CONFIG otherwise).  Device pointers. */
+int fvdb_merge_topk_tiers_packed_device(fvdb_index *h, const uint32_t *d_pack, uint32_t ranks, uint32_t nq,
+                                        uint32_t k, uint32_t *d_out_ids, float *d_out_dist,
+                                        uint32_t *d_out_count, void *stream);
 
 /* Device-resident variants of the bulk loaders (row data already in HBM, e.g. generated on
  * the device for the 100M-row sharded configuration).  `list_filter_mod`/`list_filter_rem`:

@@ -146,6 +146,80 @@ print(f"rank {rank}/{world}: lattice rows with {ties4} cross-rank tie groups in 
       f"to the oracle: {bool(same4)}", flush=True)
 ok = ok and bool(same4)
 
+# ---- hybrid search (FVDB_TIER_BOTH): the lattice rows above as the IVF tier; a recent tier in slabs (id % world)
+# holding copies of IVF rows under HIGHER ids (cross-tier ties across ranks), fresh rows, and 200 rows three times
+# longer than any IVF row.  Delete, vacuum, then a migration that moves the long rows into the IVF arenas: the
+# tensor-core proof's norm floor (FVDB_OPT_PROOF_XMAX, shared bounds) must follow them --------------------------------
+n4 = x4.shape[0]
+rng5 = np.random.default_rng(5)
+big5 = 3 * rng5.integers(0, 2, size=(200, 64)).astype(np.float32)
+fx5 = np.concatenate([x4[rng5.choice(n4, 2000, replace=False)], rng5.integers(0, 2, size=(2000, 64)).astype(np.float32), big5])
+fid5 = np.arange(n4, n4 + fx5.shape[0], dtype=np.uint32)
+q5 = np.concatenate([q4, big5[:8]])
+dq5s = [torch.from_numpy(np.ascontiguousarray(np.roll(q5, s, axis=0))).to(dev) for s in range(3)]
+
+
+def _same(g, w):
+    return bool((g[0].cpu().numpy().view(np.uint32) == w[0]).all() and (g[1].cpu().numpy().view(np.uint32) == w[1].view(np.uint32)).all()
+                and (g[2].cpu().numpy().view(np.uint32) == w[2]).all())
+
+
+for mode in (L.SCAN_EXACT, L.SCAN_TC):
+    eng = Engine(64, k_max=16, device=local)
+    eng.set_option(L.OPT_SCAN_MODE, mode)
+    eng.set_centroids(c4)
+    sh = ShardedIndex(eng, rank, world)
+    sh.add_rows_device(torch.from_numpy(x4).to(dev), torch.arange(n4, dtype=torch.int32, device=dev))
+    kept5 = sh.add_recent_rows_device(torch.from_numpy(fx5).to(dev), torch.from_numpy(fid5.view(np.int32)).to(dev))
+    s_x, s_ids, s_fx, s_fid = x4, np.arange(n4, dtype=np.uint32), fx5, fid5
+    bm5 = None
+    line = []
+    for step in ("load", "delete", "vacuum", "migrate"):
+        if step == "delete":
+            dele5 = np.concatenate([np.arange(1, n4, 7), fid5[2::5]]).astype(np.uint32)
+            sh.delete(dele5)
+            bm5 = O.make_bitmap(n4 + fx5.shape[0], dele5)
+        elif step == "vacuum":
+            removed = sh.vacuum()
+            ok = ok and removed == dele5.size
+            kx, kf = ~np.isin(s_ids, dele5), ~np.isin(s_fid, dele5)
+            s_x, s_ids, s_fx, s_fid, bm5 = s_x[kx], s_ids[kx], s_fx[kf], s_fid[kf], None
+        elif step == "migrate":
+            mig = np.concatenate([s_fid[s_fid < n4 + 4000][::2], s_fid[s_fid >= n4 + 4000]])
+            moved = sh.migrate(mig)
+            ok = ok and moved == mig.size
+            m = np.isin(s_fid, mig)
+            s_x, s_ids = np.concatenate([s_x, s_fx[m]]), np.concatenate([s_ids, s_fid[m]])
+            s_fx, s_fid = s_fx[~m], s_fid[~m]
+        ivf5 = O.IVF(c4, s_x, s_ids)
+        ws = [O.hybrid_batch_search(ivf5, s_fx, s_fid, np.roll(q5, s, axis=0), K, 6, tiers=3, deleted=bm5) for s in range(3)]
+        same_s = _same(sh.search(dq5s[0], K, 6, tiers=L.TIER_BOTH), ws[0])
+        torch.cuda.synchronize()
+        outs5 = [sh.submit(dq5s[s], K, 6, tiers=L.TIER_BOTH, slot=s) for s in range(3)]
+        sh.finish()
+        torch.cuda.synchronize()
+        same_p = all(_same(outs5[s], ws[s]) for s in range(3))
+        if step == "load":
+            # tie groups of the oracle's top-k holding a recent row and an IVF row that sit on different ranks
+            w_ids, w_dst, w_cnt = ws[0]
+            r_ivf = (ivf5.assign % world).astype(np.int64)
+            pos = np.full(n4 + fx5.shape[0], -1, dtype=np.int64)
+            pos[s_ids] = np.arange(s_ids.size)
+            ties5 = 0
+            for i in range(q5.shape[0]):
+                for v in np.unique(w_dst[i, :w_cnt[i]]):
+                    grp = w_ids[i, :w_cnt[i]][w_dst[i, :w_cnt[i]] == v]
+                    rec, iv = grp[grp >= n4], grp[grp < n4]
+                    rk = set((rec % world).tolist()) | set(r_ivf[pos[iv]].tolist())
+                    ties5 += int(rec.size > 0 and iv.size > 0 and len(rk) > 1)
+            line.append(f"{ties5} cross-tier cross-rank tie groups")
+            ok = ok and (ties5 > 0 or world == 1)
+        line.append(f"{step}: sync {same_s} pipelined {same_p}")
+        ok = ok and same_s and same_p
+    print(f"rank {rank}/{world} mode {mode}: hybrid (TIER_BOTH), {kept5} recent rows on this rank, "
+          + ", ".join(line) + f" — identical to the oracle: {all('False' not in s for s in line)}", flush=True)
+    eng.close()
+
 # ---- sharded k-means (points split over the ranks, one all-reduce per iteration) against the single-GPU
 # order-faithful training from the same initial centroids ------------------------------------------------
 eng = Engine(D, k_max=16, device=local)
