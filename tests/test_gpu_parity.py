@@ -79,7 +79,7 @@ def _set_mode(eng, mode):
     (4000, 384, 32, 8, 10, 64),
     (3000, 128, 16, 16, 5, 33),
     (5000, 384, 64, 1, 10, 1),
-    (2000, 64, 8, 3, 32, 130),
+    (2000, 64, 8, 3, 16, 130),
 ])
 def test_ivf_search_parity(mode, n, d, nlist, nprobe, k, nq):
     if mode == "tc" and d % 32:
