@@ -142,6 +142,40 @@ struct StdRng08 {
     float gen_f32() { return (float)(next_u32() >> 8) * (1.0f / 16777216.0f); }
 };
 
+// Pinned host destinations of a batch's results: the device -> host copies ride in front of the
+// batch's single synchronisation point (the NaN flag / fallback counter read-back).
+struct HostOut {
+    void* ids;
+    void* dist;
+    void* cnt;
+    size_t ob, cb;  // bytes of ids / dist, of cnt
+};
+
+// The per-batch scratch of a search: counter words, the IVF tier's proof-failure list, coarse and IVF keys,
+// tensor-core tables and the timing events.  The handle owns one for the batches on its own stream; each
+// pipeline slot owns another.
+struct BatchScratch {
+    // misc words: [0] nan flag, [2..3] scanned rows (u64), [4] kmeans changed, [6] item count,
+    // [8] kmeans++ pick, [10] IVF fallback count, [11] flat fallback count, [12] assign fallback count,
+    // [13] max |x|^2 bits
+    DevBuf<uint32_t> misc, fb_idx;
+    DevBuf<uint64_t> coarse, ivf_keys;
+    TcScratch tc;
+    cudaEvent_t ev_a = nullptr, ev_b = nullptr;     // around the batch
+    cudaEvent_t ev_s0 = nullptr, ev_s1 = nullptr;   // around the scan kernel
+    cudaError_t create_events() {
+        cudaError_t e = cudaSuccess;
+        for (cudaEvent_t* ev : {&ev_a, &ev_b, &ev_s0, &ev_s1})
+            if (e == cudaSuccess) e = cudaEventCreate(ev);
+        return e;
+    }
+    void release() {
+        tc_release(tc);
+        for (cudaEvent_t ev : {ev_a, ev_b, ev_s0, ev_s1})
+            if (ev) cudaEventDestroy(ev);
+    }
+};
+
 }  // namespace
 
 // One fvdb_search call waiting in the handle's submission queue (see fvdb_search).
@@ -162,7 +196,6 @@ struct fvdb_index {
     int metric = 0;
     int sm_count = 148;
     cudaStream_t stream = nullptr;
-    cudaEvent_t ev_a = nullptr, ev_b = nullptr, ev_s0 = nullptr, ev_s1 = nullptr;
     std::mutex mu;
     std::string err;
     uint32_t scan_mode = FVDB_SCAN_EXACT;
@@ -200,32 +233,34 @@ struct fvdb_index {
     bool track_ids = true;
 
     // scratch (grow-only)
+    BatchScratch scratch;                // per-batch scratch of everything that runs on the handle's stream
     DevBuf<float> s_q, s_x;              // staged queries / staged rows
     DevBuf<uint32_t> s_u32a, s_u32b, s_u32c, s_perm, s_keys32;
     DevBuf<uint64_t> s_filter;
-    DevBuf<uint64_t> s_partial, s_partial2, s_coarse, s_ivf_keys, s_flat_keys;
+    DevBuf<uint64_t> s_partial, s_partial2, s_flat_keys;
     DevBuf<ScanItem> s_items, s_items2;
-    DevBuf<uint32_t> s_list_cnt, s_pair_off, s_cursor, s_pair_q, s_pair_slot, s_misc;
+    DevBuf<uint32_t> s_list_cnt, s_pair_off, s_cursor, s_pair_q, s_pair_slot;
     DevBuf<unsigned char> s_group;
     DevBuf<uint32_t> s_out_ids, s_out_cnt;
     DevBuf<float> s_out_dist, s_f32a;
     DevBuf<double> s_f64;
     DevBuf<uint64_t> s_tmpbits;
-    DevBuf<uint32_t> s_fb_idx;
     DevBuf<uint32_t> s_fb_idx_flat;
-    // batches enqueued by fvdb_search_device_submit and not yet checked by ..._finish
+    // A page-locked block of u32 words and its size: the read-back record of a stream-ordered batch.
+    using Record = std::pair<uint32_t*, size_t>;
+    // A search batch whose kernels are enqueued: what a repair of its proof failures re-runs and where its figures
+    // come from.  The stream-ordered entries keep it until fvdb_search_device_finish.
     struct Pending {
         const float* d_q; uint32_t nq, k, nprobe, tiers;
         const uint64_t* d_filter; uint64_t filter_bits;
         uint32_t* d_out_ids; float* d_out_dist; uint32_t* d_out_count;
+        HostOut ho;           // the caller's pinned result buffers (ids NULL: none)
+        bool split;           // fvdb_search_device_tiers: the outputs are a two-part packed chunk
         bool used_tc, flat_tc, use_ivf, use_flat;
         uint32_t n_bitmaps;   // tombstone / filter bitmaps read per row (for the algorithmic-bytes figure)
-        uint32_t* host;       // page-locked: [16] counter words, [2 nq] IVF fallback ids, [2 nq] flat fallback ids
-        size_t host_words;
-        void *ho_ids, *ho_dist, *ho_cnt;   // fvdb_search_submit: the caller's page-locked result buffers (else NULL)
         int slot;             // pipeline slot the batch ran in (-1: the handle's own stream and scratch)
-        cudaStream_t user_stream;
-        bool split;           // fvdb_search_device_tiers_submit: the outputs are a two-part packed chunk
+        BatchScratch* scratch;   // the scratch it ran with (its timing events)
+        Record rec;           // stream-ordered: [16] counter words, [2 nq] IVF fallback ids, [2 nq] flat fallback ids
     };
     // fvdb_search_submit: device-side query / result buffers of the batches in flight and the copy stream
     // their uploads run on (so that batch i + 1 uploads while batch i is scanned)
@@ -241,24 +276,21 @@ struct fvdb_index {
     uint32_t host_slot_next = 0;
     cudaStream_t copy_stream = nullptr;
     std::vector<Pending> pending;
-    std::vector<std::pair<uint32_t*, size_t>> pending_coarse;   // records of fvdb_coarse_device_submit
-    std::vector<std::pair<uint32_t*, size_t>> pending_pool;   // recycled page-locked blocks
+    std::vector<Record> pending_coarse;   // records of fvdb_coarse_device_submit
+    std::vector<Record> pending_pool;     // recycled page-locked blocks
     DevBuf<float> s_fb_q;
     DevBuf<uint64_t> s_fb_keys, s_fb_coarse;
-    TcScratch tc;
+    DevBuf<uint32_t> s_fb_rows;          // the queries a proof-failure repair re-runs
     // Software pipeline of the stream-ordered entries (fvdb_search_device_submit / fvdb_search_submit):
-    // consecutive batches alternate between two SLOTS, each with its own stream and its own copy of the
-    // per-batch scratch (tensor-core tables, coarse keys, counters).  The scans of consecutive batches are
+    // consecutive batches alternate between two SLOTS, each with its own stream and its own per-batch
+    // scratch (tensor-core tables, coarse keys, counters).  The scans of consecutive batches are
     // serialised by an event (each one fills the machine), but batch i + 1's query norms, coarse step and
     // bucketing and batch i's shortlist merge and re-rank no longer queue behind one another: they run in
     // the scans' ramps and tails and next to kernel R's CTAs wherever registers and shared memory allow.
     struct Slot {
+        BatchScratch b;
         cudaStream_t stream = nullptr;
-        cudaEvent_t ev_a = nullptr, ev_b = nullptr, ev_s0 = nullptr, ev_s1 = nullptr;
         cudaEvent_t ev_in = nullptr, ev_scan_end = nullptr, ev_done = nullptr;
-        DevBuf<uint32_t> s_misc, s_fb_idx;
-        DevBuf<uint64_t> s_coarse, s_ivf_keys;
-        TcScratch tc;
         bool busy = false;
     };
     static constexpr int N_SLOTS = 2;
@@ -305,12 +337,12 @@ struct fvdb_index {
 };
 
 static inline void mark_arena_dirty(fvdb_index* h) {
-    h->tc.arena_dirty = true;
-    for (auto& sl : h->slots) sl.tc.arena_dirty = true;
+    h->scratch.tc.arena_dirty = true;
+    for (auto& sl : h->slots) sl.b.tc.arena_dirty = true;
 }
 static inline void mark_centroids_dirty(fvdb_index* h) {
-    h->tc.centroids_dirty = true;
-    for (auto& sl : h->slots) sl.tc.centroids_dirty = true;
+    h->scratch.tc.centroids_dirty = true;
+    for (auto& sl : h->slots) sl.b.tc.centroids_dirty = true;
 }
 // Every batch still running in a pipeline slot has to finish before anything it reads may move.
 static inline void quiesce_slots(fvdb_index* h) {
@@ -360,8 +392,8 @@ int d2h(fvdb_index* h, void* dst, const void* src, size_t bytes) {
 }
 
 int check_nan_device(fvdb_index* h, const float* d_x, size_t n, cudaStream_t st) {
-    CK(h->s_misc.ensure(64, 0, st, &h->dev_bytes));
-    int* flag = reinterpret_cast<int*>(h->s_misc.p);
+    CK(h->scratch.misc.ensure(64, 0, st, &h->dev_bytes));
+    int* flag = reinterpret_cast<int*>(h->scratch.misc.p);
     CK(cudaMemsetAsync(flag, 0, sizeof(int), st));
     CK(launch_nan_check(d_x, n, flag, st));
     int hf = 0;
@@ -493,17 +525,18 @@ int assign_device(fvdb_index* h, const float* d_x, uint64_t n, uint32_t* d_assig
                   const uint32_t* prev, uint32_t* d_changed, cudaStream_t st) {
     if (n == 0) return FVDB_OK;
     if (n >= 0xFFFFFFFFull) return h->fail(FVDB_ERR_INVALID_ARG, "batch exceeds u32 rows");
-    CK(h->s_ivf_keys.ensure(n, 0, st, &h->dev_bytes));
+    BatchScratch& b = h->scratch;
+    CK(b.ivf_keys.ensure(n, 0, st, &h->dev_bytes));
     // Large batches (k-means iterations, bulk insert / load): the rows play the "queries", the
     // centroid table the scanned row set of the tensor-core flat scan; the four approximately
     // nearest centroids are re-ranked in the reference's arithmetic and the fifth bounds the rest
     // (proof as in tc_scan.cu); rows whose proof fails are re-assigned by the exact kernel.
     const bool tc = h->scan_mode == FVDB_SCAN_TC && tc_supported(h->dim) && h->nlist >= 256 &&
-                    n * (uint64_t)h->nlist >= (64ull << 20) && !getenv("FVDB_ASSIGN_EXACT");
+                    n * (uint64_t)h->nlist >= (64ull << 20);
     if (tc) {
         const uint64_t CH = 1u << 18;   // rows per pass: bounds the shortlist scratch (256 B per row)
-        CK(h->s_misc.ensure(64, 0, st, &h->dev_bytes));
-        uint32_t* d_fb = h->s_misc.p + 12;
+        CK(b.misc.ensure(64, 0, st, &h->dev_bytes));
+        uint32_t* d_fb = b.misc.p + 12;
         for (uint64_t r0 = 0; r0 < n; r0 += CH) {
             const uint32_t m = (uint32_t)std::min<uint64_t>(CH, n - r0);
             CK(h->s_fb_idx_flat.ensure((size_t)2 * m, 0, st, &h->dev_bytes));
@@ -511,13 +544,13 @@ int assign_device(fvdb_index* h, const float* d_x, uint64_t n, uint32_t* d_assig
             TcFlatArgs fa{};
             fa.rows = h->centroids.p; fa.ids = nullptr; fa.n_rows = h->nlist;
             fa.Q = d_x + r0 * h->dim; fa.nq = m; fa.D = h->dim; fa.k = 1;
-            fa.out_keys = h->s_ivf_keys.p + r0;
+            fa.out_keys = b.ivf_keys.p + r0;
             fa.d_fallback_count = d_fb; fa.d_fallback_idx = h->s_fb_idx_flat.p;
             fa.sm_count = h->sm_count;
             fa.state = 1; fa.version = h->centroids_version; fa.rerank_r = 4;
             fa.argmin_only = d_dist == nullptr;
             uint32_t launches = 0;
-            int r = tc_flat_search(h->tc, fa, st, &h->dev_bytes, &launches, &h->err);
+            int r = tc_flat_search(b.tc, fa, st, &h->dev_bytes, &launches, &h->err);
             if (r != FVDB_OK) return r;
             uint32_t n_fb = 0;
             CK(cudaMemcpyAsync(&n_fb, d_fb, 4, cudaMemcpyDeviceToHost, st));
@@ -529,15 +562,15 @@ int assign_device(fvdb_index* h, const float* d_x, uint64_t n, uint32_t* d_assig
                 CK(launch_gather_rows(d_x + r0 * h->dim, m, nullptr, h->s_fb_idx_flat.p, n_fb, h->dim, h->s_fb_q.p, st));
                 RET(scan_all_exact(h, h->centroids.p, nullptr, h->nlist, h->s_fb_q.p, n_fb, 1, nullptr, 0, nullptr, 0,
                                    h->s_fb_keys.p, st));
-                CK(launch_scatter_keys(h->s_fb_keys.p, h->s_fb_idx_flat.p, n_fb, 1, h->s_ivf_keys.p + r0, st));
+                CK(launch_scatter_keys(h->s_fb_keys.p, h->s_fb_idx_flat.p, n_fb, 1, b.ivf_keys.p + r0, st));
             }
             h->assign_fallback_rows += n_fb;
         }
     } else {
         RET(scan_all_exact(h, h->centroids.p, nullptr, h->nlist, d_x, (uint32_t)n, 1, nullptr, 0,
-                           nullptr, 0, h->s_ivf_keys.p, st));
+                           nullptr, 0, b.ivf_keys.p, st));
     }
-    CK(launch_extract_assign(h->s_ivf_keys.p, n, d_assign, d_dist, prev, d_changed, st));
+    CK(launch_extract_assign(b.ivf_keys.p, n, d_assign, d_dist, prev, d_changed, st));
     return FVDB_OK;
 }
 
@@ -595,7 +628,7 @@ int flat_add_device_impl(fvdb_index* h, const float* d_x, const uint32_t* d_ids,
     CK(cudaMemcpyAsync(h->flat_ids.p + h->flat_n, d_ids, n * 4, cudaMemcpyDeviceToDevice, st));
     CK(cudaStreamSynchronize(st));
     h->flat_n += n;
-    h->tc.flat_dirty = true;
+    h->scratch.tc.flat_dirty = true;
     return FVDB_OK;
 }
 
@@ -713,8 +746,8 @@ int train_body(fvdb_index* h, const float* d_data, uint64_t n, uint32_t nlist, u
     DevBuf<uint32_t> assign;
     CK(assign.ensure(n, 0, st, nullptr, true));
     CK(cudaMemsetAsync(assign.p, 0, n * 4, st));  // vec![ClusterId(0); n]
-    CK(h->s_misc.ensure(64, 0, st, &h->dev_bytes));
-    uint32_t* d_changed = h->s_misc.p + 4;
+    CK(h->scratch.misc.ensure(64, 0, st, &h->dev_bytes));
+    uint32_t* d_changed = h->scratch.misc.p + 4;
     float prev_error = INFINITY;
     float initial_error = 0.f;
     RET(compute_error_device(h, d_data, n, assign.p, &initial_error));
@@ -814,10 +847,10 @@ int ivf_scan_exact(fvdb_index* h, const float* d_q, uint32_t nq, uint32_t k, uin
     // 32-query tiles that would be mostly padding
     const bool sparse = n_pairs <= (size_t)4 * h->nlist && (size_t)4 * (D * 4 + k * 8) <= 200 * 1024;
     if (sparse) {
-        if (timed) CK(cudaEventRecord(h->ev_s0, st));
+        if (timed) CK(cudaEventRecord(h->scratch.ev_s0, st));
         CK(launch_exact_pair_scan(coarse, nq, np, h->list_off.p, h->ivf_rows.p, h->ivf_ids.p, d_q, D, Ppad, k, tomb,
                                   h->tomb_bits, filt, filter_bits, h->s_partial.p, st));
-        if (timed) CK(cudaEventRecord(h->ev_s1, st));
+        if (timed) CK(cudaEventRecord(h->scratch.ev_s1, st));
         h->stats.last_launches += 1;
         if (d_scanned) CK(cudaMemsetAsync(d_scanned, 0, 8, st));
     } else {
@@ -828,7 +861,7 @@ int ivf_scan_exact(fvdb_index* h, const float* d_q, uint32_t nq, uint32_t k, uin
     CK(h->s_pair_q.ensure(n_pairs, 0, st, &h->dev_bytes));
     CK(h->s_pair_slot.ensure(n_pairs, 0, st, &h->dev_bytes));
     CK(h->s_items.ensure(max_items, 0, st, &h->dev_bytes));
-    uint32_t* d_n_items = h->s_misc.p + 6;
+    uint32_t* d_n_items = h->scratch.misc.p + 6;
     CK(launch_probe_bucketing(coarse, nq, np, h->list_off.p, h->nlist, tq, h->s_list_cnt.p,
                               h->s_pair_off.p, h->s_cursor.p, h->s_pair_q.p, h->s_pair_slot.p,
                               h->s_items.p, d_n_items, d_scanned, st));
@@ -840,9 +873,9 @@ int ivf_scan_exact(fvdb_index* h, const float* d_q, uint32_t nq, uint32_t k, uin
     a.P = Ppad; a.k = k;
     a.tomb = tomb; a.tomb_bits = h->tomb_bits; a.filt = filt; a.filt_bits = filter_bits;
     a.partial = h->s_partial.p;
-    if (timed) CK(cudaEventRecord(h->ev_s0, st));
+    if (timed) CK(cudaEventRecord(h->scratch.ev_s0, st));
     CK(launch_exact_scan(a, (uint32_t)max_items, st));
-    if (timed) CK(cudaEventRecord(h->ev_s1, st));
+    if (timed) CK(cudaEventRecord(h->scratch.ev_s1, st));
     h->stats.last_launches += 1;
     }
     // sort + truncate(k) (src/ivf/core.rs:677-678)
@@ -858,54 +891,66 @@ int ivf_scan_exact(fvdb_index* h, const float* d_q, uint32_t nq, uint32_t k, uin
     return FVDB_OK;
 }
 
+// The tensor-core IVF scan serves k <= 16 and up to 256 probed lists (np: nprobe clamped to nlist).
+bool tc_ivf_scan(uint32_t scan_mode, uint32_t D, uint32_t k, uint32_t np) {
+    return scan_mode == FVDB_SCAN_TC && tc_supported(D) && k <= TC_MAX_K && np <= TC_MAX_NPROBE;
+}
+// The tensor-core coarse step serves D <= 384 and up to 112 probed lists; else the exact CUDA-core scan ranks them.
+bool tc_coarse_step(uint32_t scan_mode, uint32_t D, uint32_t np) {
+    return scan_mode == FVDB_SCAN_TC && tc_supported(D) && D <= 384 && np <= TC_MAX_NPROBE_COARSE;
+}
+
+// A page-locked record of at least `words` u32: a recycled one from the pool, else a new one.
+cudaError_t take_record(fvdb_index* h, size_t words, fvdb_index::Record* rec) {
+    for (size_t i = 0; i < h->pending_pool.size(); ++i)
+        if (h->pending_pool[i].second >= words) {
+            *rec = h->pending_pool[i];
+            h->pending_pool.erase(h->pending_pool.begin() + i);
+            return cudaSuccess;
+        }
+    *rec = {nullptr, words};
+    return cudaHostAlloc((void**)&rec->first, words * 4, cudaHostAllocDefault);
+}
+
 // Coarse ranking only (src/ivf/core.rs:646-656) for nq queries: keys [nq][np] (distance bits << 32 |
 // list id), ascending, ties to the lower list id.  Tensor cores + exact verify when possible;
 // queries whose proof fails are re-ranked by the exact kernel.
 int coarse_device_impl(fvdb_index* h, const float* d_q, uint32_t nq, uint32_t np, uint64_t* d_out_keys,
-                       cudaStream_t st, bool defer = false) {
+                       cudaStream_t st, bool deferred = false) {
     const uint32_t D = h->dim;
     if (nq == 0) return FVDB_OK;
-    CK(h->s_misc.ensure(64, 0, st, &h->dev_bytes));
-    int* d_nan = reinterpret_cast<int*>(h->s_misc.p);
-    uint32_t* d_fb_count = h->s_misc.p + 10;
-    CK(cudaMemsetAsync(h->s_misc.p, 0, 64, st));
+    BatchScratch& b = h->scratch;
+    CK(b.misc.ensure(64, 0, st, &h->dev_bytes));
+    int* d_nan = reinterpret_cast<int*>(b.misc.p);
+    uint32_t* d_fb_count = b.misc.p + 10;
+    CK(cudaMemsetAsync(b.misc.p, 0, 64, st));
     CK(launch_nan_check(d_q, (size_t)nq * D, d_nan, st));
-    const bool tc = (h->scan_mode == FVDB_SCAN_TC) && tc_supported(D) && D <= 384 && np <= TC_MAX_NPROBE_COARSE &&
-                    !getenv("FVDB_EXACT_COARSE");
+    const bool tc = tc_coarse_step(h->scan_mode, D, np);
     if (tc) {
-        CK(h->s_fb_idx.ensure((size_t)2 * nq, 0, st, &h->dev_bytes));
+        CK(b.fb_idx.ensure((size_t)2 * nq, 0, st, &h->dev_bytes));
         TcSearchArgs ta{};
         ta.nlist = h->nlist; ta.Q = d_q; ta.nq = nq; ta.D = D; ta.k = 1; ta.nprobe = np;
         ta.centroids = h->centroids.p; ta.coarse_keys = nullptr; ta.coarse_out = d_out_keys; ta.coarse_only = true;
-        ta.d_fallback_count = d_fb_count; ta.d_fallback_idx = h->s_fb_idx.p;
+        ta.d_fallback_count = d_fb_count; ta.d_fallback_idx = b.fb_idx.p;
         ta.sm_count = h->sm_count;
         uint32_t launches = 0;
-        int r = tc_ivf_search(h->tc, ta, st, &h->dev_bytes, &launches, &h->err);
+        int r = tc_ivf_search(b.tc, ta, st, &h->dev_bytes, &launches, &h->err);
         if (r != FVDB_OK) return r;
     } else {
         RET(scan_all_exact(h, h->centroids.p, nullptr, h->nlist, d_q, nq, np, nullptr, 0, nullptr, 0, d_out_keys, st));
     }
-    if (defer) {
+    if (deferred) {
         // stream-ordered: the NaN flag and the number of queries whose tensor-core proof failed go to a
         // page-locked record that fvdb_search_device_finish looks at (it reports them; the caller re-runs
         // the batch through the synchronous entry, which repairs them)
-        uint32_t* rec = nullptr;
-        for (size_t i = 0; i < h->pending_pool.size(); ++i)
-            if (h->pending_pool[i].second >= 16) {
-                rec = h->pending_pool[i].first;
-                h->pending_coarse.push_back(h->pending_pool[i]);
-                h->pending_pool.erase(h->pending_pool.begin() + i);
-                break;
-            }
-        if (!rec) {
-            CK(cudaHostAlloc((void**)&rec, 16 * 4, cudaHostAllocDefault));
-            h->pending_coarse.push_back({rec, 16});
-        }
-        CK(cudaMemcpyAsync(rec, h->s_misc.p, 64, cudaMemcpyDeviceToHost, st));
+        fvdb_index::Record rec;
+        CK(take_record(h, 16, &rec));
+        h->pending_coarse.push_back(rec);
+        CK(cudaMemcpyAsync(rec.first, b.misc.p, 64, cudaMemcpyDeviceToHost, st));
         return FVDB_OK;
     }
     uint32_t host_misc[16] = {0};
-    CK(cudaMemcpyAsync(host_misc, h->s_misc.p, sizeof(host_misc), cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(host_misc, b.misc.p, sizeof(host_misc), cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     if (host_misc[0])
         return h->fail(FVDB_ERR_NAN, "NaN in query (the reference panics on partial_cmp().unwrap())");
@@ -913,23 +958,15 @@ int coarse_device_impl(fvdb_index* h, const float* d_q, uint32_t nq, uint32_t np
     if (n_fb) {
         CK(h->s_fb_q.ensure((size_t)n_fb * D, 0, st, &h->dev_bytes));
         CK(h->s_fb_coarse.ensure((size_t)n_fb * np, 0, st, &h->dev_bytes));
-        CK(launch_gather_rows(d_q, nq, nullptr, h->s_fb_idx.p, n_fb, D, h->s_fb_q.p, st));
+        CK(launch_gather_rows(d_q, nq, nullptr, b.fb_idx.p, n_fb, D, h->s_fb_q.p, st));
         RET(scan_all_exact(h, h->centroids.p, nullptr, h->nlist, h->s_fb_q.p, n_fb, np, nullptr, 0, nullptr, 0,
                            h->s_fb_coarse.p, st));
-        CK(launch_scatter_keys(h->s_fb_coarse.p, h->s_fb_idx.p, n_fb, np, d_out_keys, st));
+        CK(launch_scatter_keys(h->s_fb_coarse.p, b.fb_idx.p, n_fb, np, d_out_keys, st));
         CK(cudaStreamSynchronize(st));
     }
     return FVDB_OK;
 }
 
-// Pinned host destinations of a batch's results: the device -> host copies ride in front of the
-// batch's single synchronisation point (the NaN flag / fallback counter read-back).
-struct HostOut {
-    void* ids;
-    void* dist;
-    void* cnt;
-    size_t ob, cb;  // bytes of ids / dist, of cnt
-};
 cudaError_t copy_out(const HostOut* ho, const uint32_t* d_ids, const float* d_dist, const uint32_t* d_cnt,
                      cudaStream_t st) {
     cudaError_t e = cudaMemcpyAsync(ho->ids, d_ids, ho->ob, cudaMemcpyDeviceToHost, st);
@@ -944,12 +981,50 @@ bool is_pinned_host(const void* p) {
     return a.type == cudaMemoryTypeHost;
 }
 
+// The optional arguments of search_device_impl.
+struct SearchOpts {
+    const uint64_t* ext_coarse = nullptr;   // the batch's coarse keys [nq][nprobe], ranked by the caller
+    const HostOut* ho = nullptr;            // pinned host destinations of the results
+    bool deferred = false;                  // stream-ordered: finish_pending checks the batch (and repairs it)
+    cudaEvent_t wait_first = nullptr;       // the batch starts behind this event
+    bool split = false;                     // fvdb_search_device_tiers: each tier to its own part of a packed chunk
+    bool exact = false;                     // the exact path whatever the scan mode (a proof-failure repair)
+};
+
+int repair_rows(fvdb_index* h, const fvdb_index::Pending& pb, const std::vector<uint32_t>& rows, cudaStream_t st);
+
+// The figures of a finished batch into h->stats; `misc` is its counter words, read back.  Call it before anything
+// records the batch's events again.
+void set_batch_stats(fvdb_index* h, const fvdb_index::Pending& pb, const uint32_t* misc) {
+    uint64_t scanned = 0;
+    std::memcpy(&scanned, misc + 2, 8);
+    const uint64_t rows = scanned + (pb.use_flat ? h->flat_n : 0);
+    h->stats.last_nq = pb.nq;
+    h->stats.last_scanned_rows = rows;
+    h->stats.last_algorithmic_bytes = rows * h->dim * 4ull + (uint64_t)pb.nq * h->dim * 4ull + (uint64_t)pb.nq * pb.k * 8ull +
+                                      (pb.use_ivf ? (uint64_t)h->nlist * h->dim * 4ull : 0ull) + (uint64_t)pb.n_bitmaps * (rows / 8);
+    auto elapsed = [](cudaEvent_t a, cudaEvent_t b) {
+        float ms = 0.f;
+        if (cudaEventElapsedTime(&ms, a, b) != cudaSuccess) { cudaGetLastError(); ms = 0.f; }
+        return ms;
+    };
+    h->stats.last_device_ms = elapsed(pb.scratch->ev_a, pb.scratch->ev_b);
+    h->stats.last_scan_ms = pb.use_ivf ? elapsed(pb.scratch->ev_s0, pb.scratch->ev_s1) : 0.f;   // the IVF scan is timed
+}
+
+// The queries of a batch to re-run: both tiers' proof-failure lists as one ascending list without repeats.
+std::vector<uint32_t> failed_queries(const uint32_t* ivf, uint32_t n_ivf, const uint32_t* flat, uint32_t n_flat) {
+    std::vector<uint32_t> q(ivf, ivf + n_ivf);
+    q.insert(q.end(), flat, flat + n_flat);
+    std::sort(q.begin(), q.end());
+    q.erase(std::unique(q.begin(), q.end()), q.end());
+    return q;
+}
+
 int search_device_impl(fvdb_index* h, const float* d_q, uint32_t nq, uint32_t k, uint32_t nprobe,
                        uint32_t tiers, const uint64_t* d_filter, uint64_t filter_bits,
                        uint32_t* d_out_ids, float* d_out_dist, uint32_t* d_out_count,
-                       cudaStream_t st, const uint64_t* ext_coarse = nullptr, const HostOut* ho = nullptr,
-                       bool defer = false, bool want_pipe = false, cudaEvent_t wait_first = nullptr,
-                       bool split = false) {
+                       cudaStream_t st, const SearchOpts& o = {}) {
     if (k == 0) return h->fail(FVDB_ERR_INVALID_ARG, "k must be >= 1");
     if (k > h->k_max) return h->fail(FVDB_ERR_K_TOO_LARGE, "k exceeds k_max given at fvdb_create");
     h->stats.last_nq = nq;
@@ -962,58 +1037,52 @@ int search_device_impl(fvdb_index* h, const float* d_q, uint32_t nq, uint32_t k,
     if (nq == 0) return FVDB_OK;
     RET(seal(h));
     const uint32_t D = h->dim;
+    const uint32_t mode = o.exact ? FVDB_SCAN_EXACT : h->scan_mode;
     // the IVF tier exists for L2 only (fvdb_ivf_* reject a similarity handle), so use_ivf implies L2
     const bool use_ivf = (tiers & FVDB_TIER_HISTORICAL) && h->trained && h->ivf_n > 0 && nprobe > 0;
     const bool use_flat = (tiers & FVDB_TIER_RECENT) && h->flat_n > 0;
     const uint64_t* tomb = h->deleted_count ? h->tomb.p : nullptr;
     const uint64_t* filt = d_filter;
+    const uint32_t np = use_ivf ? std::min(nprobe, h->nlist) : 0;
+    if (np > 512) return h->fail(FVDB_ERR_INVALID_ARG, "nprobe > 512 is not supported");
     // the tensor-core IVF path looks at every query element anyway (query norms): it raises the flag
-    const bool tc_ivf = use_ivf && (h->scan_mode == FVDB_SCAN_TC) && tc_supported(D) && k <= TC_MAX_K &&
-                        std::min(nprobe, h->nlist) <= TC_MAX_NPROBE;
+    const bool tc_ivf = use_ivf && tc_ivf_scan(mode, D, k, np);
+    // coarse step: all centroid distances, nearest np lists (src/ivf/core.rs:646-656); exact CUDA-core
+    // scan, or tensor-core distances + exact verify (or handed in: the multi-GPU driver ranks a slice of
+    // the batch per GPU and all-gathers)
+    const bool tc_coarse = tc_ivf && !o.ext_coarse && tc_coarse_step(mode, D, np);
 
     // Pipeline slot (stream-ordered entries, IVF tier alone on the tensor-core path): this batch runs on
     // the slot's stream with the slot's scratch; `st` (the caller's stream) is only what its inputs are
     // ordered after.  Everything else runs on `st` with the handle's own scratch, after the slots drained.
-    const cudaStream_t user_st = st;
     int slot = -1;
-    const bool tc_coarse_ok = D <= 384 && std::min(nprobe, h->nlist) <= TC_MAX_NPROBE_COARSE && !getenv("FVDB_EXACT_COARSE");
-    if (defer && want_pipe && h->pipeline && tc_ivf && (tc_coarse_ok || ext_coarse) && !use_flat) {
+    if (o.deferred && h->pipeline && tc_ivf && (tc_coarse || o.ext_coarse) && !use_flat) {
         slot = (int)(h->slot_next++ % fvdb_index::N_SLOTS);
         fvdb_index::Slot& sl = h->slots[slot];
         if (!sl.stream) {
             CK(cudaStreamCreateWithFlags(&sl.stream, cudaStreamNonBlocking));
-            CK(cudaEventCreate(&sl.ev_a)); CK(cudaEventCreate(&sl.ev_b));
-            CK(cudaEventCreate(&sl.ev_s0)); CK(cudaEventCreate(&sl.ev_s1));
+            CK(sl.b.create_events());
             CK(cudaEventCreateWithFlags(&sl.ev_in, cudaEventDisableTiming));
             CK(cudaEventCreateWithFlags(&sl.ev_scan_end, cudaEventDisableTiming));
             CK(cudaEventCreateWithFlags(&sl.ev_done, cudaEventDisableTiming));
         }
-        CK(cudaEventRecord(sl.ev_in, user_st));
+        CK(cudaEventRecord(sl.ev_in, st));
         CK(cudaStreamWaitEvent(sl.stream, sl.ev_in, 0));
-        if (wait_first) CK(cudaStreamWaitEvent(sl.stream, wait_first, 0));
+        if (o.wait_first) CK(cudaStreamWaitEvent(sl.stream, o.wait_first, 0));
         st = sl.stream;
         sl.busy = true;
     } else {
         quiesce_slots(h);
-        if (wait_first) CK(cudaStreamWaitEvent(st, wait_first, 0));
+        if (o.wait_first) CK(cudaStreamWaitEvent(st, o.wait_first, 0));
     }
     fvdb_index::Slot* const sl = slot >= 0 ? &h->slots[slot] : nullptr;
-    DevBuf<uint32_t>& b_misc = sl ? sl->s_misc : h->s_misc;
-    DevBuf<uint32_t>& b_fb_idx = sl ? sl->s_fb_idx : h->s_fb_idx;
-    DevBuf<uint64_t>& b_coarse = sl ? sl->s_coarse : h->s_coarse;
-    DevBuf<uint64_t>& b_ivf_keys = sl ? sl->s_ivf_keys : h->s_ivf_keys;
-    TcScratch& b_tc = sl ? sl->tc : h->tc;
-    const cudaEvent_t e_a = sl ? sl->ev_a : h->ev_a, e_b = sl ? sl->ev_b : h->ev_b;
-    const cudaEvent_t e_s0 = sl ? sl->ev_s0 : h->ev_s0, e_s1 = sl ? sl->ev_s1 : h->ev_s1;
+    BatchScratch& b = sl ? sl->b : h->scratch;
 
-    CK(cudaEventRecord(e_a, st));
-    CK(b_misc.ensure(64, 0, st, &h->dev_bytes));
-    // s_misc words: [0] nan flag, [2..3] scanned rows (u64), [4] kmeans changed, [6] item count,
-    // [8] kmeans++ pick, [10] TC fallback count
-    int* d_nan = reinterpret_cast<int*>(b_misc.p);
-    uint64_t* d_scanned = reinterpret_cast<uint64_t*>(b_misc.p + 2);
-    uint32_t* d_fb_count = b_misc.p + 10;
-    CK(cudaMemsetAsync(b_misc.p, 0, 64, st));
+    CK(cudaEventRecord(b.ev_a, st));
+    CK(b.misc.ensure(64, 0, st, &h->dev_bytes));
+    int* d_nan = reinterpret_cast<int*>(b.misc.p);
+    uint64_t* d_scanned = reinterpret_cast<uint64_t*>(b.misc.p + 2);
+    CK(cudaMemsetAsync(b.misc.p, 0, 64, st));
     if (!tc_ivf) {
         CK(launch_nan_check(d_q, (size_t)nq * D, d_nan, st));
         h->stats.last_launches += 1;
@@ -1024,33 +1093,24 @@ int search_device_impl(fvdb_index* h, const float* d_q, uint32_t nq, uint32_t k,
     // split (fvdb_search_device_tiers): the result arrays are the recent-tier part of a packed chunk
     // [ids nq*k | dist nq*k | count nq]; the IVF tier's part follows it, one part length further on
     const size_t part_words = (size_t)2 * nq * k + nq;
-    uint32_t* const ivf_out_ids = split ? d_out_ids + part_words : nullptr;
-    float* const ivf_out_dist = split ? d_out_dist + part_words : nullptr;
-    uint32_t* const ivf_out_count = split ? d_out_count + part_words : nullptr;
-    bool scan_timed = false, used_tc = false, fused_finalize = false;
-    uint32_t np = 0;
+    uint32_t* const ivf_out_ids = o.split ? d_out_ids + part_words : nullptr;
+    float* const ivf_out_dist = o.split ? d_out_dist + part_words : nullptr;
+    uint32_t* const ivf_out_count = o.split ? d_out_count + part_words : nullptr;
+    bool fused_finalize = false;
 
     if (use_ivf) {
-        np = std::min(nprobe, h->nlist);
-        if (np > 512) return h->fail(FVDB_ERR_INVALID_ARG, "nprobe > 512 is not supported");
-        CK(b_ivf_keys.ensure((size_t)nq * k, 0, st, &h->dev_bytes));
-        ivf_keys = b_ivf_keys.p;
-        used_tc = (h->scan_mode == FVDB_SCAN_TC) && tc_supported(D) && k <= TC_MAX_K && np <= TC_MAX_NPROBE;
-        // coarse step: all centroid distances, nearest np lists (src/ivf/core.rs:646-656); exact
-        // CUDA-core scan, or (TC mode, D <= 384, np <= 128) tensor-core distances + exact verify
-        // (or handed in: the multi-GPU driver ranks a slice of the batch per GPU and all-gathers)
-        const bool tc_coarse = !ext_coarse && used_tc && D <= 384 && np <= TC_MAX_NPROBE_COARSE &&
-                               !getenv("FVDB_EXACT_COARSE");
-        const uint64_t* coarse_in = ext_coarse;
-        if (!ext_coarse) {
-            CK(b_coarse.ensure((size_t)nq * np, 0, st, &h->dev_bytes));
-            coarse_in = b_coarse.p;
+        CK(b.ivf_keys.ensure((size_t)nq * k, 0, st, &h->dev_bytes));
+        ivf_keys = b.ivf_keys.p;
+        const uint64_t* coarse_in = o.ext_coarse;
+        if (!o.ext_coarse) {
+            CK(b.coarse.ensure((size_t)nq * np, 0, st, &h->dev_bytes));
+            coarse_in = b.coarse.p;
             if (!tc_coarse)
                 RET(scan_all_exact(h, h->centroids.p, nullptr, h->nlist, d_q, nq, np, nullptr, 0, nullptr, 0,
-                                   b_coarse.p, st));
+                                   b.coarse.p, st));
         }
-        if (used_tc) {
-            CK(b_fb_idx.ensure((size_t)2 * nq, 0, st, &h->dev_bytes));
+        if (tc_ivf) {
+            CK(b.fb_idx.ensure((size_t)2 * nq, 0, st, &h->dev_bytes));
             TcSearchArgs ta{};
             ta.rows = h->ivf_rows.p; ta.ids = h->ivf_ids.p; ta.n_rows = h->ivf_n;
             ta.list_off = h->list_off.p; ta.nlist = h->nlist;
@@ -1061,13 +1121,13 @@ int search_device_impl(fvdb_index* h, const float* d_q, uint32_t nq, uint32_t k,
             ta.tomb = tomb; ta.tomb_bits = h->tomb_bits; ta.filt = filt; ta.filt_bits = filter_bits;
             ta.out_keys = ivf_keys;
             ta.d_scanned_rows = d_scanned;
-            ta.d_fallback_count = d_fb_count; ta.d_fallback_idx = b_fb_idx.p;
-            ta.ev_scan0 = e_s0; ta.ev_scan1 = e_s1;
+            ta.d_fallback_count = b.misc.p + 10; ta.d_fallback_idx = b.fb_idx.p;
+            ta.ev_scan0 = b.ev_s0; ta.ev_scan1 = b.ev_s1;
             ta.sm_count = h->sm_count;
             ta.xmax_floor_sq = h->proof_xmax_sq;
             ta.scan_sms = sl ? h->scan_sms : 0;   // only pipelined batches have neighbours to leave room for
             ta.d_nan = d_nan;
-            if (!use_flat && !split) {   // the only tier: the re-rank writes the result arrays itself
+            if (!use_flat && !o.split) {   // the only tier: the re-rank writes the result arrays itself
                 ta.fin_ids = d_out_ids; ta.fin_dist = d_out_dist; ta.fin_count = d_out_count;
                 fused_finalize = true;
             }
@@ -1081,30 +1141,26 @@ int search_device_impl(fvdb_index* h, const float* d_q, uint32_t nq, uint32_t k,
             uint32_t launches = 0;
             if (sl) {
                 // one scan at a time: this one waits for the scan of the batch enqueued before it
-                ta.wait_before_scan = getenv("FVDB_PIPE_NOSERIAL") ? nullptr : h->prev_scan_end;
+                ta.wait_before_scan = h->prev_scan_end;
                 ta.record_after_scan = sl->ev_scan_end;
             }
-            int r = tc_ivf_search(b_tc, ta, st, &h->dev_bytes, &launches, &h->err);
+            int r = tc_ivf_search(b.tc, ta, st, &h->dev_bytes, &launches, &h->err);
             if (sl && r == FVDB_OK) h->prev_scan_end = sl->ev_scan_end;
             if (r != FVDB_OK) return r;
             h->stats.last_launches += launches;
-            scan_timed = true;
         } else {
             RET(ivf_scan_exact(h, d_q, nq, k, np, coarse_in, tomb, filt, filter_bits, ivf_keys,
                                d_scanned, true, st));
-            scan_timed = true;
         }
     }
     bool flat_tc = false;
-    uint32_t* d_fb_count_flat = b_misc.p + 11;
     if (use_flat) {
         CK(h->s_flat_keys.ensure((size_t)nq * k, 0, st, &h->dev_bytes));
         flat_keys = h->s_flat_keys.p;
         // recent tier: exhaustive scan instead of the HNSW walk (src/hnsw/core.rs:398-467); on the
         // tensor cores when the batch is large enough to amortise the item set-up
-        flat_tc = (h->scan_mode == FVDB_SCAN_TC) && tc_supported(D) && k <= TC_MAX_K &&
-                  (uint64_t)h->flat_n * nq >= (4ull << 20) && !getenv("FVDB_FLAT_EXACT") &&
-                  (h->metric == FVDB_METRIC_L2 || D <= 384);
+        flat_tc = mode == FVDB_SCAN_TC && tc_supported(D) && k <= TC_MAX_K &&
+                  (uint64_t)h->flat_n * nq >= (4ull << 20) && (h->metric == FVDB_METRIC_L2 || D <= 384);
         if (flat_tc) {
             CK(h->s_fb_idx_flat.ensure((size_t)2 * nq, 0, st, &h->dev_bytes));
             TcFlatArgs fa{};
@@ -1112,11 +1168,11 @@ int search_device_impl(fvdb_index* h, const float* d_q, uint32_t nq, uint32_t k,
             fa.Q = d_q; fa.nq = nq; fa.D = D; fa.k = k;
             fa.tomb = tomb; fa.tomb_bits = h->tomb_bits; fa.filt = filt; fa.filt_bits = filter_bits;
             fa.out_keys = flat_keys;
-            fa.d_fallback_count = d_fb_count_flat; fa.d_fallback_idx = h->s_fb_idx_flat.p;
+            fa.d_fallback_count = b.misc.p + 11; fa.d_fallback_idx = h->s_fb_idx_flat.p;
             fa.sm_count = h->sm_count;
             fa.metric = h->metric;
             uint32_t launches = 0;
-            int r = tc_flat_search(h->tc, fa, st, &h->dev_bytes, &launches, &h->err);
+            int r = tc_flat_search(h->scratch.tc, fa, st, &h->dev_bytes, &launches, &h->err);
             if (r != FVDB_OK) return r;
             h->stats.last_launches += launches;
         } else {
@@ -1129,94 +1185,81 @@ int search_device_impl(fvdb_index* h, const float* d_q, uint32_t nq, uint32_t k,
                            ivf_out_ids, ivf_out_dist, ivf_out_count));
         h->stats.last_launches += 1;
     }
-    CK(cudaEventRecord(e_b, st));
-    if (ho) CK(copy_out(ho, d_out_ids, d_out_dist, d_out_count, st));
+    CK(cudaEventRecord(b.ev_b, st));
+    if (o.ho) CK(copy_out(o.ho, d_out_ids, d_out_dist, d_out_count, st));
 
-    if (defer) {
+    fvdb_index::Pending pb{d_q, nq, k, nprobe, tiers, d_filter, filter_bits, d_out_ids, d_out_dist, d_out_count,
+                           o.ho ? *o.ho : HostOut{}, o.split, tc_ivf, flat_tc, use_ivf, use_flat,
+                           (tomb ? 1u : 0u) + (filt ? 1u : 0u), slot, &b, {nullptr, 0}};
+    if (o.deferred) {
         // stream-ordered variant: the counters and the fallback lists are copied to a page-locked
         // record in stream order; fvdb_search_device_finish looks at them after ONE synchronisation
         // for any number of batches (no GPU idle time between consecutive batches)
-        const size_t words = 16 + (size_t)4 * nq;
-        fvdb_index::Pending pb{d_q, nq, k, nprobe, tiers, d_filter, filter_bits, d_out_ids, d_out_dist, d_out_count,
-                               used_tc, flat_tc, use_ivf, use_flat, (tomb ? 1u : 0u) + (filt ? 1u : 0u), nullptr, 0,
-                               ho ? ho->ids : nullptr, ho ? ho->dist : nullptr, ho ? ho->cnt : nullptr, slot, user_st,
-                               split};
-        for (size_t i = 0; i < h->pending_pool.size(); ++i)
-            if (h->pending_pool[i].second >= words) {
-                pb.host = h->pending_pool[i].first; pb.host_words = h->pending_pool[i].second;
-                h->pending_pool.erase(h->pending_pool.begin() + i);
-                break;
-            }
-        if (!pb.host) {
-            CK(cudaHostAlloc((void**)&pb.host, words * 4, cudaHostAllocDefault));
-            pb.host_words = words;
-        }
-        CK(cudaMemcpyAsync(pb.host, b_misc.p, 64, cudaMemcpyDeviceToHost, st));
-        if (used_tc) CK(cudaMemcpyAsync(pb.host + 16, b_fb_idx.p, (size_t)2 * nq * 4, cudaMemcpyDeviceToHost, st));
-        if (flat_tc) CK(cudaMemcpyAsync(pb.host + 16 + 2 * nq, h->s_fb_idx_flat.p, (size_t)2 * nq * 4, cudaMemcpyDeviceToHost, st));
+        CK(take_record(h, 16 + (size_t)4 * nq, &pb.rec));
+        uint32_t* rec = pb.rec.first;
+        CK(cudaMemcpyAsync(rec, b.misc.p, 64, cudaMemcpyDeviceToHost, st));
+        if (tc_ivf) CK(cudaMemcpyAsync(rec + 16, b.fb_idx.p, (size_t)2 * nq * 4, cudaMemcpyDeviceToHost, st));
+        if (flat_tc) CK(cudaMemcpyAsync(rec + 16 + 2 * nq, h->s_fb_idx_flat.p, (size_t)2 * nq * 4, cudaMemcpyDeviceToHost, st));
         if (sl) CK(cudaEventRecord(sl->ev_done, st));
         h->pending.push_back(pb);
         return FVDB_OK;
     }
     // one synchronisation point per batch: NaN flag + counters
     uint32_t host_misc[16] = {0};
-    CK(cudaMemcpyAsync(host_misc, h->s_misc.p, sizeof(host_misc), cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(host_misc, b.misc.p, sizeof(host_misc), cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     if (host_misc[0])
         return h->fail(FVDB_ERR_NAN, "NaN in query (the reference panics on partial_cmp().unwrap())");
-    uint64_t scanned = 0;
-    std::memcpy(&scanned, &host_misc[2], 8);
-    float ms = 0.f;
-    CK(cudaEventElapsedTime(&ms, h->ev_a, h->ev_b));
-    h->stats.last_device_ms = ms;
-    if (scan_timed) {
-        float sms = 0.f;
-        if (cudaEventElapsedTime(&sms, h->ev_s0, h->ev_s1) == cudaSuccess) h->stats.last_scan_ms = sms;
-        else cudaGetLastError();
-    }
-    const uint32_t n_fb_flat = flat_tc ? std::min(host_misc[11], 2 * nq) : 0;
-    if (n_fb_flat) {
-        // flat-tier proof failures: exact scan of the recent tier for exactly those queries
-        CK(h->s_fb_q.ensure((size_t)n_fb_flat * D, 0, st, &h->dev_bytes));
-        CK(h->s_fb_keys.ensure((size_t)n_fb_flat * k, 0, st, &h->dev_bytes));
-        CK(launch_gather_rows(d_q, nq, nullptr, h->s_fb_idx_flat.p, n_fb_flat, D, h->s_fb_q.p, st));
-        RET(scan_all_exact(h, h->flat_rows.p, h->flat_ids.p, h->flat_n, h->s_fb_q.p, n_fb_flat, k, tomb, h->tomb_bits,
-                           filt, filter_bits, h->s_fb_keys.p, st, h->metric));
-        CK(launch_scatter_keys(h->s_fb_keys.p, h->s_fb_idx_flat.p, n_fb_flat, k, flat_keys, st));
-        CK(launch_finalize(flat_keys, ivf_keys, nq, k, d_out_ids, d_out_dist, d_out_count, st, h->metric,
-                           ivf_out_ids, ivf_out_dist, ivf_out_count));
-        if (ho) CK(copy_out(ho, d_out_ids, d_out_dist, d_out_count, st));
+    set_batch_stats(h, pb, host_misc);
+    const uint32_t n_ivf = tc_ivf ? std::min(host_misc[10], 2 * nq) : 0;
+    const uint32_t n_flat = flat_tc ? std::min(host_misc[11], 2 * nq) : 0;
+    if (n_ivf || n_flat) {
+        // the tensor-core proof failed for some queries (rare: only near-duplicate-heavy neighbourhoods):
+        // their lists come back, and the repair re-runs them on the exact path
+        std::vector<uint32_t> lists(n_ivf + n_flat);
+        if (n_ivf) CK(cudaMemcpyAsync(lists.data(), b.fb_idx.p, (size_t)n_ivf * 4, cudaMemcpyDeviceToHost, st));
+        if (n_flat)
+            CK(cudaMemcpyAsync(lists.data() + n_ivf, h->s_fb_idx_flat.p, (size_t)n_flat * 4, cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));
-        h->stats.last_launches += 3;
-        h->stats.last_fallback_queries += n_fb_flat;
+        const std::vector<uint32_t> rows = failed_queries(lists.data(), n_ivf, lists.data() + n_ivf, n_flat);
+        RET(repair_rows(h, pb, rows, st));
+        h->stats.last_fallback_queries = (uint32_t)rows.size();
     }
-    const uint32_t n_fb = used_tc ? std::min(host_misc[10], 2 * nq) : 0;
-    if (n_fb) {
-        // the tensor-core proof failed for n_fb queries: re-run exactly those on the exact path
-        // and patch their rows of the result (rare: only near-duplicate-heavy neighbourhoods)
-        CK(h->s_fb_q.ensure((size_t)n_fb * D, 0, st, &h->dev_bytes));
-        CK(h->s_fb_keys.ensure((size_t)n_fb * k, 0, st, &h->dev_bytes));
-        CK(h->s_fb_coarse.ensure((size_t)n_fb * np, 0, st, &h->dev_bytes));
-        CK(launch_gather_rows(d_q, nq, nullptr, h->s_fb_idx.p, n_fb, D, h->s_fb_q.p, st));
-        RET(scan_all_exact(h, h->centroids.p, nullptr, h->nlist, h->s_fb_q.p, n_fb, np, nullptr, 0, nullptr,
-                           0, h->s_fb_coarse.p, st));
-        RET(ivf_scan_exact(h, h->s_fb_q.p, n_fb, k, np, h->s_fb_coarse.p, tomb, filt, filter_bits,
-                           h->s_fb_keys.p, nullptr, false, st));
-        CK(launch_scatter_keys(h->s_fb_keys.p, h->s_fb_idx.p, n_fb, k, ivf_keys, st));
-        CK(launch_finalize(flat_keys, ivf_keys, nq, k, d_out_ids, d_out_dist, d_out_count, st, h->metric,
-                           ivf_out_ids, ivf_out_dist, ivf_out_count));
-        if (ho) CK(copy_out(ho, d_out_ids, d_out_dist, d_out_count, st));
-        CK(cudaStreamSynchronize(st));
-        h->stats.last_launches += 3;
-        h->stats.last_fallback_queries += n_fb;
+    return FVDB_OK;
+}
+
+// Proof failures of a batch: the queries `rows` (ascending, distinct) are searched again on the exact path,
+// every tier the batch asked for (a tier whose proof held returns the same bits there), and their result rows
+// are replaced: in both parts of a split batch, and in the pinned host outputs when the batch has them.
+// h->stats keep describing the batch; last_launches adds the repair's launches.
+int repair_rows(fvdb_index* h, const fvdb_index::Pending& pb, const std::vector<uint32_t>& rows, cudaStream_t st) {
+    const uint32_t m = (uint32_t)rows.size(), k = pb.k;
+    // the row list, the gathered queries and the re-run results sit in buffers the nested search does not use
+    CK(h->s_fb_rows.ensure(m, 0, st, &h->dev_bytes));
+    CK(h->s_fb_q.ensure((size_t)m * h->dim, 0, st, &h->dev_bytes));
+    CK(h->s_fb_keys.ensure((size_t)m * k * 2 + m, 0, st, &h->dev_bytes));   // ids | dist | counts, two parts
+    CK(cudaMemcpyAsync(h->s_fb_rows.p, rows.data(), (size_t)m * 4, cudaMemcpyHostToDevice, st));
+    CK(launch_gather_rows(pb.d_q, pb.nq, nullptr, h->s_fb_rows.p, m, h->dim, h->s_fb_q.p, st));
+    uint32_t* t_ids = reinterpret_cast<uint32_t*>(h->s_fb_keys.p);
+    float* t_dist = reinterpret_cast<float*>(t_ids + (size_t)m * k);
+    uint32_t* t_cnt = t_ids + (size_t)2 * m * k;
+    const fvdb_stats batch = h->stats;
+    SearchOpts o; o.split = pb.split; o.exact = true;
+    RET(search_device_impl(h, h->s_fb_q.p, m, k, pb.nprobe, pb.tiers, pb.d_filter, pb.filter_bits, t_ids, t_dist,
+                           t_cnt, st, o));
+    uint32_t launches = h->stats.last_launches + 2;   // and the gather and the scatter
+    CK(launch_scatter_result_rows(t_ids, t_dist, t_cnt, h->s_fb_rows.p, m, k, pb.d_out_ids, pb.d_out_dist,
+                                  pb.d_out_count, st));
+    if (pb.split) {   // the IVF tier's part follows the recent tier's, one part length further on
+        const size_t tp = (size_t)2 * m * k + m, bp = (size_t)2 * pb.nq * k + pb.nq;
+        CK(launch_scatter_result_rows(t_ids + tp, t_dist + tp, t_cnt + tp, h->s_fb_rows.p, m, k, pb.d_out_ids + bp,
+                                      pb.d_out_dist + bp, pb.d_out_count + bp, st));
+        launches += 1;
     }
-    uint64_t rows = scanned + (use_flat ? h->flat_n : 0);
-    h->stats.last_scanned_rows = rows;
-    uint64_t bytes = rows * D * 4ull + (uint64_t)nq * D * 4ull + (uint64_t)nq * k * 8ull;
-    if (use_ivf) bytes += (uint64_t)h->nlist * D * 4ull;
-    if (tomb) bytes += rows / 8;
-    if (filt) bytes += rows / 8;
-    h->stats.last_algorithmic_bytes = bytes;
+    if (pb.ho.ids) CK(copy_out(&pb.ho, pb.d_out_ids, pb.d_out_dist, pb.d_out_count, st));
+    CK(cudaStreamSynchronize(st));
+    h->stats = batch;
+    h->stats.last_launches += launches;
     return FVDB_OK;
 }
 
@@ -1270,10 +1313,8 @@ int fvdb_create(int device, uint32_t dim, int metric, uint32_t k_max, fvdb_index
     h->k_max = k_max;
     h->sm_count = prop.multiProcessorCount;
     h->scan_mode = tc_supported(dim) ? FVDB_SCAN_TC : FVDB_SCAN_EXACT;
-    if (const char* e = getenv("FVDB_SCAN_SMS")) h->scan_sms = (uint32_t)std::max(0, atoi(e));
     if (cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking) != cudaSuccess ||
-        cudaEventCreate(&h->ev_a) != cudaSuccess || cudaEventCreate(&h->ev_b) != cudaSuccess ||
-        cudaEventCreate(&h->ev_s0) != cudaSuccess || cudaEventCreate(&h->ev_s1) != cudaSuccess) {
+        h->scratch.create_events() != cudaSuccess) {
         delete h;
         return fail(FVDB_ERR_CUDA, "stream/event creation failed");
     }
@@ -1287,14 +1328,14 @@ void fvdb_destroy(fvdb_index* h) {
     if (h->stream) cudaStreamSynchronize(h->stream);
     for (auto& sl : h->slots) {
         if (sl.stream) cudaStreamSynchronize(sl.stream);
-        tc_release(sl.tc);
-        for (cudaEvent_t e : {sl.ev_a, sl.ev_b, sl.ev_s0, sl.ev_s1, sl.ev_in, sl.ev_scan_end, sl.ev_done})
+        sl.b.release();
+        for (cudaEvent_t e : {sl.ev_in, sl.ev_scan_end, sl.ev_done})
             if (e) cudaEventDestroy(e);
         if (sl.stream) cudaStreamDestroy(sl.stream);
     }
-    tc_release(h->tc);
+    h->scratch.release();
     if (h->pin) cudaFreeHost(h->pin);
-    for (auto& pb : h->pending) cudaFreeHost(pb.host);
+    for (auto& pb : h->pending) cudaFreeHost(pb.rec.first);
     for (auto& pp : h->pending_pool) cudaFreeHost(pp.first);
     for (auto& pp : h->pending_coarse) cudaFreeHost(pp.first);
     for (auto& sl : h->host_slots) {
@@ -1302,10 +1343,6 @@ void fvdb_destroy(fvdb_index* h) {
         if (sl.done) cudaEventDestroy(sl.done);
     }
     if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
-    if (h->ev_a) cudaEventDestroy(h->ev_a);
-    if (h->ev_b) cudaEventDestroy(h->ev_b);
-    if (h->ev_s0) cudaEventDestroy(h->ev_s0);
-    if (h->ev_s1) cudaEventDestroy(h->ev_s1);
     for (uint32_t* pb : h->peer_bounds) cudaIpcCloseMemHandle(pb);
     if (h->bounds) cudaFree(h->bounds);
     if (h->stream) cudaStreamDestroy(h->stream);
@@ -1674,7 +1711,7 @@ int fvdb_vacuum(fvdb_index* h, uint64_t* removed) {
         h->flat_ids.swap(nids);
         gone += n - kept;
         h->flat_n = kept;
-        h->tc.flat_dirty = true;
+        h->scratch.tc.flat_dirty = true;
     }
     CK(cudaMemsetAsync(h->tomb.p, 0, (h->tomb_bits + 63) / 64 * 8, st));
     CK(cudaStreamSynchronize(st));
@@ -1733,7 +1770,7 @@ int fvdb_move_flat_to_ivf(fvdb_index* h, const uint32_t* row_ids, uint64_t n, ui
     h->flat_rows.swap(nrows);
     h->flat_ids.swap(nids);
     h->flat_n = stay;
-    h->tc.flat_dirty = true;
+    h->scratch.tc.flat_dirty = true;
     if (h->track_ids)
         for (uint64_t i = 0; i < n; ++i)
             if (row_ids[i] < h->id_state.size() && (h->id_state[row_ids[i]] & 3) == 1)
@@ -1757,8 +1794,9 @@ int fvdb_search_device_submit(fvdb_index* h, const float* d_q, uint32_t nq, uint
     ENTER_PIPE(h);
     cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
     if (h->pending.size() >= 64) return h->fail(FVDB_ERR_INVALID_ARG, "64 batches are pending: call fvdb_search_device_finish");
+    SearchOpts o; o.deferred = true;
     return search_device_impl(h, d_q, nq, k, nprobe, tiers, d_filter_bits, filter_nbits, d_out_ids,
-                              d_out_dist, d_out_count, st, nullptr, nullptr, true, true);
+                              d_out_dist, d_out_count, st, o);
 }
 
 static int finish_pending(fvdb_index* h, cudaStream_t st);
@@ -1797,8 +1835,8 @@ int fvdb_search_submit(fvdb_index* h, const float* q, uint32_t nq, uint32_t k, u
     CK(cudaEventRecord(sl.uploaded, h->copy_stream));
     const HostOut ho{out_ids, out_dist, out_count, (size_t)nq * k * 4, (size_t)nq * 4};
     // the batch (in a pipeline slot when it qualifies) starts once its queries are on the device
-    const int rc = search_device_impl(h, sl.q.p, nq, k, nprobe, tiers, nullptr, 0, sl.ids.p, sl.dist.p, sl.cnt.p, st,
-                                      nullptr, &ho, true, true, sl.uploaded);
+    SearchOpts o; o.ho = &ho; o.deferred = true; o.wait_first = sl.uploaded;
+    const int rc = search_device_impl(h, sl.q.p, nq, k, nprobe, tiers, nullptr, 0, sl.ids.p, sl.dist.p, sl.cnt.p, st, o);
     if (rc == FVDB_OK && !h->pending.empty()) {
         const int ps = h->pending.back().slot;
         CK(cudaEventRecord(sl.done, ps >= 0 ? h->slots[ps].stream : st));
@@ -1821,7 +1859,7 @@ static int finish_pending(fvdb_index* h, cudaStream_t st) {
         if (sl.busy && sl.stream) { bad |= cudaStreamSynchronize(sl.stream) != cudaSuccess; sl.busy = false; }
     if (bad || cudaStreamSynchronize(st) != cudaSuccess) {
         cudaGetLastError();
-        for (const fvdb_index::Pending& pb : h->pending) h->pending_pool.push_back({pb.host, pb.host_words});
+        for (const fvdb_index::Pending& pb : h->pending) h->pending_pool.push_back(pb.rec);
         for (auto& rec : h->pending_coarse) h->pending_pool.push_back(rec);
         h->pending.clear();
         h->pending_coarse.clear();
@@ -1830,61 +1868,23 @@ static int finish_pending(fvdb_index* h, cudaStream_t st) {
     int rc = FVDB_OK;
     std::vector<fvdb_index::Pending> todo;
     todo.swap(h->pending);
+    // the figures of the last batch, as the synchronous call reports them
+    if (!todo.empty()) set_batch_stats(h, todo.back(), todo.back().rec.first);
     uint32_t fallbacks = 0;
     for (const fvdb_index::Pending& pb : todo) {
-        if (rc == FVDB_OK && pb.host[0])
+        const uint32_t* host = pb.rec.first;
+        if (rc == FVDB_OK && host[0])
             rc = h->fail(FVDB_ERR_NAN, "NaN in query (the reference panics on partial_cmp().unwrap())");
-        const uint32_t n_ivf = pb.used_tc ? std::min(pb.host[10], 2 * pb.nq) : 0;
-        const uint32_t n_flat = pb.flat_tc ? std::min(pb.host[11], 2 * pb.nq) : 0;
+        const uint32_t n_ivf = pb.used_tc ? std::min(host[10], 2 * pb.nq) : 0;
+        const uint32_t n_flat = pb.flat_tc ? std::min(host[11], 2 * pb.nq) : 0;
         if (rc == FVDB_OK && (n_ivf || n_flat)) {
-            // proof failures: these queries are searched again on the exact path (both tiers as asked
-            // for) and their result rows replaced
-            std::vector<uint32_t> idx(pb.host + 16, pb.host + 16 + n_ivf);
-            idx.insert(idx.end(), pb.host + 16 + 2 * pb.nq, pb.host + 16 + 2 * pb.nq + n_flat);
-            std::sort(idx.begin(), idx.end());
-            idx.erase(std::unique(idx.begin(), idx.end()), idx.end());
-            const uint32_t m = (uint32_t)idx.size();
-            int r2 = [&]() -> int {
-                CK(h->s_fb_q.ensure((size_t)m * h->dim, 0, st, &h->dev_bytes));
-                CK(h->s_fb_idx.ensure(std::max<size_t>(m, 2 * pb.nq), 0, st, &h->dev_bytes));
-                CK(h->s_fb_keys.ensure((size_t)m * pb.k * 2 + m, 0, st, &h->dev_bytes));   // ids | dist | counts
-                CK(cudaMemcpyAsync(h->s_fb_idx.p, idx.data(), (size_t)m * 4, cudaMemcpyHostToDevice, st));
-                CK(launch_gather_rows(pb.d_q, pb.nq, nullptr, h->s_fb_idx.p, m, h->dim, h->s_fb_q.p, st));
-                uint32_t* t_ids = reinterpret_cast<uint32_t*>(h->s_fb_keys.p);
-                float* t_dist = reinterpret_cast<float*>(t_ids + (size_t)m * pb.k);
-                uint32_t* t_cnt = t_ids + (size_t)2 * m * pb.k;
-                // keep the fallback ids out of the recursion's scratch: a second buffer holds them
-                CK(h->s_fb_coarse.ensure(m, 0, st, &h->dev_bytes));
-                CK(cudaMemcpyAsync(h->s_fb_coarse.p, h->s_fb_idx.p, (size_t)m * 4, cudaMemcpyDeviceToDevice, st));
-                CK(cudaStreamSynchronize(st));   // idx (host vector) has been consumed
-                const uint32_t mode = h->scan_mode;
-                h->scan_mode = FVDB_SCAN_EXACT;
-                // (a split batch: t_ids / t_dist / t_cnt are the packed layout, its IVF part follows; the
-                // buffer holds 4 m k + 2 m words, two such parts)
-                const int r3 = search_device_impl(h, h->s_fb_q.p, m, pb.k, pb.nprobe, pb.tiers, pb.d_filter, pb.filter_bits,
-                                                  t_ids, t_dist, t_cnt, st, nullptr, nullptr, false, false, nullptr, pb.split);
-                h->scan_mode = mode;
-                if (r3 != FVDB_OK) return r3;
-                const uint32_t* fb_rows = reinterpret_cast<const uint32_t*>(h->s_fb_coarse.p);
-                CK(launch_scatter_result_rows(t_ids, t_dist, t_cnt, fb_rows, m, pb.k, pb.d_out_ids, pb.d_out_dist,
-                                              pb.d_out_count, st));
-                if (pb.split) {
-                    const size_t tp = (size_t)2 * m * pb.k + m, bp = (size_t)2 * pb.nq * pb.k + pb.nq;
-                    CK(launch_scatter_result_rows(t_ids + tp, t_dist + tp, t_cnt + tp, fb_rows, m, pb.k, pb.d_out_ids + bp,
-                                                  pb.d_out_dist + bp, pb.d_out_count + bp, st));
-                }
-                if (pb.ho_ids) {
-                    const HostOut ho2{pb.ho_ids, pb.ho_dist, pb.ho_cnt, (size_t)pb.nq * pb.k * 4, (size_t)pb.nq * 4};
-                    CK(copy_out(&ho2, pb.d_out_ids, pb.d_out_dist, pb.d_out_count, st));
-                }
-                CK(cudaStreamSynchronize(st));
-                return FVDB_OK;
-            }();
-            if (r2 != FVDB_OK) rc = r2;
-            fallbacks += m;
+            const std::vector<uint32_t> rows = failed_queries(host + 16, n_ivf, host + 16 + 2 * pb.nq, n_flat);
+            const int r = repair_rows(h, pb, rows, st);
+            if (r != FVDB_OK) rc = r;
+            fallbacks += (uint32_t)rows.size();
         }
     }
-    for (const fvdb_index::Pending& pb : todo) h->pending_pool.push_back({pb.host, pb.host_words});
+    for (const fvdb_index::Pending& pb : todo) h->pending_pool.push_back(pb.rec);
     for (auto& rec : h->pending_coarse) {
         if (rc == FVDB_OK && rec.first[0])
             rc = h->fail(FVDB_ERR_NAN, "NaN in query (the reference panics on partial_cmp().unwrap())");
@@ -1892,22 +1892,7 @@ static int finish_pending(fvdb_index* h, cudaStream_t st) {
         h->pending_pool.push_back(rec);
     }
     h->pending_coarse.clear();
-    if (todo.empty()) h->stats.last_fallback_queries = fallbacks;
-    if (!todo.empty()) {
-        const fvdb_index::Pending& lb = todo.back();   // the figures of the last batch, as the synchronous call reports them
-        uint64_t scanned = 0;
-        std::memcpy(&scanned, &lb.host[2], 8);
-        const uint64_t rows = scanned + (lb.use_flat ? h->flat_n : 0);
-        h->stats.last_nq = lb.nq;
-        h->stats.last_scanned_rows = rows;
-        h->stats.last_algorithmic_bytes = rows * h->dim * 4ull + (uint64_t)lb.nq * h->dim * 4ull + (uint64_t)lb.nq * lb.k * 8ull +
-                                          (lb.use_ivf ? (uint64_t)h->nlist * h->dim * 4ull : 0ull) + (uint64_t)lb.n_bitmaps * (rows / 8);
-        h->stats.last_fallback_queries = fallbacks;
-        float ms = 0.f;
-        const fvdb_index::Slot* ls = lb.slot >= 0 ? &h->slots[lb.slot] : nullptr;
-        if (cudaEventElapsedTime(&ms, ls ? ls->ev_a : h->ev_a, ls ? ls->ev_b : h->ev_b) == cudaSuccess) h->stats.last_device_ms = ms; else cudaGetLastError();
-        if (cudaEventElapsedTime(&ms, ls ? ls->ev_s0 : h->ev_s0, ls ? ls->ev_s1 : h->ev_s1) == cudaSuccess) h->stats.last_scan_ms = ms; else cudaGetLastError();
-    }
+    h->stats.last_fallback_queries = fallbacks;
     return rc;
 }
 
@@ -1940,8 +1925,9 @@ int fvdb_search_device_coarse_submit(fvdb_index* h, const float* d_q, uint32_t n
         return h->fail(FVDB_ERR_INVALID_ARG, "coarse keys are [nq x nprobe]: nprobe must not exceed nlist");
     if (h->pending.size() >= 64) return h->fail(FVDB_ERR_INVALID_ARG, "64 batches are pending: call fvdb_search_device_finish");
     cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
+    SearchOpts o; o.ext_coarse = d_coarse_keys; o.deferred = true;
     return search_device_impl(h, d_q, nq, k, nprobe, tiers, d_filter_bits, filter_nbits, d_out_ids,
-                              d_out_dist, d_out_count, st, d_coarse_keys, nullptr, true, true);
+                              d_out_dist, d_out_count, st, o);
 }
 
 // Device-side join: `stream` waits for the batch submitted `age` submits ago (0 = the latest).
@@ -1962,8 +1948,9 @@ int fvdb_search_device_coarse(fvdb_index* h, const float* d_q, uint32_t nq, uint
     if (d_coarse_keys && nprobe > h->nlist)
         return h->fail(FVDB_ERR_INVALID_ARG, "coarse keys are [nq x nprobe]: nprobe must not exceed nlist");
     cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
+    SearchOpts o; o.ext_coarse = d_coarse_keys;
     return search_device_impl(h, d_q, nq, k, nprobe, tiers, d_filter_bits, filter_nbits, d_out_ids,
-                              d_out_dist, d_out_count, st, d_coarse_keys);
+                              d_out_dist, d_out_count, st, o);
 }
 
 // fvdb_search_device_coarse / _coarse_submit with the tiers kept apart: one flag through search_device_impl,
@@ -1980,9 +1967,9 @@ static int search_device_tiers_common(fvdb_index* h, const float* d_q, uint32_t 
         return h->fail(FVDB_ERR_INVALID_ARG, "64 batches are pending: call fvdb_search_device_finish");
     cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
     const size_t nk = (size_t)nq * k;
+    SearchOpts o; o.ext_coarse = d_coarse_keys; o.deferred = submit; o.split = true;
     return search_device_impl(h, d_q, nq, k, nprobe, tiers, d_filter_bits, filter_nbits, d_out_pack,
-                              reinterpret_cast<float*>(d_out_pack + nk), d_out_pack + 2 * nk, st, d_coarse_keys,
-                              nullptr, submit, submit, nullptr, true);
+                              reinterpret_cast<float*>(d_out_pack + nk), d_out_pack + 2 * nk, st, o);
 }
 
 int fvdb_search_device_tiers(fvdb_index* h, const float* d_q, uint32_t nq, uint32_t k, uint32_t nprobe,
@@ -2040,8 +2027,9 @@ int search_host_locked(fvdb_index* h, const float* q, uint32_t nq, uint32_t k, u
     HostOut ho{out_pinned ? (void*)out_ids : (void*)pin, out_pinned ? (void*)out_dist : (void*)(pin + ob),
                out_pinned ? (void*)out_count : (void*)(pin + 2 * ob), ob, cb};
     // the result copies are enqueued in front of the batch's one synchronisation point
+    SearchOpts o; o.ho = &ho;
     RET(search_device_impl(h, h->s_q.p, nq, k, nprobe, tiers, d_filter, filter_nbits, h->s_out_ids.p,
-                           h->s_out_dist.p, h->s_out_cnt.p, st, nullptr, &ho));
+                           h->s_out_dist.p, h->s_out_cnt.p, st, o));
     if (!out_pinned) {
         std::memcpy(out_ids, pin, ob);
         std::memcpy(out_dist, pin + ob, ob);
@@ -2082,8 +2070,9 @@ void run_coalesced(fvdb_index* h, std::vector<SearchReq*>& batch) {
         CK(cudaMemcpyAsync(h->s_q.p, h->pin, qb, cudaMemcpyHostToDevice, st));
         char* pin = (char*)h->pin;
         HostOut ho{pin, pin + ob, pin + 2 * ob, ob, cb};
+        SearchOpts o; o.ho = &ho;
         RET(search_device_impl(h, h->s_q.p, (uint32_t)total, k, batch[0]->nprobe, batch[0]->tiers, nullptr, 0,
-                               h->s_out_ids.p, h->s_out_dist.p, h->s_out_cnt.p, st, nullptr, &ho));
+                               h->s_out_ids.p, h->s_out_dist.p, h->s_out_cnt.p, st, o));
         size_t row = 0;
         for (SearchReq* r : batch) {
             std::memcpy(r->out_ids, pin + row * k * 4, (size_t)r->nq * k * 4);
@@ -2247,8 +2236,8 @@ int fvdb_ivf_max_sqnorm(fvdb_index* h, float* out) {
     if (h->ivf_n == 0) return FVDB_OK;
     cudaStream_t st = h->stream;
     CK(h->s_f32a.ensure(h->ivf_n, 0, st, &h->dev_bytes));
-    CK(h->s_misc.ensure(64, 0, st, &h->dev_bytes));
-    uint32_t* d_max = h->s_misc.p + 13;
+    CK(h->scratch.misc.ensure(64, 0, st, &h->dev_bytes));
+    uint32_t* d_max = h->scratch.misc.p + 13;
     CK(cudaMemsetAsync(d_max, 0, 4, st));
     CK(launch_max_sqnorm(h->ivf_rows.p, h->ivf_n, h->dim, h->s_f32a.p, d_max, st));
     uint32_t bits = 0;
