@@ -1365,7 +1365,7 @@ int fvdb_set_option(fvdb_index* h, int option, uint64_t value) {
     switch (option) {
         case FVDB_OPT_SCAN_MODE:
             if (value == FVDB_SCAN_TC && !tc_supported(h->dim))
-                return h->fail(FVDB_ERR_INVALID_CONFIG, "tensor-core scan needs dim % 32 == 0 and dim <= 512");
+                return h->fail(FVDB_ERR_INVALID_CONFIG, "tensor-core scan needs dim % 32 == 0 and 32 <= dim <= 2048");
             if (value > FVDB_SCAN_TC) return h->fail(FVDB_ERR_INVALID_ARG, "unknown scan mode");
             h->scan_mode = (uint32_t)value;
             return FVDB_OK;

@@ -99,9 +99,11 @@ using namespace tcx;
 //               stores) as soon as the MMA warp has retired the current item.
 // ================================================================================================
 constexpr int R2_ROWS = 128;                     // rows per tile (MMA M = TMEM lanes)
-constexpr int R2_NQ = (int)TC_TILE_Q;            // queries per item (MMA N max)
 constexpr int R2_STAGE_BYTES = R2_ROWS * 128;    // 16 KB: 128 rows x one 128-byte k-block
-constexpr int R2_QBLK_BYTES = R2_NQ * 128;       // 8 KB per k-block of the query tile
+// Queries per item (the kernel's template parameter NQ, MMA N max) by dimension: the query tile,
+// KB x NQ x 128 B, stays resident for the whole item, so the width halves as D doubles past 512 and
+// the tile never exceeds the 128 KB it takes at D = 512 (a 64-query tile of D = 1024 would need 256 KB)
+constexpr uint32_t r2_tile_q(uint32_t D) { return D <= 512 ? TC_TILE_Q : D <= 1024 ? 32u : 16u; }
 #ifndef FVDB_R2_CAP
 #define FVDB_R2_CAP 32
 #endif
@@ -116,54 +118,54 @@ constexpr int R2_QBLK_BYTES = R2_NQ * 128;       // 8 KB per k-block of the quer
 #endif
 constexpr int R2_CAP = FVDB_R2_CAP;              // pending candidates per query (<= 32: one sorting network)
 constexpr int R2_FLUSH = FVDB_R2_FLUSH;          // merge a query once it holds more pending than this
-constexpr int R2_NBUF = 8;                       // accumulator buffers of R2_NQ columns
+constexpr int R2_NBUF = 8;                       // accumulator buffers of NQ columns
 constexpr int R2_NSLOT = FVDB_R2_NSLOT;          // |x|^2 strips in flight
 constexpr int R2_SLACK = FVDB_R2_SLACK;          // bytes reserved for aligning the dynamic shared memory to 1024 (0: trap if it is not)
 static_assert(R2_CAP <= 32 && R2_FLUSH < R2_CAP && R2_NSLOT > R2_NBUF + 2, "kernel R pools");
 constexpr int R2_THREADS = 320;
 constexpr uint32_t TC_SPLIT_MAX = 4;          // row ranges a long posting list is split into, at most
 constexpr uint32_t TC_SPLIT_MIN_ROWS = 2048;  // lists up to this length are never split
-constexpr int R2_TMEM_COLS = 512;
 
 struct R2Smem {
-    unsigned char* q_tile;    // KB x 8 KB, 128B-swizzled K-major [query][32 floats]
+    unsigned char* q_tile;    // KB x NQ x 128 B, 128B-swizzled K-major [query][32 floats]
     unsigned char* ring;      // STAGES x 16 KB
-    uint64_t* sorted;         // [R2_NQ][TC_KP]  ascending approx keys of this item
-    uint64_t* pend;           // [R2_NQ][R2_CAP] unsorted pending candidates
+    uint64_t* sorted;         // [NQ][TC_KP]  ascending approx keys of this item
+    uint64_t* pend;           // [NQ][R2_CAP] unsorted pending candidates
     float* xn_ring;           // [R2_NSLOT][R2_ROWS]
-    float* thrp;              // [R2_NQ] threshold - |q|^2   (-inf for padded columns)
-    uint32_t* pcnt;           // [2][R2_NQ] pending count (may exceed the capacity: overflow marker)
-    uint32_t* qidx;           // [2][R2_NQ]
-    uint32_t* qslot;          // [2][R2_NQ]
-    float* qn;                // [2][R2_NQ]
+    float* thrp;              // [NQ] threshold - |q|^2   (-inf for padded columns)
+    uint32_t* pcnt;           // [2][NQ] pending count (may exceed the capacity: overflow marker)
+    uint32_t* qidx;           // [2][NQ]
+    uint32_t* qslot;          // [2][NQ]
+    float* qn;                // [2][NQ]
     uint32_t* redo;           // [8] bitmask of queries to replay ([half][round parity][2] with offloaded merges)
     uint64_t* bars;
     uint32_t* tmem_ptr;
     uint32_t* sched;          // [TC_SCHED]
 };
 
+template <int NQ>
 __device__ __forceinline__ R2Smem r2_carve(unsigned char* smem, uint32_t KB, uint32_t STAGES) {
     R2Smem m;
     m.q_tile = smem;
-    m.ring = m.q_tile + (size_t)KB * R2_QBLK_BYTES;
+    m.ring = m.q_tile + (size_t)KB * NQ * 128;
     m.sorted = reinterpret_cast<uint64_t*>(m.ring + (size_t)STAGES * R2_STAGE_BYTES);
-    m.pend = m.sorted + R2_NQ * TC_KP;
-    m.xn_ring = reinterpret_cast<float*>(m.pend + R2_NQ * R2_CAP);
+    m.pend = m.sorted + NQ * TC_KP;
+    m.xn_ring = reinterpret_cast<float*>(m.pend + NQ * R2_CAP);
     m.thrp = m.xn_ring + R2_NSLOT * R2_ROWS;
-    m.pcnt = reinterpret_cast<uint32_t*>(m.thrp + R2_NQ);
-    m.qidx = m.pcnt + 2 * R2_NQ;
-    m.qslot = m.qidx + 2 * R2_NQ;
-    m.qn = reinterpret_cast<float*>(m.qslot + 2 * R2_NQ);
-    m.redo = reinterpret_cast<uint32_t*>(m.qn + 2 * R2_NQ);
+    m.pcnt = reinterpret_cast<uint32_t*>(m.thrp + NQ);
+    m.qidx = m.pcnt + 2 * NQ;
+    m.qslot = m.qidx + 2 * NQ;
+    m.qn = reinterpret_cast<float*>(m.qslot + 2 * NQ);
+    m.redo = reinterpret_cast<uint32_t*>(m.qn + 2 * NQ);
     m.bars = reinterpret_cast<uint64_t*>(m.redo + 8);
     m.tmem_ptr = reinterpret_cast<uint32_t*>(m.bars + 2 * STAGES + 2 * R2_NBUF + R2_NSLOT + 2 * TC_SCHED + 8);
     m.sched = m.tmem_ptr + 1;
     return m;
 }
 
-size_t tc_scan_smem_bytes(uint32_t KB, uint32_t stages) {
-    return (size_t)KB * R2_QBLK_BYTES + (size_t)stages * R2_STAGE_BYTES + (size_t)R2_NQ * TC_KP * 8 +
-           (size_t)R2_NQ * R2_CAP * 8 + (size_t)R2_NSLOT * R2_ROWS * 4 + (size_t)R2_NQ * 9 * 4 + 32 +
+size_t tc_scan_smem_bytes(uint32_t KB, uint32_t stages, uint32_t NQ) {
+    return (size_t)KB * NQ * 128 + (size_t)stages * R2_STAGE_BYTES + (size_t)NQ * TC_KP * 8 +
+           (size_t)NQ * R2_CAP * 8 + (size_t)R2_NSLOT * R2_ROWS * 4 + (size_t)NQ * 9 * 4 + 32 +
            (size_t)(2 * stages + 2 * R2_NBUF + R2_NSLOT + 2 * TC_SCHED + 8) * 8 + 16 + (size_t)TC_SCHED * 4;
 }
 
@@ -221,15 +223,19 @@ __device__ __forceinline__ void publish_bound(const TcScanParams& p, uint32_t qi
 #define Q1_LAP(i) do { if (p.prof) { const long long n_ = clock64(); lap[i] += (unsigned long long)(n_ - tl); tl = n_; } } while (0)
 #define Q1_LAP_DUMP(role) do { if (p.prof && lane == 0) { for (int i_ = 0; i_ < 8; ++i_) p.prof[((size_t)blockIdx.x * 6 + (role)) * 8 + i_] = lap[i_]; } } while (0)
 
+template <int NQ>   // queries per item: r2_tile_q(D)
 __global__ void __launch_bounds__(R2_THREADS, 1)
 tc_scan_kernel(const __grid_constant__ CUtensorMap tmap, const TcScanParams p) {
+    static_assert(NQ == 16 || NQ == 32 || NQ == 64, "kind::tf32 with M = 128 and one 16-column epilogue chunk");
+    constexpr int QBLK_BYTES = NQ * 128;          // one k-block of the query tile (a multiple of the 1 KB swizzle atom)
+    constexpr uint32_t TMEM_COLS = R2_NBUF * NQ;  // a power of two >= 32, as tcgen05.alloc needs
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     // SWIZZLE_128B tiles need 1024-byte alignment; the launch reserves 1 KB of slack for this
     unsigned char* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
     if (R2_SLACK < 1024 && smem != smem_raw) __trap();   // built without slack: the declared alignment must hold
     const uint32_t KB = p.KB;
     const uint32_t STAGES = p.stages;
-    const R2Smem sm = r2_carve(smem, KB, STAGES);
+    const R2Smem sm = r2_carve<NQ>(smem, KB, STAGES);
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t bar_full = smem_u32(sm.bars);
@@ -265,7 +271,7 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap tmap, const TcScanParams p) {
     }
     if (warp == 1) {
         asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(sm.tmem_ptr)),
-                     "r"((uint32_t)R2_TMEM_COLS)
+                     "r"(TMEM_COLS)
                      : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
@@ -380,7 +386,7 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap tmap, const TcScanParams p) {
                 mbar_wait(bar_tempty + 8 * buf, ((tile / R2_NBUF) & 1u) ^ 1u);
                 tc_fence_after();
                 Q1_LAP(2);
-                const uint32_t d_tmem = tmem_base + buf * R2_NQ;
+                const uint32_t d_tmem = tmem_base + buf * NQ;
                 const bool last_tile = rt + R2_ROWS >= it.row_end;
                 for (uint32_t kb = 0; kb < KB; ++kb) {
                     Q1_LAP(4);
@@ -389,7 +395,7 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap tmap, const TcScanParams p) {
                     Q1_LAP(3);
                     if (elect_one()) {
                         const uint64_t a0 = umma_desc_sw128(ring_base + stage * R2_STAGE_BYTES);
-                        const uint64_t b0 = umma_desc_sw128(q_base + kb * R2_QBLK_BYTES);
+                        const uint64_t b0 = umma_desc_sw128(q_base + kb * QBLK_BYTES);
 #pragma unroll
                         for (uint32_t k4 = 0; k4 < 4; ++k4)  // UMMA_K = 8 tf32 = 32 bytes = +2 in the descriptor
                             if (!(p.debug & 8u) && (!(p.debug & 16u) || k4 == 0))   // timing experiments: no / a quarter of the MMAs
@@ -442,11 +448,17 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap tmap, const TcScanParams p) {
             if (nit >= 2) mbar_wait(bar_mfree, nit & 1u);
             Q1_LAP(1);
             if (lw == 0) {
-                const uint32_t mb = (nit & 1u) * R2_NQ;
-                sm.qidx[mb + lane] = qi0; sm.qidx[mb + 32 + lane] = qi1;
-                sm.qslot[mb + lane] = sl0; sm.qslot[mb + 32 + lane] = sl1;
-                sm.qn[mb + lane] = (qi0 != ID_NONE) ? p.qnorm[qi0] : 0.f;
-                sm.qn[mb + 32 + lane] = (qi1 != ID_NONE) ? p.qnorm[qi1] : 0.f;
+                const uint32_t mb = (nit & 1u) * NQ;
+                if (lane < NQ) {
+                    sm.qidx[mb + lane] = qi0;
+                    sm.qslot[mb + lane] = sl0;
+                    sm.qn[mb + lane] = (qi0 != ID_NONE) ? p.qnorm[qi0] : 0.f;
+                }
+                if (NQ > 32) {
+                    sm.qidx[mb + 32 + lane] = qi1;
+                    sm.qslot[mb + 32 + lane] = sl1;
+                    sm.qn[mb + 32 + lane] = (qi1 != ID_NONE) ? p.qnorm[qi1] : 0.f;
+                }
             }
             // the query tile may be overwritten once every MMA of the previous item has retired
             Q1_LAP(3);
@@ -483,7 +495,7 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap tmap, const TcScanParams p) {
                             for (int g = 0; g < 4; ++g) {
                                 const uint32_t q = q0 + 4 * g;
                                 if (q < ncols)
-                                    *reinterpret_cast<float4*>(sm.q_tile + (size_t)kb * R2_QBLK_BYTES + q * 128 +
+                                    *reinterpret_cast<float4*>(sm.q_tile + (size_t)kb * QBLK_BYTES + q * 128 +
                                                                ((ch ^ (q & 7)) << 4)) = v[u][g];
                             }
                         }
@@ -523,7 +535,7 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap tmap, const TcScanParams p) {
             if (it.pair_count == 0 || it.row_begin >= it.row_end) continue;
             const uint32_t cnt = it.pair_count;
             const uint32_t ncols = (cnt + 15u) & ~15u;
-            const uint32_t mb = (nit & 1u) * R2_NQ;
+            const uint32_t mb = (nit & 1u) * NQ;
             mbar_wait(bar_qready, nit & 1u);           // metadata of this item is staged
             Q1_LAP(1);
             if (nit >= 1) {                            // ... and only now release the previous item's
@@ -531,7 +543,7 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap tmap, const TcScanParams p) {
                 if (lane == 0) mbar_arrive(bar_mfree);
             }
             // ---- item prologue: empty shortlists, thresholds from the shared bounds ----
-            if (et < R2_NQ) {
+            if (et < NQ) {
                 float thr = -__uint_as_float(F32_INF_BITS);  // padded columns never pass
                 if ((uint32_t)et < cnt) {
                     const uint32_t g = p.thr_g ? *(volatile uint32_t*)(p.thr_g + sm.qidx[mb + et]) : (uint32_t)0x7f800000u;
@@ -541,7 +553,7 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap tmap, const TcScanParams p) {
                 sm.pcnt[et] = 0;
             }
             if (et < 2) sm.redo[et] = 0;
-            for (int i = et; i < R2_NQ * TC_KP; i += 128) sm.sorted[i] = KEY_NONE;
+            for (int i = et; i < NQ * TC_KP; i += 128) sm.sorted[i] = KEY_NONE;
             const bool own = lane < 16 && jown < cnt;
             const uint32_t qi_own = own ? sm.qidx[mb + jown] : 0u;
             const float qn_own = own ? sm.qn[mb + jown] : 0.f;
@@ -622,7 +634,7 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap tmap, const TcScanParams p) {
                 mbar_wait(bar_tfull + 8 * buf, (tile / R2_NBUF) & 1u);
                 tc_fence_after();
                 Q1_LAP(2);
-                const uint32_t taddr = tmem_base + buf * R2_NQ + lane_taddr;
+                const uint32_t taddr = tmem_base + buf * NQ + lane_taddr;
                 const uint32_t pos = rt + (uint32_t)trow;
                 uint64_t ovf = 0;  // queries whose pending list was full when this row passed
 
@@ -759,7 +771,7 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap tmap, const TcScanParams p) {
     if (warp == 1) {
         tc_fence_after();
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base),
-                     "r"((uint32_t)R2_TMEM_COLS)
+                     "r"(TMEM_COLS)
                      : "memory");
     }
 }
@@ -1245,6 +1257,18 @@ __device__ __forceinline__ float exact_l2_lane_gather(const float* __restrict__ 
     return (na == 0.0f || nb == 0.0f) ? 0.0f : __fdiv_rn(acc, __fmul_rn(na, nb));
 }
 
+// Bound on |approximate d2 - exact d2| for a D-dimensional pair (DESIGN §3.1): qn = |q|, xmax = the largest |x|
+// of the row set, a = the approximate d2.  The absolute term covers the TF32 operands (2^-10 relative each, 2^-8
+// |q| |x| on 2 x.q) and the fp32 sums of D terms on the tensor cores and in the norms (2 D 2^-24 |q| |x|, within
+// the 5 % margin up to D = 1638); the relative term covers the reference's sequential fp32 sum of D squared
+// differences ((D + 2) 2^-24 relative, rounded up to D + 4).  For D <= 512 both are the constants
+// 1.05 * 2^-8 and 3.1e-5, so the proofs of those shapes are unchanged bit for bit.
+__device__ __forceinline__ float tc_proof_eps(uint32_t D, float qn, float xmax, float a) {
+    const float c_abs = fmaxf(1.05f * 0.00390625f, 0.00390625f + (float)(2u * D) * 0x1p-24f);
+    const float c_rel = fmaxf(3.1e-5f, (float)(D + 4u) * 0x1p-24f);
+    return c_abs * qn * xmax + c_rel * a + 1e-30f;
+}
+
 // Exact re-rank + proof.  One warp per query, lane = shortlist entry.  Distances are recomputed
 // as euclidean_distance_scalar does (sequential f32, (q - x)^2, no FMA, sqrt), so the returned
 // keys are bit-identical to the exact path.  Proof: every row outside the shortlist has
@@ -1282,7 +1306,7 @@ __global__ void __launch_bounds__(128) rerank_kernel(const uint64_t* __restrict_
             const float a0 = __uint_as_float((uint32_t)(k0 >> 32));
             const float a1 = k1 != KEY_NONE ? __uint_as_float((uint32_t)(k1 >> 32)) : __uint_as_float(0x7f800000u);
             const float xmax = sqrtf(fmaxf(__uint_as_float(*xmax_bits), xmax_floor_sq));
-            const float eps = 1.05f * 0.00390625f * sqrtf(qnorm[q]) * xmax + 3.1e-5f * a1 + 1e-30f;
+            const float eps = tc_proof_eps(D, sqrtf(qnorm[q]), xmax, a1);
             if (a1 - a0 > 2.02f * eps) {
                 const uint32_t pos0 = (uint32_t)k0;
                 if (lane == 0) out_keys[(size_t)q * k] = make_key(sqrtf(a0), ids ? ids[pos0] : pos0);
@@ -1323,7 +1347,7 @@ __global__ void __launch_bounds__(128) rerank_kernel(const uint64_t* __restrict_
         // xmax_floor_sq: list-sharded search with shared bounds — a row of THIS shard may have been
         // dropped by a bound a peer published, so every shard has to use the same (largest) norm term
         const float xmax = sqrtf(fmaxf(__uint_as_float(*xmax_bits), xmax_floor_sq));
-        const float eps = 1.05f * 0.00390625f * sqrtf(qnorm[q]) * xmax + 3.1e-5f * a_last + 1e-30f;
+        const float eps = tc_proof_eps(D, sqrtf(qnorm[q]), xmax, a_last);
         bool ok = false;
         if (kth != KEY_NONE) {
             if (METRIC == METRIC_L2) {
@@ -1375,7 +1399,7 @@ __global__ void coarse_items_kernel(ScanItem* items, uint32_t nq, uint32_t nlist
     items[i] = it;
 }
 
-// identity work items of the flat-tier scan: (query group of TC_TILE_Q) x (row chunk); `slot` = chunk
+// identity work items of the flat-tier scan: (query group of tile_q) x (row chunk); `slot` = chunk
 // index = the partial slot the item's shortlists are published to
 __global__ void flat_items_kernel(ScanItem* items, uint32_t nq, uint32_t n_rows, uint32_t chunk_rows,
                                   uint32_t n_chunks, uint32_t* n_items, uint32_t tile_q) {
@@ -1599,7 +1623,7 @@ __global__ void __launch_bounds__(128) coarse_select_kernel(const float* __restr
         else if (next_d2 != 0xFFFFFFFFu) {
             const float a_next = __uint_as_float(next_d2);
             const float cmax = sqrtf(__uint_as_float(*cmax_bits));
-            const float eps = 1.05f * 0.00390625f * sqrtf(qnorm[q]) * cmax + 3.1e-5f * a_next + 1e-30f;
+            const float eps = tc_proof_eps(D, sqrtf(qnorm[q]), cmax, a_next);
             ok = false;
             if (kth != KEY_NONE) {
                 const float dk = key_dist(kth);
@@ -1824,7 +1848,7 @@ struct TcScratchImpl {
     bool smem_attr_set_q = false;
     const float* tmap_rows = nullptr;
     uint64_t tmap_n = 0;
-    bool smem_attr_set = false;
+    uint32_t smem_attr_set_r = 0;   // bit per item width of kernel R
     bool smem_attr_set_rerank = false;
     // experiment (FVDB_TC_FORK=1): kernel W of an IVF batch on a side stream, forked behind the bucketing and joined
     // before the shortlist merge: its CTA pairs start wherever kernel R's CTAs have left an SM pair, instead of
@@ -1833,7 +1857,7 @@ struct TcScratchImpl {
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
 };
 
-bool tc_supported(uint32_t D) { return D % 32 == 0 && D >= 32 && D <= 512; }
+bool tc_supported(uint32_t D) { return D % 32 == 0 && D >= 32 && D <= TC_MAX_D; }
 
 static size_t rerank_smem_bytes(uint32_t D) { return (size_t)4 * gather_warp_bytes(GATHER_STAGES_ROWS) + (size_t)4 * D * sizeof(float); }
 static size_t coarse_select_smem_bytes(uint32_t D, uint32_t KC) {
@@ -1841,10 +1865,10 @@ static size_t coarse_select_smem_bytes(uint32_t D, uint32_t KC) {
 }
 static cudaError_t rerank_prepare(TcScratchImpl* m) {
     if (m->smem_attr_set_rerank) return cudaSuccess;
-    cudaError_t e = cudaFuncSetAttribute(rerank_kernel<METRIC_L2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rerank_smem_bytes(512));
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(rerank_kernel<METRIC_COS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rerank_smem_bytes(512));
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(rerank_kernel<METRIC_DOT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rerank_smem_bytes(512));
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(coarse_select_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)coarse_select_smem_bytes(512, 128));
+    cudaError_t e = cudaFuncSetAttribute(rerank_kernel<METRIC_L2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rerank_smem_bytes(TC_MAX_D));
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(rerank_kernel<METRIC_COS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rerank_smem_bytes(TC_MAX_D));
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(rerank_kernel<METRIC_DOT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rerank_smem_bytes(TC_MAX_D));
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(coarse_select_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)coarse_select_smem_bytes(TC_MAX_D, 128));
     if (e == cudaSuccess) m->smem_attr_set_rerank = true;
     return e;
 }
@@ -1876,7 +1900,7 @@ void tc_release(TcScratch& s) {
 
 // Which scan kernel(s): 'W' = kernel W for heavily probed lists and dense scans plus kernel R for the
 // sparsely probed lists (needs the query tile in tensor memory: D <= 384); 'R' (FVDB_TC_KERNEL=R, or
-// 384 < D <= 512) = kernel R alone
+// 384 < D <= TC_MAX_D) = kernel R alone
 static char tc_kernel_choice(uint32_t D, int sm_count) {
     const char* kenv = getenv("FVDB_TC_KERNEL");
     char c = (kenv && kenv[0] == 'R') ? 'R' : 'W';
@@ -1929,6 +1953,31 @@ static cudaError_t launch_wide(TcScratchImpl* m, const CUtensorMap& tmap, TcScan
     if (e != cudaSuccess) return e;
     if (p.prof) return dump_prof(m->prof.p, grid, st);
     return cudaSuccess;
+}
+
+// Kernel R at the item width of D, with the deepest ring that fits; the norm-strip window (see the producer)
+// caps the ring at 6 tiles.  *smem = 0 when not even two stages fit.
+static uint32_t r2_pick_stages(uint32_t D, size_t* smem) {
+    const uint32_t KB = D / 32, nq = r2_tile_q(D);
+    uint32_t stages = std::min<uint32_t>(12u, (uint32_t)(R2_NSLOT - 2 - R2_NBUF) * KB);
+    while (stages > 2 && tc_scan_smem_bytes(KB, stages, nq) + R2_SLACK > 232448) --stages;
+    *smem = tc_scan_smem_bytes(KB, stages, nq) + R2_SLACK;   // slack for the 1024-byte alignment
+    if (*smem > 232448) *smem = 0;
+    return stages;
+}
+
+static cudaError_t launch_r2(TcScratchImpl* m, const CUtensorMap& tmap, const TcScanParams& p, uint32_t grid, size_t smem,
+                             cudaStream_t st) {
+    const uint32_t nq = r2_tile_q(p.D);
+    auto kern = nq == 64 ? tc_scan_kernel<64> : nq == 32 ? tc_scan_kernel<32> : tc_scan_kernel<16>;
+    const uint32_t bit = nq / 16;
+    if (!(m->smem_attr_set_r & bit)) {
+        const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
+        if (e != cudaSuccess) return e;
+        m->smem_attr_set_r |= bit;
+    }
+    kern<<<grid, R2_THREADS, smem, st>>>(tmap, p);
+    return cudaGetLastError();
 }
 
 static CUresult encode_rows_tmap(CUtensorMap* out, const float* rows, uint64_t n_rows, uint32_t D, uint32_t box_rows) {
@@ -2008,7 +2057,7 @@ int tc_ivf_search(TcScratch& s, const TcSearchArgs& a, cudaStream_t st, size_t* 
     // Two scan kernels share a batch.  Kernel W (wide query tiles on CTA pairs, queries in tensor
     // memory: D <= 384) takes the lists probed by at least `wide_min` queries: a row enters one SM once
     // per 256 queries, and with many live queries per warp its thread-per-query epilogue runs lane-
-    // parallel.  Kernel R (64-query items, query tile in shared memory, rows on the accumulator lanes,
+    // parallel.  Kernel R (items of up to 64 queries, query tile in shared memory, rows on the accumulator lanes,
     // candidate handling shared by the 128 row threads) takes the sparsely probed lists, where its MMA
     // cost (proportional to the queries of the item) and its cooperative epilogue are the cheaper ones.
     const char kch = tc_kernel_choice(D, a.sm_count);
@@ -2018,7 +2067,7 @@ int tc_ivf_search(TcScratch& s, const TcSearchArgs& a, cudaStream_t st, size_t* 
         if (const char* e = getenv("FVDB_TC_WIDE_MIN")) wide_min = (uint32_t)std::max(1, atoi(e));
     }
     const bool use_wide = wide_min != 0;
-    const uint32_t tile_q = TC_TILE_Q;
+    const uint32_t tile_q = r2_tile_q(D);   // kernel R's items; a list probed by more queries becomes several
     // Long posting lists are cut into row ranges (one work item and one shortlist slot each): a hub
     // list of 9 K rows probed by 64 queries is otherwise ONE item of 71 tiles — a third of the whole
     // scan on one SM, and the tail every other SM waits for.  At most TC_SPLIT_MAX ranges per list.
@@ -2193,17 +2242,14 @@ int tc_ivf_search(TcScratch& s, const TcSearchArgs& a, cudaStream_t st, size_t* 
     };
     auto run_narrow = [&]() -> int {
     {
-        // deepest ring that fits; the norm-strip window (see the producer) caps it at 6 tiles
-        uint32_t stages = std::min<uint32_t>(12u, (uint32_t)(R2_NSLOT - 2 - R2_NBUF) * KB);
-        while (stages > 2 && tc_scan_smem_bytes(KB, stages) + R2_SLACK > 232448) --stages;
-        if (const char* e = getenv("FVDB_TC_STAGES")) { const uint32_t v = (uint32_t)atoi(e); if (v >= 2 && v < stages) stages = v; }
-        p.stages = stages;
-        const size_t smem = tc_scan_smem_bytes(KB, stages) + R2_SLACK;  // slack for the 1024-byte alignment
-        if (smem > 232448) { if (err) *err = "TC scan does not fit shared memory for this dim"; return FVDB_ERR_INVALID_CONFIG; }
-        if (!m->smem_attr_set) {
-            TCK(cudaFuncSetAttribute(tc_scan_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
-            m->smem_attr_set = true;
+        size_t smem = 0;
+        uint32_t stages = r2_pick_stages(D, &smem);
+        if (!smem) { if (err) *err = "TC scan does not fit shared memory for this dim"; return FVDB_ERR_INVALID_CONFIG; }
+        if (const char* e = getenv("FVDB_TC_STAGES")) {
+            const uint32_t v = (uint32_t)atoi(e);
+            if (v >= 2 && v < stages) { stages = v; smem = tc_scan_smem_bytes(KB, stages, tile_q) + R2_SLACK; }
         }
+        p.stages = stages;
         uint32_t grid = (uint32_t)std::min<size_t>((size_t)a.sm_count, max_items);
         if (p.scan_sms && p.scan_sms < grid) grid = p.scan_sms;
         if (p.debug & 128u) {
@@ -2211,8 +2257,7 @@ int tc_ivf_search(TcScratch& s, const TcSearchArgs& a, cudaStream_t st, size_t* 
             TCK(cudaMemsetAsync(m->prof.p, 0, (size_t)grid * 48 * 8, st));
             p.prof = m->prof.p;
         }
-        tc_scan_kernel<<<grid, R2_THREADS, smem, st>>>(m->tmap_arena, p);
-        TCK(cudaGetLastError());
+        TCK(launch_r2(m, m->tmap_arena, p, grid, smem, st));
         if (p.prof) TCK(dump_prof(m->prof.p, grid, st));
     }
     return FVDB_OK;
@@ -2280,7 +2325,7 @@ int tc_flat_search(TcScratch& s, const TcFlatArgs& a, cudaStream_t st, size_t* d
     // ---- work items: every query group (256 queries for kernel W, 64 for kernel R) against every row chunk ----
     const bool use_wide = tc_kernel_choice(D, a.sm_count) == 'W';
     if (a.metric != METRIC_L2 && !use_wide) { if (err) *err = "cosine / dot scans need kernel W (dim <= 384)"; return FVDB_ERR_INVALID_CONFIG; }
-    const uint32_t tile_q = use_wide ? (uint32_t)W_NQ : TC_TILE_Q;
+    const uint32_t tile_q = use_wide ? (uint32_t)W_NQ : r2_tile_q(D);
     const uint32_t tile_rows = use_wide ? (uint32_t)W_N : (uint32_t)TC_ROWS;
     const uint32_t n_qg = (nq + tile_q - 1) / tile_q;
     const uint32_t tiles = (uint32_t)((a.n_rows + tile_rows - 1) / tile_rows);
@@ -2327,17 +2372,10 @@ int tc_flat_search(TcScratch& s, const TcFlatArgs& a, cudaStream_t st, size_t* d
     if (use_wide) {
         TCK(launch_wide(m, rs.tmap_w, p, KB, a.sm_count, dev_bytes, st, a.ev_scan0));
     } else {
-        uint32_t stages = std::min<uint32_t>(12u, 6u * KB);
-        while (stages > 2 && tc_scan_smem_bytes(KB, stages) + 1024 > 232448) --stages;
-        p.stages = stages;
-        const size_t smem = tc_scan_smem_bytes(KB, stages) + 1024;
-        if (smem > 232448) { if (err) *err = "TC scan does not fit shared memory for this dim"; return FVDB_ERR_INVALID_CONFIG; }
-        if (!m->smem_attr_set) {
-            TCK(cudaFuncSetAttribute(tc_scan_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
-            m->smem_attr_set = true;
-        }
-        tc_scan_kernel<<<std::min<uint32_t>((uint32_t)a.sm_count, n_items), R2_THREADS, smem, st>>>(rs.tmap, p);
-        TCK(cudaGetLastError());
+        size_t smem = 0;
+        p.stages = r2_pick_stages(D, &smem);
+        if (!smem) { if (err) *err = "TC scan does not fit shared memory for this dim"; return FVDB_ERR_INVALID_CONFIG; }
+        TCK(launch_r2(m, rs.tmap, p, std::min<uint32_t>((uint32_t)a.sm_count, n_items), smem, st));
     }
     if (a.ev_scan1) TCK(cudaEventRecord(a.ev_scan1, st));
     TCK(launch_merge_rows32(m->partial.p, nq, n_chunks * frows, m->shortlist.p, st, m->row_stamp.p, stamp));

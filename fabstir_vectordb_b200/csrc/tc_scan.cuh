@@ -24,7 +24,8 @@ struct TcScratch {
 constexpr uint32_t TC_MAX_K = 16;        // largest k served by the 32-entry shortlist
 constexpr uint32_t TC_MAX_NPROBE = 256;  // partial lists merged in one pass
 constexpr uint32_t TC_MAX_NPROBE_COARSE = 112;  // tensor-core coarse step (else exact coarse)
-constexpr uint32_t TC_TILE_Q = 64;       // queries per work item of kernel R
+constexpr uint32_t TC_TILE_Q = 64;       // queries per work item of kernel R up to D = 512 (32 up to 1024, 16 above)
+constexpr uint32_t TC_MAX_D = 2048;      // widest row served (kernel R alone above D = 384)
 constexpr uint32_t TC_WIDE_MIN_QUERIES = 129;  // lists probed by at least this many queries of a batch go to kernel W
 constexpr uint32_t TC_MAX_PEERS = 7;     // peer GPUs whose bound arrays one scan can push to
 
@@ -95,7 +96,8 @@ struct TcFlatArgs {
     cudaEvent_t ev_scan0 = nullptr, ev_scan1 = nullptr;   // optional: recorded around the scan kernel
 };
 
-// dim % 32 == 0 (one 128-byte swizzle atom per k-block), dim <= 512 (query tile in smem)
+// dim % 32 == 0 (one 128-byte swizzle atom per k-block), 32 <= dim <= TC_MAX_D (the query tile of a kernel R
+// item, at most 128 KB, stays resident in shared memory)
 bool tc_supported(uint32_t D);
 
 // Tensor-core shortlist scan of the probed posting lists + exact fp32 re-rank + proof check.

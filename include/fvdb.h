@@ -91,7 +91,8 @@ typedef enum fvdb_metric {
                               falling back to EXACT for any query whose proof fails */
 
 typedef enum fvdb_option {
-    FVDB_OPT_SCAN_MODE = 1,   /* FVDB_SCAN_EXACT | FVDB_SCAN_TC (default TC when dim%32==0) */
+    FVDB_OPT_SCAN_MODE = 1,   /* FVDB_SCAN_EXACT | FVDB_SCAN_TC (default TC when dim % 32 == 0 and
+                                 32 <= dim <= 2048; FVDB_ERR_INVALID_CONFIG for TC at other dims) */
     FVDB_OPT_SHORTLIST = 2,   /* shortlist length k' of the TC mode (default max(32, ..)) */
     FVDB_OPT_KMEANS_TC = 3,   /* 1: k-means assignment on tensor cores with exact verify */
     FVDB_OPT_COALESCE = 4,    /* 1 (default): concurrent fvdb_search calls are coalesced into one device batch */
