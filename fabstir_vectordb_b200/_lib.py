@@ -85,6 +85,9 @@ SIGNATURES = {
     "fvdb_ivf_train": (C.c_int, [_vp, _f32p, C.c_uint64, C.c_uint32, C.c_uint32, _f32p, C.c_uint64,
                                  C.POINTER(TrainResult)]),
     "fvdb_ivf_retrain": (C.c_int, [_vp, C.c_uint32, C.c_uint32, _f32p, C.c_uint64, C.POINTER(TrainResult)]),
+    "fvdb_ivf_arena_device": (C.c_int, [_vp, C.POINTER(_vp), C.POINTER(_vp), _u64p]),
+    "fvdb_ivf_reassign": (C.c_int, [_vp, _f32p, C.c_uint32]),
+    "fvdb_ivf_take_unowned_device": (C.c_int, [_vp, _vp, C.c_uint32, C.c_uint32, _vp, _vp, C.c_uint64, _u64p, _vp]),
     "fvdb_ivf_dump_lists": (C.c_int, [_vp, _u32p, _u32p, C.c_uint64, _u64p]),
     "fvdb_assign": (C.c_int, [_vp, _f32p, C.c_uint64, _u32p]),
     "fvdb_ivf_add": (C.c_int, [_vp, _f32p, _u32p, C.c_uint64, _u32p]),

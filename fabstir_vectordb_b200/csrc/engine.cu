@@ -830,6 +830,41 @@ int train_device_impl(fvdb_index* h, const float* d_data, uint64_t n, uint32_t n
     return FVDB_OK;
 }
 
+// Install a host centroid table [nlist x dim] (checked for NaN by the caller) with empty list offsets; the
+// posting lists themselves are the caller's business.
+int install_centroids(fvdb_index* h, const float* centroids, uint32_t nlist) {
+    CK(h->centroids.ensure((size_t)nlist * h->dim, 0, h->stream, &h->dev_bytes));
+    RET(h2d(h, h->centroids.p, centroids, (size_t)nlist * h->dim * 4));
+    h->nlist = nlist;
+    h->trained = true;
+    mark_centroids_dirty(h); ++h->centroids_version;
+    CK(h->list_off.ensure(nlist + 2, 0, h->stream, &h->dev_bytes));
+    CK(cudaMemsetAsync(h->list_off.p, 0, (nlist + 2) * 4, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    return FVDB_OK;
+}
+
+// The second half of a retrain: the n rows (rows, ids), moved out of the arena by the caller, go back in, each
+// to its nearest centroid of the table now installed.  On failure the rows are put back where they were and
+// the handle reports "not trained" (its centroids no longer group them).
+int reassign_arena(fvdb_index* h, DevBuf<float>& rows, DevBuf<uint32_t>& ids, uint64_t n) {
+    h->ivf_n = 0;
+    h->pend_n = 0;
+    mark_arena_dirty(h);
+    int r = ivf_add_device_impl(h, rows.p, ids.p, n, 1, 0, nullptr, nullptr);
+    if (r == FVDB_OK) r = seal(h);
+    if (r == FVDB_OK) h->dev_bytes -= rows.cap * sizeof(float) + ids.cap * sizeof(uint32_t);   // freed on return
+    if (r != FVDB_OK) {
+        h->ivf_rows.swap(rows);
+        h->ivf_ids.swap(ids);
+        h->ivf_n = n;
+        h->pend_n = 0;
+        h->trained = false;
+        mark_arena_dirty(h);
+    }
+    return r;
+}
+
 // Exact IVF search of `nq` queries given their exact coarse ranking (src/ivf/core.rs:661-678):
 // bucket (query, probe) pairs by list, scan every probed list once, merge per query.
 int ivf_scan_exact(fvdb_index* h, const float* d_q, uint32_t nq, uint32_t k, uint32_t np,
@@ -1420,15 +1455,8 @@ int fvdb_ivf_set_centroids(fvdb_index* h, const float* centroids, uint32_t nlist
     if (!centroids || nlist == 0) return h->fail(FVDB_ERR_INVALID_CONFIG, "centroids empty");
     for (size_t i = 0; i < (size_t)nlist * h->dim; ++i)
         if (std::isnan(centroids[i])) return h->fail(FVDB_ERR_NAN, "NaN in centroids");
-    CK(h->centroids.ensure((size_t)nlist * h->dim, 0, h->stream, &h->dev_bytes));
-    RET(h2d(h, h->centroids.p, centroids, (size_t)nlist * h->dim * 4));
-    h->nlist = nlist;
-    h->trained = true;
-    mark_centroids_dirty(h); ++h->centroids_version;
+    RET(install_centroids(h, centroids, nlist));
     clear_lists(h);
-    CK(h->list_off.ensure(nlist + 2, 0, h->stream, &h->dev_bytes));
-    CK(cudaMemsetAsync(h->list_off.p, 0, (nlist + 2) * 4, h->stream));
-    CK(cudaStreamSynchronize(h->stream));
     return FVDB_OK;
 }
 
@@ -1506,19 +1534,106 @@ int fvdb_ivf_retrain(fvdb_index* h, uint32_t nlist, uint32_t max_iterations, con
         mark_arena_dirty(h);
         return r;
     }
-    r = ivf_add_device_impl(h, rows.p, ids.p, n, 1, 0, nullptr, nullptr);
-    if (r == FVDB_OK) r = seal(h);
-    if (r == FVDB_OK) h->dev_bytes -= rows.cap * sizeof(float) + ids.cap * sizeof(uint32_t);   // freed on return
+    return reassign_arena(h, rows, ids, n);
+}
+
+int fvdb_ivf_reassign(fvdb_index* h, const float* centroids, uint32_t nlist) {
+    ENTER(h);
+    if (h->metric != FVDB_METRIC_L2)
+        return h->fail(FVDB_ERR_INVALID_CONFIG, "the IVF tier is L2 only, like the reference's IVFIndex (src/ivf/core.rs:373-386, 646-678): "
+                       "a cosine / dot handle serves the flat tier (batch_cosine_similarity + top_k_indices, src/core/vector_ops.rs:8-23)");
+    if (!h->trained) return h->fail(FVDB_ERR_NOT_TRAINED, "Index not trained. Call train() before inserting or searching.");
+    if (!centroids || nlist == 0) return h->fail(FVDB_ERR_INVALID_CONFIG, "centroids empty");
+    for (size_t i = 0; i < (size_t)nlist * h->dim; ++i)
+        if (std::isnan(centroids[i])) return h->fail(FVDB_ERR_NAN, "NaN in centroids");
+    RET(seal(h));
+    const uint64_t n = h->ivf_n;
+    DevBuf<float> rows;
+    DevBuf<uint32_t> ids;
+    rows.swap(h->ivf_rows);
+    ids.swap(h->ivf_ids);
+    const int r = install_centroids(h, centroids, nlist);
     if (r != FVDB_OK) {
-        // new centroids, rows still grouped by the old ones: keep the rows, report "not trained"
         h->ivf_rows.swap(rows);
         h->ivf_ids.swap(ids);
-        h->ivf_n = n;
-        h->pend_n = 0;
         h->trained = false;
         mark_arena_dirty(h);
+        return r;
     }
-    return r;
+    return reassign_arena(h, rows, ids, n);
+}
+
+int fvdb_ivf_arena_device(fvdb_index* h, const float** d_rows, const uint32_t** d_ids, uint64_t* n) {
+    ENTER(h);
+    if (h->metric != FVDB_METRIC_L2)
+        return h->fail(FVDB_ERR_INVALID_CONFIG, "the IVF tier is L2 only, like the reference's IVFIndex (src/ivf/core.rs:373-386, 646-678): "
+                       "a cosine / dot handle serves the flat tier (batch_cosine_similarity + top_k_indices, src/core/vector_ops.rs:8-23)");
+    if (!d_rows || !d_ids || !n) return h->fail(FVDB_ERR_INVALID_ARG, "NULL output");
+    RET(seal(h));
+    *d_rows = h->ivf_rows.p;
+    *d_ids = h->ivf_ids.p;
+    *n = h->ivf_n;
+    return FVDB_OK;
+}
+
+int fvdb_ivf_take_unowned_device(fvdb_index* h, const uint32_t* d_owner, uint32_t my_rank, uint32_t world,
+                                 float* d_rows_out, uint32_t* d_ids_out, uint64_t cap, uint64_t* counts,
+                                 void* stream) {
+    ENTER(h);
+    if (h->metric != FVDB_METRIC_L2)
+        return h->fail(FVDB_ERR_INVALID_CONFIG, "the IVF tier is L2 only, like the reference's IVFIndex (src/ivf/core.rs:373-386, 646-678): "
+                       "a cosine / dot handle serves the flat tier (batch_cosine_similarity + top_k_indices, src/core/vector_ops.rs:8-23)");
+    if (!h->trained) return h->fail(FVDB_ERR_NOT_TRAINED, "Index not trained. Call train() before inserting or searching.");
+    if (!d_owner) return h->fail(FVDB_ERR_INVALID_ARG, "owner table is NULL");
+    if (!counts) return h->fail(FVDB_ERR_INVALID_ARG, "counts is NULL");
+    if (my_rank >= world) return h->fail(FVDB_ERR_INVALID_ARG, "my_rank >= world");
+    if (!d_rows_out != !d_ids_out) return h->fail(FVDB_ERR_INVALID_ARG, "give both output buffers or neither");
+    if ((uint64_t)h->nlist + world >= 0xFFFFFFF0ull) return h->fail(FVDB_ERR_INVALID_ARG, "world too large");
+    RET(seal(h));
+    cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
+    const uint64_t n = h->ivf_n;
+    const uint32_t D = h->dim, nl = h->nlist, nk = nl + world;
+    std::fill(counts, counts + world, 0);
+    if (n == 0) return FVDB_OK;
+    // one stable grouping: the kept rows first, by list (their new list offsets), then each rank's rows
+    CK(h->s_keys32.ensure(n, 0, st, &h->dev_bytes));
+    CK(launch_owner_keys(h->ivf_list.p, n, d_owner, my_rank, world, nl, h->s_keys32.p, st));
+    CK(h->s_perm.ensure(n, 0, st, &h->dev_bytes));
+    CK(h->s_group.ensure(stable_group_scratch_bytes(n, nk), 0, st, &h->dev_bytes));
+    CK(h->s_u32c.ensure(nk + 2, 0, st, &h->dev_bytes));
+    CK(launch_stable_group(h->s_keys32.p, n, nk, h->s_u32c.p, h->s_perm.p, h->s_group.p, st));
+    std::vector<uint32_t> off(world + 1);
+    CK(cudaMemcpyAsync(off.data(), h->s_u32c.p + nl, (world + 1) * 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    if (off[world] != n) return h->fail(FVDB_ERR_INVALID_ARG, "owner table names a rank >= world");
+    for (uint32_t r = 0; r < world; ++r) counts[r] = off[r + 1] - off[r];
+    const uint64_t kept = off[0], moved = n - kept;
+    if (!d_rows_out || moved == 0) return FVDB_OK;
+    if (cap < moved) return h->fail(FVDB_ERR_INVALID_ARG, "fvdb_ivf_take_unowned_device: buffers too small");
+    const uint32_t* perm = h->s_perm.p;
+    CK(launch_gather_rows(h->ivf_rows.p, n, nullptr, perm + kept, moved, D, d_rows_out, st));
+    CK(launch_gather_u32(h->ivf_ids.p, n, nullptr, perm + kept, moved, d_ids_out, st));
+    DevBuf<float> nrows;
+    DevBuf<uint32_t> nids, nlists;
+    CK(nrows.ensure((size_t)std::max<uint64_t>(kept, 1) * D, 0, st, &h->dev_bytes, true));
+    CK(nids.ensure(std::max<uint64_t>(kept, 1), 0, st, &h->dev_bytes, true));
+    CK(nlists.ensure(std::max<uint64_t>(kept, 1), 0, st, &h->dev_bytes, true));
+    CK(launch_gather_rows(h->ivf_rows.p, n, nullptr, perm, kept, D, nrows.p, st));
+    CK(launch_gather_u32(h->ivf_ids.p, n, nullptr, perm, kept, nids.p, st));
+    CK(launch_gather_u32(h->ivf_list.p, n, nullptr, perm, kept, nlists.p, st));
+    CK(cudaStreamSynchronize(st));
+    // groups 0..nlist-1 of the grouping are the kept lists: offsets[0..nlist] are the new list offsets, and
+    // list_off[nlist + 1] is one past the arena, as seal() leaves it
+    CK(cudaMemcpyAsync(h->list_off.p, h->s_u32c.p, (size_t)(nl + 1) * 4, cudaMemcpyDeviceToDevice, st));
+    CK(cudaMemcpyAsync(h->list_off.p + nl + 1, h->s_u32c.p + nl, 4, cudaMemcpyDeviceToDevice, st));
+    CK(cudaStreamSynchronize(st));
+    h->dev_bytes -= h->ivf_rows.cap * sizeof(float) + (h->ivf_ids.cap + h->ivf_list.cap) * 4;
+    h->ivf_rows.swap(nrows);
+    h->ivf_ids.swap(nids);
+    h->ivf_list.swap(nlists);
+    h->ivf_n = kept;
+    mark_arena_dirty(h);
+    return FVDB_OK;
 }
 
 int fvdb_ivf_dump_lists(fvdb_index* h, uint32_t* out_row_ids, uint32_t* out_lists, uint64_t cap, uint64_t* n_out) {

@@ -192,6 +192,20 @@ __global__ void filter_keys_owner_kernel(const uint32_t* __restrict__ keys, uint
     }
 }
 
+// re-placement after a sharded retrain: a row of a list this rank owns keeps its list as key (group l), a
+// row of another rank's list gets nlist + that rank; an owner >= world goes to the drop group
+__global__ void owner_keys_kernel(const uint32_t* __restrict__ lists, uint64_t n,
+                                  const uint32_t* __restrict__ owner, uint32_t rank, uint32_t world,
+                                  uint32_t nlist, uint32_t* __restrict__ keys) {
+    uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (; i < n; i += stride) {
+        const uint32_t l = lists[i];
+        const uint32_t o = __ldg(owner + l);
+        keys[i] = o == rank ? l : (o < world ? nlist + o : nlist + world);
+    }
+}
+
 __global__ void iota_kernel(uint32_t* __restrict__ p, uint64_t n, uint32_t start) {
     uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
@@ -285,6 +299,13 @@ cudaError_t launch_filter_keys_owner(const uint32_t* keys, uint64_t n, const uin
                                      uint32_t drop, uint32_t* keys_out, cudaStream_t stream) {
     if (n == 0) return cudaSuccess;
     filter_keys_owner_kernel<<<grid_for(n), 256, 0, stream>>>(keys, n, owner, rank, drop, keys_out);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_owner_keys(const uint32_t* lists, uint64_t n, const uint32_t* owner, uint32_t rank,
+                              uint32_t world, uint32_t nlist, uint32_t* keys, cudaStream_t stream) {
+    if (n == 0) return cudaSuccess;
+    owner_keys_kernel<<<grid_for(n), 256, 0, stream>>>(lists, n, owner, rank, world, nlist, keys);
     return cudaGetLastError();
 }
 

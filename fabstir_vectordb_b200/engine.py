@@ -204,6 +204,29 @@ class Engine:
         return dict(iterations=res.iterations, converged=bool(res.converged),
                     initial_error=res.initial_error, final_error=res.final_error)
 
+    def ivf_arena_device(self):
+        """(device address of the rows [n x dim] f32, of the ids [n] u32, n): the sealed IVF arena, read-only,
+        valid until the next call that changes the IVF tier (fvdb_ivf_arena_device)."""
+        rows, ids, n = C.c_void_p(), C.c_void_p(), C.c_uint64()
+        self._ck(self._lib.fvdb_ivf_arena_device(self._h, C.byref(rows), C.byref(ids), C.byref(n)))
+        return rows.value or 0, ids.value or 0, n.value
+
+    def ivf_reassign(self, centroids):
+        """Install `centroids` [nlist x dim] and move every IVF row to its nearest new centroid in place
+        (fvdb_ivf_reassign)."""
+        c = _f32(centroids, self.dim)
+        self._ck(self._lib.fvdb_ivf_reassign(self._h, _p(c, _f32p), c.shape[0]))
+
+    def ivf_take_unowned_device(self, d_owner: int, my_rank: int, world: int, d_rows_out: int = 0,
+                                d_ids_out: int = 0, cap: int = 0, stream: int = 0) -> np.ndarray:
+        """Remove the rows of lists other ranks own into the device buffers, grouped by rank; returns the rows
+        per rank (u64 [world]).  Without buffers: the counts only (fvdb_ivf_take_unowned_device)."""
+        counts = np.zeros(world, dtype=np.uint64)
+        self._ck(self._lib.fvdb_ivf_take_unowned_device(self._h, d_owner, my_rank, world, d_rows_out or None,
+                                                        d_ids_out or None, cap, _p(counts, _u64p),
+                                                        _stream(stream)))
+        return counts
+
     def dump_lists(self):
         """(row ids, lists) of the IVF tier in arena order."""
         n = C.c_uint64()

@@ -15,12 +15,15 @@ both tiers are split over the ranks.
 Mutations (delete, vacuum, migrate) are broadcast: every rank applies them to the rows it holds.  The
 tombstone and filter bitmaps are indexed by global row id, so a rank accepts ids it does not hold.  A
 migrated row joins its nearest list in the arena of the rank that held it, whichever rank owns that list.
+retrain / optimize_clusters re-cluster the IVF rows where they are and then move every row to the rank that
+owns its new list, which restores a size-balanced placement.
 
 The collective is torch.distributed (NCCL on GPUs; gloo in the CPU tests of the layout logic).
 """
 from __future__ import annotations
 
 import os
+import time
 from typing import Optional, Tuple
 
 import numpy as np
@@ -137,6 +140,23 @@ def _cur_stream(t=None) -> int:
     return torch.cuda.current_stream().cuda_stream
 
 
+def _tensor_at(ptr: int, shape, typestr: str, device):
+    """A torch tensor over memory the engine owns (no copy): __cuda_array_interface__ on a GPU, the raw bytes on
+    the host (the gloo tests' stand-in engines)."""
+    import ctypes
+    import torch
+    n = int(np.prod(shape))
+    dtype = {"<f4": torch.float32, "<i4": torch.int32}[typestr]
+    if n == 0:
+        return torch.empty(shape, dtype=dtype, device=device)
+    if device.type == "cuda":
+        # torch refuses the read-only flag; the callers only read through the tensor
+        view = type("_DeviceView", (), {"__cuda_array_interface__": dict(shape=tuple(shape), typestr=typestr,
+                                                                          data=(ptr, False), version=3)})()
+        return torch.as_tensor(view, device=device)
+    return torch.frombuffer((ctypes.c_char * (4 * n)).from_address(ptr), dtype=dtype).view(shape)
+
+
 class ShardedIndex:
     """One rank's shard + the exchange step.  All tensors are torch CUDA tensors."""
 
@@ -199,12 +219,20 @@ class ShardedIndex:
         if q.is_cuda:
             self.eng.bounds_begin_batch(nq, stream)
 
+    def _device(self):
+        """Where this rank's collectives run: the host under gloo (the CPU tests), else the current GPU."""
+        import torch
+        import torch.distributed as dist
+        if self.world > 1 and dist.is_initialized() and dist.get_backend(self.group) == "gloo":
+            return torch.device("cpu")
+        return torch.device("cuda", torch.cuda.current_device())
+
     def set_placement(self, owner):
         """Install a list -> rank table (place_lists) in place of the l % world rule; `owner` is a host
         array [nlist].  Rows loaded afterwards are kept when owner[list] == rank."""
         import torch
         self.owner_host = np.ascontiguousarray(owner, dtype=np.uint32)
-        self.owner = torch.from_numpy(self.owner_host.view(np.int32)).to(torch.device("cuda", torch.cuda.current_device()))
+        self.owner = torch.from_numpy(self.owner_host.view(np.int32)).to(self._device())
 
     def list_histogram_device(self, x, hist):
         """hist[l] += number of rows of x (CUDA tensor [n x dim]) whose nearest centroid is l: the input of
@@ -239,9 +267,7 @@ class ShardedIndex:
             return int(v)
         import torch
         import torch.distributed as dist
-        dev = torch.device("cpu") if dist.get_backend(self.group) == "gloo" else \
-            torch.device("cuda", torch.cuda.current_device())
-        t = torch.tensor([int(v)], dtype=torch.int64, device=dev)
+        t = torch.tensor([int(v)], dtype=torch.int64, device=self._device())
         dist.all_reduce(t, op=dist.ReduceOp.SUM, group=self.group)
         return int(t.item())
 
@@ -267,10 +293,11 @@ class ShardedIndex:
         self._xmax_dirty = True
         return self._sum_over_ranks(self.eng.move_flat_to_ivf(np.ascontiguousarray(row_ids, dtype=np.uint32)))
 
-    def train(self, points, nlist: int, max_iterations: int, init_centroids):
+    def train(self, points, nlist: int, max_iterations: int, init_centroids, eng: Optional[Engine] = None):
         """IVFIndex::train (src/ivf/core.rs:240-334) with the points sharded over the ranks (SURVEY §8e):
         `points` is THIS rank's slice (CUDA tensor [n_r x dim]), `init_centroids` [nlist x dim] (host array,
-        the same on every rank).  Per iteration every rank assigns its points against the replicated
+        the same on every rank).  The centroids are trained on `eng` (default: this rank's engine; retrain
+        passes a scratch handle).  Per iteration every rank assigns its points against the replicated
         centroid table and accumulates per-cluster sums and counts (fvdb_kmeans_accumulate_device), one
         all-reduce makes them global (kmeans_allreduce_step), every rank installs the same means
         (fvdb_kmeans_apply_device; an empty cluster keeps its centroid, :410-415).  Stop rule of :303-321 on
@@ -279,11 +306,12 @@ class ShardedIndex:
         Returns dict(iterations, converged, initial_error, final_error); like the reference, training
         leaves every posting list empty."""
         import torch
+        eng = self.eng if eng is None else eng
         dev = points.device
         dim = points.shape[1]
         n_r = points.shape[0]
-        stream = torch.cuda.current_stream().cuda_stream
-        self.eng.set_centroids(np.ascontiguousarray(init_centroids, dtype=np.float32))
+        stream = _cur_stream(points)
+        eng.set_centroids(np.ascontiguousarray(init_centroids, dtype=np.float32))
         sums = torch.zeros((nlist, dim), dtype=torch.float32, device=dev)
         counts = torch.zeros((nlist,), dtype=torch.int32, device=dev)
         sqerr = torch.zeros((1,), dtype=torch.float64, device=dev)
@@ -295,8 +323,8 @@ class ShardedIndex:
             iterations = it + 1
             sums.zero_(); counts.zero_(); sqerr.zero_(); changed.zero_()
             if n_r:
-                self.eng.kmeans_accumulate_device(points.data_ptr(), n_r, sums.data_ptr(), counts.data_ptr(),
-                                                  sqerr.data_ptr(), assign.data_ptr(), changed.data_ptr(), stream)
+                eng.kmeans_accumulate_device(points.data_ptr(), n_r, sums.data_ptr(), counts.data_ptr(),
+                                             sqerr.data_ptr(), assign.data_ptr(), changed.data_ptr(), stream)
             if self.world > 1:
                 tot, n_changed, n_total = kmeans_allreduce_step(sums, counts, sqerr, changed, self.group)
             else:
@@ -304,15 +332,142 @@ class ShardedIndex:
             err = tot / max(1, n_total)
             if initial is None:
                 initial = err
-            self.eng.kmeans_apply_device(sums.data_ptr(), counts.data_ptr(), stream)
+            eng.kmeans_apply_device(sums.data_ptr(), counts.data_ptr(), stream)
             if iterations >= max_iterations:
                 break
             if n_changed == 0 or (prev_err != float("inf") and abs(prev_err - err) / prev_err < 1e-4):
                 converged = True
                 break
             prev_err = err
-        torch.cuda.synchronize()
+        if points.is_cuda:
+            torch.cuda.synchronize()
         return dict(iterations=iterations, converged=converged, initial_error=initial, final_error=err)
+
+    def retrain(self, nlist: int, max_iterations: int, init_centroids) -> dict:
+        """IVFIndex::retrain (src/ivf/operations.rs:148-193) over the list-sharded IVF tier, without a host copy of
+        any row.  Every rank calls it with the same arguments; `init_centroids` [nlist x dim] is a host array.
+
+        1. The sharded Lloyd of train() runs on a scratch handle over this rank's arena as it is
+           (fvdb_ivf_arena_device: every IVF row, tombstoned rows included); this handle's centroids keep
+           grouping the arena meanwhile.  The final centroids are bit-identical on every rank (all-reduced sums).
+        2. fvdb_ivf_reassign installs them and moves every row to its nearest new list, in place.
+        3. The list histogram is all-reduced and place_lists makes the new placement (set_placement).
+        4. fvdb_ivf_take_unowned_device takes out the rows of lists other ranks own; two all_to_all_single
+           exchanges (the counts, then the rows and ids) deliver them, and each rank adds what it received
+           (add_rows_device).
+        Afterwards every row sits on the rank that owns its list, as after a fresh balanced build.
+
+        Failure rule: a row on a rank that does not own its list is legal (migrate makes such rows), so when the
+        exchange fails each rank puts the rows it took back into its own arena (fvdb_ivf_add_device, mod 1) and
+        the error propagates: results stay exact, only the balance is lost.
+
+        Peak device memory per rank is about three times its arena: the arena, the rows it sends and the rows it
+        receives, while the received rows are added.
+
+        Pipelined batches must be finished first (RuntimeError otherwise).  Returns dict(old_nlist, new_nlist,
+        rows_reassigned and rows_moved summed over the ranks, converged, iterations, seconds): `seconds` holds this
+        rank's host-clock time of each step (lloyd, reassign, placement, exchange); every step ends in a
+        synchronisation."""
+        import torch
+        import torch.distributed as dist
+        if self._inflight is not None or self._group:
+            raise RuntimeError("retrain: submitted search batches are in flight; call finish() first")
+        dev = self._device()
+        old_nlist = int(self.eng.stats().nlist)
+        init = np.ascontiguousarray(init_centroids, dtype=np.float32).reshape(nlist, self.eng.dim)
+
+        secs, t0 = {}, time.perf_counter()
+
+        def lap(name):
+            nonlocal t0
+            t1 = time.perf_counter()
+            secs[name], t0 = t1 - t0, t1
+
+        # 1. Lloyd on a scratch handle over the arena as it stands
+        p_rows, _, n = self.eng.ivf_arena_device()
+        rows = _tensor_at(p_rows, (n, self.eng.dim), "<f4", dev)
+        scratch = self._new_scratch()
+        try:
+            tr = self.train(rows, nlist, max_iterations, init, eng=scratch)
+            cents = scratch.get_centroids()
+        finally:
+            scratch.close()
+        del rows
+        lap("lloyd")
+        try:
+            # 2. every row to its nearest new list, in place
+            self.eng.ivf_reassign(cents)
+            lap("reassign")
+            # 3. the new placement from the global list histogram
+            _, lists = self.eng.dump_lists()
+            hist = torch.from_numpy(np.bincount(lists, minlength=nlist).astype(np.int64)).to(dev)
+            if self.world > 1:
+                dist.all_reduce(hist, op=dist.ReduceOp.SUM, group=self.group)
+            self.set_placement(place_lists(hist.cpu().numpy(), self.world))
+            lap("placement")
+            # 4. rows to their owners
+            moved = self._exchange_unowned(dev) if self.world > 1 else 0
+            lap("exchange")
+        finally:
+            # the centroid table (and with it nlist) and the rows of the IVF tier have changed
+            self._xmax_dirty = True
+            self._nlist = None
+            self._bufs = {k: v for k, v in self._bufs.items() if k[0] != "coarse"}
+        self._nlist = nlist
+        return dict(old_nlist=old_nlist, new_nlist=nlist, rows_reassigned=self._sum_over_ranks(n),
+                    rows_moved=self._sum_over_ranks(moved), converged=tr["converged"], iterations=tr["iterations"],
+                    seconds=secs)
+
+    def optimize_clusters(self, max_iterations: int = 25) -> dict:
+        """IVFIndex::optimize_clusters (src/ivf/operations.rs:221-260) on the sharded index: retrain with the same
+        nlist, starting from the current centroids."""
+        cents = self.eng.get_centroids()
+        return self.retrain(cents.shape[0], max_iterations, cents)
+
+    def add_clusters(self, n_clusters_to_add: int, init_centroids, max_iterations: int = 25) -> dict:
+        """IVFIndex::add_clusters (src/ivf/operations.rs:195-219) on the sharded index: retrain with nlist +
+        n_clusters_to_add from `init_centroids` [nlist + n x dim] (host, the same on every rank)."""
+        return self.retrain(int(self.eng.stats().nlist) + n_clusters_to_add, max_iterations, init_centroids)
+
+    def _new_scratch(self) -> Engine:
+        """The handle the working centroids of a retrain live on (this rank's device, no rows)."""
+        return Engine(self.eng.dim, k_max=1, device=self.eng.device)
+
+    def _exchange_unowned(self, dev) -> int:
+        """Step 4 of retrain: take out the rows of other ranks' lists, exchange, add.  Returns the rows sent."""
+        import torch
+        import torch.distributed as dist
+        stream = _cur_stream(self.owner)
+        counts = self.eng.ivf_take_unowned_device(self.owner.data_ptr(), self.rank, self.world, stream=stream)
+        n_send = int(counts.sum())
+        send_x = torch.empty((n_send, self.eng.dim), dtype=torch.float32, device=dev)
+        send_ids = torch.empty((n_send,), dtype=torch.int32, device=dev)
+        if n_send:
+            self.eng.ivf_take_unowned_device(self.owner.data_ptr(), self.rank, self.world, send_x.data_ptr(),
+                                             send_ids.data_ptr(), n_send, stream)
+        try:
+            send_counts = torch.from_numpy(counts.astype(np.int64)).to(dev)
+            recv_counts = torch.empty_like(send_counts)
+            dist.all_to_all_single(recv_counts, send_counts, group=self.group)
+            recv_counts = recv_counts.cpu().numpy().tolist()
+            recv_x = torch.empty((sum(recv_counts), self.eng.dim), dtype=torch.float32, device=dev)
+            recv_ids = torch.empty((sum(recv_counts),), dtype=torch.int32, device=dev)
+            split = counts.astype(np.int64).tolist()
+            dist.all_to_all_single(recv_x, send_x, recv_counts, split, group=self.group)
+            dist.all_to_all_single(recv_ids, send_ids, recv_counts, split, group=self.group)
+        except Exception:
+            if n_send:      # the failure rule: the taken rows go back into this rank's own arena
+                self.eng.ivf_add_device(send_x.data_ptr(), send_ids.data_ptr(), n_send, 1, 0)
+            raise
+        del send_x, send_ids
+        n_recv = int(recv_x.shape[0])
+        if recv_x.is_cuda:      # the engine reads the rows on its own stream
+            torch.cuda.current_stream().synchronize()
+        if n_recv:
+            kept = self.add_rows_device(recv_x, recv_ids)
+            if kept != n_recv:
+                raise RuntimeError(f"retrain: rank {self.rank} kept {kept} of the {n_recv} rows it received")
+        return n_send
 
     def _buffers(self, nq: int, k: int, device, slot: int = 0, tiered: bool = False):
         import torch

@@ -247,6 +247,41 @@ int fvdb_search_postfilter(fvdb_index *h, const float *q, uint32_t nq, uint32_t 
 int fvdb_ivf_retrain(fvdb_index *h, uint32_t nlist, uint32_t max_iterations,
                      const float *init_centroids, uint64_t seed, fvdb_train_result *out);
 
+/* The two halves of fvdb_ivf_retrain for a list-sharded index (IVFIndex::retrain, src/ivf/operations.rs:148-193,
+ * with the rows spread over several GPUs), plus the step that gives every rank back the lists it owns.
+ *
+ * fvdb_ivf_arena_device: seals pending rows, then returns read-only device pointers to the IVF arena —
+ * d_rows [n x dim] f32 and d_ids [n] u32, arena order (by list, insertion order inside a list), tombstoned rows
+ * included — and its row count.  No copy is made.  This is the training set of a sharded retrain: the driver
+ * runs fvdb_kmeans_accumulate_device / fvdb_kmeans_apply_device over it on a second handle that holds the
+ * working centroids, while this handle's own centroids keep grouping its arena.  The pointers stay valid until
+ * the next call on this handle that changes the IVF tier (insert, set_centroids, train, retrain, reassign,
+ * take_unowned, vacuum, move_flat_to_ivf, destroy).
+ *
+ * fvdb_ivf_reassign: installs a new centroid table [nlist x dim] (host) and moves every IVF row, tombstoned rows
+ * included, to its nearest new centroid (find_nearest_centroid: strict '<', the lowest list id on ties; :186-188
+ * -> insert, src/ivf/core.rs:431-455).  The rows stay on the device.  Row ids, tombstones and the recent tier
+ * are unchanged; the result is the one fvdb_ivf_retrain leaves when its k-means ends at these centroids.
+ * Errors: NOT_TRAINED before centroids exist, INVALID_CONFIG for an empty table, NAN for NaN in it.  A failure
+ * after the table was replaced (CUDA error, out of memory) keeps every row and leaves the handle "not trained".
+ *
+ * fvdb_ivf_take_unowned_device: removes from the arena every row whose list l has d_owner[l] != my_rank
+ * (d_owner: [nlist] u32, device — the place_lists table of the multi-GPU driver) and writes them to d_rows_out
+ * [cap x dim] / d_ids_out [cap] (device), grouped by destination rank (ascending), arena order within a rank.
+ * counts (host, [world]) receives the number of rows for each rank; counts[my_rank] = 0.  The kept rows are
+ * compacted in the same pass and stay grouped by list.  With both buffers NULL only counts is filled and nothing
+ * is removed (like fvdb_ivf_dump_lists).  Work runs on `stream` (NULL = the handle's stream) and is complete on
+ * return.  The receiving rank adds the rows with fvdb_ivf_add_device_owned, which assigns them to the same lists
+ * (assignment is exact).  Errors: NOT_TRAINED; INVALID_ARG when d_owner or counts is NULL, my_rank >= world, only
+ * one buffer is given, cap is below the rows to move, or the table names a rank >= world (nothing removed).
+ *
+ * All three are L2 only (FVDB_ERR_INVALID_CONFIG on a COS / DOT handle) and wait for the pipeline slots. */
+int fvdb_ivf_arena_device(fvdb_index *h, const float **d_rows, const uint32_t **d_ids, uint64_t *n);
+int fvdb_ivf_reassign(fvdb_index *h, const float *centroids, uint32_t nlist);
+int fvdb_ivf_take_unowned_device(fvdb_index *h, const uint32_t *d_owner, uint32_t my_rank, uint32_t world,
+                                 float *d_rows_out, uint32_t *d_ids_out, uint64_t cap, uint64_t *counts,
+                                 void *stream);
+
 /* (row id, list) of every row of the IVF tier in arena order — the membership the host keeps
  * per VectorId (InvertedList, src/ivf/core.rs:112-157) after a retrain, and what
  * save_index_chunked (src/hybrid/persistence.rs:188) walks.  NULL buffers: only *n_out. */
