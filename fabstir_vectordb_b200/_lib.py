@@ -8,8 +8,7 @@ import ctypes as C
 import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# FVDB_LIB selects an experiment build of the same library (fabstir_vectordb_b200/build.py variants)
-SO_PATH = os.environ.get("FVDB_LIB") or os.path.join(_HERE, "libfvdb_b200.so")
+SO_PATH = os.path.join(_HERE, "libfvdb_b200.so")
 
 # fvdb_status (include/fvdb.h)
 OK = 0
@@ -164,8 +163,6 @@ def load():
             "(there is no CPU fallback)")
     lib = C.CDLL(SO_PATH)
     for name, (res, args) in SIGNATURES.items():
-        if os.environ.get("FVDB_LIB") and not hasattr(lib, name):
-            continue  # an experiment build of an older source tree may lack newer entry points
         fn = getattr(lib, name)  # AttributeError if the .so does not export it
         fn.restype = res
         fn.argtypes = args

@@ -14,13 +14,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 ROOT = os.path.dirname(HERE)
-# experiment builds: FVDB_BUILD_VARIANT=name FVDB_BUILD_DEFINES="-DFVDB_R2_CAP=16 ..." python -m ...build
-# writes libfvdb_b200.<name>.so next to the product library (selected at load time with FVDB_LIB)
-VARIANT = os.environ.get("FVDB_BUILD_VARIANT", "")
-DEFINES = os.environ.get("FVDB_BUILD_DEFINES", "").split()
-_TAG = ("." + VARIANT) if VARIANT else ""
-SO = os.path.join(HERE, f"libfvdb_b200{_TAG}.so")
-STAMP = os.path.join(HERE, f".libfvdb_b200{_TAG}.stamp")
+SO = os.path.join(HERE, "libfvdb_b200.so")
+STAMP = os.path.join(HERE, ".libfvdb_b200.stamp")
 
 SOURCES = ["engine.cu", "exact_scan.cu", "layout.cu", "kmeans.cu", "tc_scan.cu", "synth.cu", "chunk_codec.cu"]
 HEADERS = ["common.cuh", "kernels.cuh", "tc_scan.cuh", "tc_ptx.cuh", "tc_scan_wide.cuh"]
@@ -43,7 +38,7 @@ def _digest() -> str:
     for f in ("fvdb.h", "fvdb_synth.h", "fvdb_chunk.h"):
         with open(os.path.join(ROOT, "include", f), "rb") as fh:
             h.update(fh.read())
-    h.update(" ".join(FLAGS + DEFINES).encode())
+    h.update(" ".join(FLAGS).encode())
     return h.hexdigest()
 
 
@@ -56,8 +51,8 @@ def build(force: bool = False, verbose: bool = False) -> str:
     objs = []
     procs = []
     for src in SOURCES:
-        obj = os.path.join(CSRC, src.replace(".cu", f"{_TAG}.o"))
-        cmd = [NVCC, *FLAGS, *DEFINES, "-c", os.path.join(CSRC, src), "-o", obj]
+        obj = os.path.join(CSRC, src.replace(".cu", ".o"))
+        cmd = [NVCC, *FLAGS, "-c", os.path.join(CSRC, src), "-o", obj]
         if verbose:
             cmd.insert(1, "-Xptxas=-v")
             print(" ".join(cmd), flush=True)

@@ -386,8 +386,8 @@ __global__ void __launch_bounds__(1024) probe_scan_kernel(const uint32_t* __rest
                                   uint32_t tile_q, uint32_t* __restrict__ pair_off,
                                   uint32_t* __restrict__ cursor, ScanItem* __restrict__ items,
                                   uint32_t* __restrict__ n_items, uint64_t* __restrict__ scanned_rows,
-                                  bool order_near_in, uint32_t rows_cap, uint32_t wide_min, uint32_t tile_q_w,
-                                  ScanItem* __restrict__ items_w, uint32_t* __restrict__ n_items_w, bool wide_longest_first,
+                                  uint32_t rows_cap, uint32_t wide_min, uint32_t tile_q_w,
+                                  ScanItem* __restrict__ items_w, uint32_t* __restrict__ n_items_w,
                                   const uint32_t* __restrict__ live_ids, uint32_t n_live) {
     // live_ids (optional, with list_order): the n_live non-empty lists in ascending id order; list_order then
     // holds them first (longest first).  A list-sharded index owns 1 / world of the lists: walking only those
@@ -402,7 +402,6 @@ __global__ void __launch_bounds__(1024) probe_scan_kernel(const uint32_t* __rest
         const bool wide = wide_min && tbl == 0;
         const uint32_t tq = wide ? tile_q_w : tile_q;
         ScanItem* out = wide ? items_w : items;
-        const bool order_near = order_near_in || (wide && wide_longest_first);
         // offsets and items.  g = 0: the nearest-first group in list order; g = 1: the other
         // lists, longest first when list_order is given — the dynamic tile scheduler then ends with
         // the cheapest items, which keeps the tail of the scan short.  (Ordering the nearest group by
@@ -420,7 +419,7 @@ __global__ void __launch_bounds__(1024) probe_scan_kernel(const uint32_t* __rest
         };
         for (int g = 0; g < 2; ++g) {
             for (uint32_t base = 0; base < n_walk; base += 1024) {
-                const uint32_t l = (base + t < n_walk) ? (((g || order_near) && list_order) ? list_order[base + t]
+                const uint32_t l = (base + t < n_walk) ? ((g && list_order) ? list_order[base + t]
                                                           : (live_ids && list_order) ? live_ids[base + t] : base + t) : nlist;
                 uint32_t c, len;
                 bool nearest;
@@ -466,8 +465,8 @@ __global__ void __launch_bounds__(1024) probe_scan_kernel(const uint32_t* __rest
                 for (uint32_t sb = 1; sb < 64; ++sb) {
                     uint32_t any = 0;
                     for (uint32_t base = 0; base < n_walk; base += 1024) {
-                        const uint32_t l = (base + t < n_walk) ? ((order_near && list_order) ? list_order[base + t]
-                                                                  : (live_ids && list_order) ? live_ids[base + t] : base + t) : nlist;
+                        const uint32_t l = (base + t < n_walk) ? ((live_ids && list_order) ? live_ids[base + t] : base + t)
+                                                               : nlist;
                         uint32_t c, len;
                         bool nearest;
                         mine(l, c, len, nearest);
@@ -529,9 +528,9 @@ cudaError_t launch_probe_bucketing(const uint64_t* coarse_keys, uint32_t nq, uin
                                    uint32_t* list_cnt, uint32_t* pair_off, uint32_t* cursor,
                                    uint32_t* pair_q, uint32_t* pair_slot, ScanItem* items,
                                    uint32_t* n_items, uint64_t* scanned_rows, cudaStream_t stream,
-                                   const uint32_t* list_order, bool order_near, uint32_t rows_cap,
+                                   const uint32_t* list_order, uint32_t rows_cap,
                                    uint32_t wide_min, uint32_t tile_q_w, ScanItem* items_w, uint32_t* n_items_w,
-                                   bool wide_longest_first, const uint32_t* live_ids, uint32_t n_live) {
+                                   const uint32_t* live_ids, uint32_t n_live) {
     const uint32_t n_pairs = nq * nprobe;
     cudaError_t e = cudaMemsetAsync(list_cnt, 0, sizeof(uint32_t) * nlist, stream);
     if (e != cudaSuccess) return e;
@@ -541,8 +540,8 @@ cudaError_t launch_probe_bucketing(const uint64_t* coarse_keys, uint32_t nq, uin
     }
     probe_hist_kernel<<<(n_pairs + 255) / 256, 256, 0, stream>>>(coarse_keys, n_pairs, nprobe, list_cnt);
     probe_scan_kernel<<<1, 1024, 0, stream>>>(list_cnt, list_off, list_order, nlist, tile_q, pair_off, cursor,
-                                              items, n_items, scanned_rows, order_near, rows_cap, wide_min, tile_q_w,
-                                              items_w, n_items_w, wide_longest_first, live_ids, n_live);
+                                              items, n_items, scanned_rows, rows_cap, wide_min, tile_q_w,
+                                              items_w, n_items_w, live_ids, n_live);
     probe_scatter_kernel<<<(n_pairs + 255) / 256, 256, 0, stream>>>(coarse_keys, n_pairs, nprobe,
                                                                    list_off, cursor, pair_q,
                                                                    pair_slot);

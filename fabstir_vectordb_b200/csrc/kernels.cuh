@@ -38,12 +38,11 @@ cudaError_t launch_probe_bucketing(const uint64_t* coarse_keys, uint32_t nq, uin
                                    uint32_t* list_cnt, uint32_t* pair_off, uint32_t* cursor,
                                    uint32_t* pair_q, uint32_t* pair_slot, ScanItem* items,
                                    uint32_t* n_items, uint64_t* scanned_rows, cudaStream_t stream,
-                                   const uint32_t* list_order = nullptr, bool order_near = false,
-                                   uint32_t rows_cap = 0,
+                                   const uint32_t* list_order = nullptr, uint32_t rows_cap = 0,
                                    // optional second table: lists probed by >= wide_min queries become items
                                    // of tile_q_w queries in items_w (the wide-tile scan kernel's share)
                                    uint32_t wide_min = 0, uint32_t tile_q_w = 0, ScanItem* items_w = nullptr,
-                                   uint32_t* n_items_w = nullptr, bool wide_longest_first = false,
+                                   uint32_t* n_items_w = nullptr,
                                    // optional (with list_order): the non-empty lists, ascending — only those are walked
                                    const uint32_t* live_ids = nullptr, uint32_t n_live = 0);
 // one warp per (query, probed list): sparse batches (few queries per list)

@@ -61,7 +61,7 @@ struct TcScanParams {
     uint32_t* work_counter;  // dynamic tile scheduler: next unclaimed work item
     uint32_t stages;
     uint32_t kbs;            // kernel Q: k-blocks (128 B each) per pipeline stage
-    const float* rows_raw;   // layout experiment (debug bit 4): arena base for 1-D bulk copies
+    const float* rows_raw;   // read by no kernel; kept because removing it would move the fields below in kernel R and W
     uint64_t rows_bytes;
     float* dense_out;        // kernel Q dense mode (coarse step): out[q * dense_ld + row] = approx d2
     uint32_t dense_ld;
@@ -104,23 +104,11 @@ constexpr int R2_STAGE_BYTES = R2_ROWS * 128;    // 16 KB: 128 rows x one 128-by
 // KB x NQ x 128 B, stays resident for the whole item, so the width halves as D doubles past 512 and
 // the tile never exceeds the 128 KB it takes at D = 512 (a 64-query tile of D = 1024 would need 256 KB)
 constexpr uint32_t r2_tile_q(uint32_t D) { return D <= 512 ? TC_TILE_Q : D <= 1024 ? 32u : 16u; }
-#ifndef FVDB_R2_CAP
-#define FVDB_R2_CAP 32
-#endif
-#ifndef FVDB_R2_FLUSH
-#define FVDB_R2_FLUSH (FVDB_R2_CAP / 2)
-#endif
-#ifndef FVDB_R2_NSLOT
-#define FVDB_R2_NSLOT 16
-#endif
-#ifndef FVDB_R2_SLACK
-#define FVDB_R2_SLACK 1024
-#endif
-constexpr int R2_CAP = FVDB_R2_CAP;              // pending candidates per query (<= 32: one sorting network)
-constexpr int R2_FLUSH = FVDB_R2_FLUSH;          // merge a query once it holds more pending than this
+constexpr int R2_CAP = 32;                       // pending candidates per query (<= 32: one sorting network)
+constexpr int R2_FLUSH = R2_CAP / 2;             // merge a query once it holds more pending than this
 constexpr int R2_NBUF = 8;                       // accumulator buffers of NQ columns
-constexpr int R2_NSLOT = FVDB_R2_NSLOT;          // |x|^2 strips in flight
-constexpr int R2_SLACK = FVDB_R2_SLACK;          // bytes reserved for aligning the dynamic shared memory to 1024 (0: trap if it is not)
+constexpr int R2_NSLOT = 16;                     // |x|^2 strips in flight
+constexpr int R2_SLACK = 1024;                   // bytes reserved for aligning the dynamic shared memory to 1024 (0: trap if it is not)
 static_assert(R2_CAP <= 32 && R2_FLUSH < R2_CAP && R2_NSLOT > R2_NBUF + 2, "kernel R pools");
 constexpr int R2_THREADS = 320;
 constexpr uint32_t TC_SPLIT_MAX = 4;          // row ranges a long posting list is split into, at most
@@ -1801,20 +1789,25 @@ cudaError_t launch_merge_rows32(const uint64_t* in, uint32_t nq, uint32_t P, uin
     return cudaGetLastError();
 }
 
+// A row matrix the scan kernels read, with what they need of it besides the rows: |x|^2 per row and the
+// TMA descriptors.  Set s keeps its max |x|^2 (f32 bits) in misc[4 * s].
+enum RowSetId : uint32_t { SET_ARENA, SET_CENTROIDS, SET_RECENT, SET_ASSIGN, N_ROW_SETS };
+struct RowSet {
+    Buf<float> xnorm;
+    CUtensorMap tmap;      // box 32 floats x 128 rows (kernel R), or x 64 rows for the centroid table (kernel Q)
+    CUtensorMap tmap_w;    // box 32 floats x W_NH rows (kernel W: each CTA of a pair streams half a tile)
+    const float* rows = nullptr;
+    uint64_t n = 0, version = ~0ull;
+};
+
 struct TcScratchImpl {
-    Buf<float> xnorm, qnorm;
-    Buf<uint32_t> misc;  // [0] = max |x|^2 bits
+    Buf<float> qnorm;
+    Buf<uint32_t> misc;  // [4 * s] = max |x|^2 bits of row set s
     Buf<unsigned long long> prof;
     Buf<uint32_t> list_order;  // lists by descending length (tile-scheduler order)
     Buf<uint32_t> live_ids;    // the non-empty lists, ascending (the bucketing pass walks only these)
     uint32_t n_live = 0;
-    struct RowSet {            // cached per scanned row matrix: |x|^2, TMA descriptor (box 32 x 128)
-        Buf<float> xnorm;
-        CUtensorMap tmap;
-        CUtensorMap tmap_w;    // box 32 floats x 32 rows (kernel W)
-        const float* rows = nullptr;
-        uint64_t n = 0, version = ~0ull;
-    } rs[2];                   // [0] recent tier, [1] centroid table (assignment)
+    RowSet sets[N_ROW_SETS];
     Buf<ScanItem> fitems;
     uint32_t list_order_n = 0;
     uint32_t max_list_len = 0;
@@ -1836,25 +1829,13 @@ struct TcScratchImpl {
         *out = ++stamp;
         return cudaSuccess;
     }
-    Buf<float> cnorm, dense;
+    Buf<float> dense;
     Buf<uint64_t> coarse;
     Buf<ScanItem> citems;
-    CUtensorMap tmap_cent;   // centroid table, box 32 floats x 64 rows
-    const float* tmap_cent_ptr = nullptr;
-    uint32_t tmap_cent_n = 0;
-    CUtensorMap tmap_arena;  // box 32 floats x 128 rows (kernel R)
-    CUtensorMap tmap_w;      // box 32 floats x 32 rows  (kernel W: each CTA of a pair streams half a tile)
     uint32_t smem_attr_set_w = 0;   // bit per metric instantiation of kernel W
     bool smem_attr_set_q = false;
-    const float* tmap_rows = nullptr;
-    uint64_t tmap_n = 0;
     uint32_t smem_attr_set_r = 0;   // bit per item width of kernel R
     bool smem_attr_set_rerank = false;
-    // experiment (FVDB_TC_FORK=1): kernel W of an IVF batch on a side stream, forked behind the bucketing and joined
-    // before the shortlist merge: its CTA pairs start wherever kernel R's CTAs have left an SM pair, instead of
-    // behind kernel R's slowest CTA
-    cudaStream_t side = nullptr;
-    cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
 };
 
 bool tc_supported(uint32_t D) { return D % 32 == 0 && D >= 32 && D <= TC_MAX_D; }
@@ -1876,14 +1857,12 @@ static cudaError_t rerank_prepare(TcScratchImpl* m) {
 void tc_release(TcScratch& s) {
     if (!s.impl) return;
     TcScratchImpl* m = s.impl;
-    m->xnorm.release(); m->qnorm.release(); m->misc.release(); m->thr_g.release(); m->list_cnt.release();
+    m->qnorm.release(); m->misc.release(); m->thr_g.release(); m->list_cnt.release();
     m->pair_off.release(); m->cursor.release(); m->pair_q.release(); m->pair_slot.release(); m->n_items.release();
     m->items.release(); m->items_w.release(); m->partial.release(); m->shortlist.release(); m->row_stamp.release();
-    m->prof.release(); m->list_order.release(); m->live_ids.release(); m->rs[0].xnorm.release(); m->rs[1].xnorm.release(); m->fitems.release();
-    m->cnorm.release(); m->dense.release(); m->coarse.release(); m->citems.release();
-    if (m->ev_fork) cudaEventDestroy(m->ev_fork);
-    if (m->ev_join) cudaEventDestroy(m->ev_join);
-    if (m->side) cudaStreamDestroy(m->side);
+    m->prof.release(); m->list_order.release(); m->live_ids.release(); m->fitems.release();
+    for (RowSet& rs : m->sets) rs.xnorm.release();
+    m->dense.release(); m->coarse.release(); m->citems.release();
     delete m;
     s.impl = nullptr;
 }
@@ -1898,21 +1877,29 @@ void tc_release(TcScratch& s) {
         }                                                                              \
     } while (0)
 
-// Which scan kernel(s): 'W' = kernel W for heavily probed lists and dense scans plus kernel R for the
-// sparsely probed lists (needs the query tile in tensor memory: D <= 384); 'R' (FVDB_TC_KERNEL=R, or
-// 384 < D <= TC_MAX_D) = kernel R alone
-static char tc_kernel_choice(uint32_t D, int sm_count) {
-    const char* kenv = getenv("FVDB_TC_KERNEL");
-    char c = (kenv && kenv[0] == 'R') ? 'R' : 'W';
-    if (c == 'W' && (D > 384 || sm_count < 2)) c = 'R';
-    return c;
+// Which scan kernel(s), as the least number of a batch's queries that puts a posting list on kernel W; 0 = kernel
+// R alone.  Kernel W (query tile in tensor memory: D <= 384, on SM pairs) takes the heavily probed lists and the
+// dense scans, kernel R the sparsely probed lists; above D = 384 kernel R scans alone.  Test hook, read on every
+// call: FVDB_TC_KERNEL=R puts every list on kernel R, FVDB_TC_KERNEL=W every list on kernel W where it exists.
+static uint32_t tc_kernel_choice(uint32_t D, int sm_count) {
+    if (D > 384 || sm_count < 2) return 0;
+    const char* e = getenv("FVDB_TC_KERNEL");
+    if (e && e[0] == 'R') return 0;
+    if (e && e[0] == 'W') return 1;
+    return TC_WIDE_MIN_QUERIES;
+}
+
+// FVDB_TC_DEBUG: the scan kernels' timing-only modes and per-role stopwatch (bit 7, dump_prof), and bit 9: keep
+// the previous batch's per-query bounds
+static uint32_t tc_debug_bits() {
+    const char* e = getenv("FVDB_TC_DEBUG");
+    return e ? (uint32_t)atoi(e) : 0u;
 }
 
 static cudaError_t launch_wide(TcScratchImpl* m, const CUtensorMap& tmap, TcScanParams& p, uint32_t KB, int sm_count,
                                size_t* dev_bytes, cudaStream_t st, cudaEvent_t ev0) {
     const uint32_t kbs = wide_pick_kbs(KB);
-    uint32_t stages = wide_pick_stages(KB, kbs);
-    if (const char* e = getenv("FVDB_TC_STAGES")) { const uint32_t v = (uint32_t)atoi(e); if (v >= 2 && v < stages) stages = v; }
+    const uint32_t stages = wide_pick_stages(KB, kbs);
     p.kbs = kbs;
     p.stages = stages;
     const size_t smem = tc_scan_wide_smem_bytes(stages, kbs) + 1024;
@@ -1992,64 +1979,72 @@ static CUresult encode_rows_tmap(CUtensorMap* out, const float* rows, uint64_t n
                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
 }
 
+// Brings row set `id` up to date with `rows` when the caller marks it stale or the rows moved: zeroes its max word,
+// launches row_norms_kernel once (|x|^2 per row and their max) and encodes its TMA descriptors.  *refreshed (when
+// given) tells whether it did.
+static int refresh_row_set(TcScratchImpl* m, RowSetId id, const float* rows, uint64_t n, uint32_t D, bool stale,
+                           int sm_count, cudaStream_t st, size_t* dev_bytes, uint32_t* launches, std::string* err,
+                           bool* refreshed = nullptr) {
+    RowSet& rs = m->sets[id];
+    if (refreshed) *refreshed = false;
+    if (!stale && rs.rows == rows && rs.n == n) return FVDB_OK;
+    uint32_t* max_bits = m->misc.p + 4 * id;
+    TCK(rs.xnorm.ensure(n, dev_bytes));
+    TCK(cudaMemsetAsync(max_bits, 0, 4, st));
+    const uint32_t blocks = (uint32_t)std::min<uint64_t>((n * 32 + 255) / 256, (uint64_t)sm_count * 16);
+    row_norms_kernel<<<blocks, 256, 0, st>>>(rows, n, D, rs.xnorm.p, max_bits);
+    TCK(cudaGetLastError());
+    (*launches)++;
+    // kernel Q alone reads the centroid table; kernels R and W read the other sets
+    CUresult r = encode_rows_tmap(&rs.tmap, rows, n, D, id == SET_CENTROIDS ? Q1_N : TC_ROWS);
+    if (r == CUDA_SUCCESS && id != SET_CENTROIDS) r = encode_rows_tmap(&rs.tmap_w, rows, n, D, W_NH);
+    if (r != CUDA_SUCCESS) {
+        if (err) *err = "cuTensorMapEncodeTiled failed with code " + std::to_string((int)r);
+        return FVDB_ERR_CUDA;
+    }
+    rs.rows = rows;
+    rs.n = n;
+    if (refreshed) *refreshed = true;
+    return FVDB_OK;
+}
+
 int tc_ivf_search(TcScratch& s, const TcSearchArgs& a, cudaStream_t st, size_t* dev_bytes, uint32_t* launches,
                   std::string* err) {
     if (!s.impl) s.impl = new TcScratchImpl();
     TcScratchImpl* m = s.impl;
     const uint32_t D = a.D, KB = D / 32, nq = a.nq, np = a.nprobe;
     if (a.n_rows >= 0x7FFFFFFFull) { if (err) *err = "arena too large for the TC path"; return FVDB_ERR_INVALID_ARG; }
+    const uint32_t debug = tc_debug_bits();
 
-    // ---- per-arena state: row norms, max norm, TMA descriptor ----
-    TCK(m->misc.ensure(16, dev_bytes));
-    if (!a.coarse_only && (s.arena_dirty || m->tmap_rows != a.rows || m->tmap_n != a.n_rows)) {
-        TCK(m->xnorm.ensure(a.n_rows, dev_bytes));
-        TCK(cudaMemsetAsync(m->misc.p, 0, 4, st));  // [0] = max |x|^2 bits; [4] = max |c|^2 bits (coarse)
-        const uint32_t blocks = (uint32_t)std::min<uint64_t>((a.n_rows * 32 + 255) / 256, (uint64_t)a.sm_count * 16);
-        row_norms_kernel<<<blocks, 256, 0, st>>>(a.rows, a.n_rows, D, m->xnorm.p, m->misc.p);
-        TCK(cudaGetLastError());
-        (*launches)++;
-        EncodeTiledFn enc = get_encode_fn();
-        if (!enc) { if (err) *err = "cuTensorMapEncodeTiled unavailable"; return FVDB_ERR_CUDA; }
-        const cuuint64_t gdim[2] = {D, a.n_rows};
-        const cuuint64_t gstride[1] = {(cuuint64_t)D * 4};
-        const cuuint32_t box[2] = {TC_KB_FLOATS, TC_ROWS};
-        const cuuint32_t estr[2] = {1, 1};
-        CUresult r = enc(&m->tmap_arena, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(a.rows), gdim, gstride,
-                         box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                         CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) {
-            if (err) *err = "cuTensorMapEncodeTiled failed with code " + std::to_string((int)r);
-            return FVDB_ERR_CUDA;
-        }
-        if (encode_rows_tmap(&m->tmap_w, a.rows, a.n_rows, D, W_NH) != CUDA_SUCCESS) {
-            if (err) *err = "cuTensorMapEncodeTiled (kernel W) failed";
-            return FVDB_ERR_CUDA;
-        }
-        {
-            // longest-list-first order for the dynamic tile scheduler (once per arena layout)
-            std::vector<uint32_t> off(a.nlist + 1), order(a.nlist);
-            TCK(cudaMemcpyAsync(off.data(), a.list_off, (size_t)(a.nlist + 1) * 4, cudaMemcpyDeviceToHost, st));
-            TCK(cudaStreamSynchronize(st));
-            m->max_list_len = 0;
-            for (uint32_t l = 0; l < a.nlist; ++l) m->max_list_len = std::max(m->max_list_len, off[l + 1] - off[l]);
-            for (uint32_t l = 0; l < a.nlist; ++l) order[l] = l;
-            std::stable_sort(order.begin(), order.end(), [&](uint32_t x, uint32_t y) {
-                return off[x + 1] - off[x] > off[y + 1] - off[y];
-            });
-            TCK(m->list_order.ensure(a.nlist, dev_bytes));
-            TCK(cudaMemcpyAsync(m->list_order.p, order.data(), (size_t)a.nlist * 4, cudaMemcpyHostToDevice, st));
-            // the non-empty lists in id order (a shard of a list-sharded index owns 1 / world of them)
-            std::vector<uint32_t> live;
-            for (uint32_t l = 0; l < a.nlist; ++l) if (off[l + 1] > off[l]) live.push_back(l);
-            m->n_live = (uint32_t)live.size();
-            TCK(m->live_ids.ensure(std::max<size_t>(live.size(), 1), dev_bytes));
-            if (!live.empty()) TCK(cudaMemcpyAsync(m->live_ids.p, live.data(), live.size() * 4, cudaMemcpyHostToDevice, st));
-            TCK(cudaStreamSynchronize(st));
-            m->list_order_n = a.nlist;
-        }
-        m->tmap_rows = a.rows;
-        m->tmap_n = a.n_rows;
+    TCK(m->misc.ensure(4 * N_ROW_SETS, dev_bytes));
+    bool arena_refreshed = false;
+    if (!a.coarse_only) {
+        const int r = refresh_row_set(m, SET_ARENA, a.rows, a.n_rows, D, s.arena_dirty, a.sm_count, st, dev_bytes,
+                                      launches, err, &arena_refreshed);
+        if (r != FVDB_OK) return r;
         s.arena_dirty = false;
+    }
+    if (arena_refreshed) {
+        // longest-list-first order for the dynamic tile scheduler (once per arena layout)
+        std::vector<uint32_t> off(a.nlist + 1), order(a.nlist);
+        TCK(cudaMemcpyAsync(off.data(), a.list_off, (size_t)(a.nlist + 1) * 4, cudaMemcpyDeviceToHost, st));
+        TCK(cudaStreamSynchronize(st));
+        m->max_list_len = 0;
+        for (uint32_t l = 0; l < a.nlist; ++l) m->max_list_len = std::max(m->max_list_len, off[l + 1] - off[l]);
+        for (uint32_t l = 0; l < a.nlist; ++l) order[l] = l;
+        std::stable_sort(order.begin(), order.end(), [&](uint32_t x, uint32_t y) {
+            return off[x + 1] - off[x] > off[y + 1] - off[y];
+        });
+        TCK(m->list_order.ensure(a.nlist, dev_bytes));
+        TCK(cudaMemcpyAsync(m->list_order.p, order.data(), (size_t)a.nlist * 4, cudaMemcpyHostToDevice, st));
+        // the non-empty lists in id order (a shard of a list-sharded index owns 1 / world of them)
+        std::vector<uint32_t> live;
+        for (uint32_t l = 0; l < a.nlist; ++l) if (off[l + 1] > off[l]) live.push_back(l);
+        m->n_live = (uint32_t)live.size();
+        TCK(m->live_ids.ensure(std::max<size_t>(live.size(), 1), dev_bytes));
+        if (!live.empty()) TCK(cudaMemcpyAsync(m->live_ids.p, live.data(), live.size() * 4, cudaMemcpyHostToDevice, st));
+        TCK(cudaStreamSynchronize(st));
+        m->list_order_n = a.nlist;
     }
 
     // ---- per-batch state ----
@@ -2060,27 +2055,19 @@ int tc_ivf_search(TcScratch& s, const TcSearchArgs& a, cudaStream_t st, size_t* 
     // parallel.  Kernel R (items of up to 64 queries, query tile in shared memory, rows on the accumulator lanes,
     // candidate handling shared by the 128 row threads) takes the sparsely probed lists, where its MMA
     // cost (proportional to the queries of the item) and its cooperative epilogue are the cheaper ones.
-    const char kch = tc_kernel_choice(D, a.sm_count);
-    uint32_t wide_min = 0;                       // 0: kernel R only
-    if (kch == 'W') {
-        wide_min = TC_WIDE_MIN_QUERIES;
-        if (const char* e = getenv("FVDB_TC_WIDE_MIN")) wide_min = (uint32_t)std::max(1, atoi(e));
-    }
+    const uint32_t wide_min = tc_kernel_choice(D, a.sm_count);   // 0: kernel R only
     const bool use_wide = wide_min != 0;
     const uint32_t tile_q = r2_tile_q(D);   // kernel R's items; a list probed by more queries becomes several
     // Long posting lists are cut into row ranges (one work item and one shortlist slot each): a hub
     // list of 9 K rows probed by 64 queries is otherwise ONE item of 71 tiles — a third of the whole
     // scan on one SM, and the tail every other SM waits for.  At most TC_SPLIT_MAX ranges per list.
     uint32_t n_split = 1, rows_cap = 0;
-    {
-        uint32_t want = TC_SPLIT_MAX;
-        if (const char* e = getenv("FVDB_TC_SPLIT")) want = std::min<uint32_t>(std::max(1, atoi(e)), 16u);
+    if (m->max_list_len > TC_SPLIT_MIN_ROWS) {
         const uint32_t unit = (uint32_t)R2_ROWS;   // a multiple of both kernels' tile heights
-        if (want > 1 && m->max_list_len > TC_SPLIT_MIN_ROWS) {
-            rows_cap = std::max<uint32_t>(TC_SPLIT_MIN_ROWS / 2, ((m->max_list_len + want - 1) / want + unit - 1) / unit * unit);
-            n_split = (m->max_list_len + rows_cap - 1) / rows_cap;
-            if (n_split <= 1) { n_split = 1; rows_cap = 0; }
-        }
+        rows_cap = std::max<uint32_t>(TC_SPLIT_MIN_ROWS / 2,
+                                      ((m->max_list_len + TC_SPLIT_MAX - 1) / TC_SPLIT_MAX + unit - 1) / unit * unit);
+        n_split = (m->max_list_len + rows_cap - 1) / rows_cap;
+        if (n_split <= 1) { n_split = 1; rows_cap = 0; }
     }
     // shortlist rows per (query, probe): one per row range, times two when kernel W takes part (each
     // half of its tiles publishes its own row; kernel R writes row `range` of the same block)
@@ -2105,8 +2092,7 @@ int tc_ivf_search(TcScratch& s, const TcSearchArgs& a, cudaStream_t st, size_t* 
         // query norms; the same pass resets the per-query bounds (unless the caller shares an array it
         // has reset itself) and raises the batch's NaN flag
         // experiment (FVDB_TC_DEBUG bit 9): keep the previous batch's bounds = perfectly seeded thresholds
-        const char* dbg = getenv("FVDB_TC_DEBUG");
-        const bool reset_bounds = !(dbg && (atoi(dbg) & 512)) && !a.thr_ext;
+        const bool reset_bounds = !(debug & 512u) && !a.thr_ext;
         row_norms_kernel<<<blocks, 256, 0, st>>>(a.Q, nq, D, m->qnorm.p, nullptr, reset_bounds ? m->thr_g.p : nullptr,
                                                  F32_INF_BITS, a.d_nan);
         TCK(cudaGetLastError());
@@ -2115,26 +2101,10 @@ int tc_ivf_search(TcScratch& s, const TcSearchArgs& a, cudaStream_t st, size_t* 
     const uint64_t* coarse_keys = a.coarse_keys;
     if (!coarse_keys) {
         if (D > 384 || np > TC_MAX_NPROBE_COARSE) { if (err) *err = "TC coarse step unsupported for this shape"; return FVDB_ERR_INVALID_ARG; }
-        // centroid norms + TMA descriptor of the centroid table
-        if (s.centroids_dirty || m->tmap_cent_ptr != a.centroids || m->tmap_cent_n != a.nlist) {
-            TCK(m->cnorm.ensure(a.nlist, dev_bytes));
-            TCK(cudaMemsetAsync(m->misc.p + 4, 0, 4, st));
-            const uint32_t blocks = (uint32_t)std::min<uint64_t>(((uint64_t)a.nlist * 32 + 255) / 256, (uint64_t)a.sm_count * 8);
-            row_norms_kernel<<<blocks, 256, 0, st>>>(a.centroids, a.nlist, D, m->cnorm.p, m->misc.p + 4);
-            TCK(cudaGetLastError());
-            (*launches)++;
-            EncodeTiledFn enc = get_encode_fn();
-            if (!enc) { if (err) *err = "cuTensorMapEncodeTiled unavailable"; return FVDB_ERR_CUDA; }
-            const cuuint64_t gdim[2] = {D, a.nlist};
-            const cuuint64_t gstride[1] = {(cuuint64_t)D * 4};
-            const cuuint32_t box[2] = {TC_KB_FLOATS, Q1_N};
-            const cuuint32_t estr[2] = {1, 1};
-            CUresult r = enc(&m->tmap_cent, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(a.centroids), gdim,
-                             gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                             CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-            if (r != CUDA_SUCCESS) { if (err) *err = "cuTensorMapEncodeTiled (centroids) failed"; return FVDB_ERR_CUDA; }
-            m->tmap_cent_ptr = a.centroids;
-            m->tmap_cent_n = a.nlist;
+        {
+            const int r = refresh_row_set(m, SET_CENTROIDS, a.centroids, a.nlist, D, s.centroids_dirty, a.sm_count, st,
+                                          dev_bytes, launches, err);
+            if (r != FVDB_OK) return r;
             s.centroids_dirty = false;
         }
         const uint32_t ld = (a.nlist + 63) / 64 * 64;
@@ -2152,7 +2122,7 @@ int tc_ivf_search(TcScratch& s, const TcSearchArgs& a, cudaStream_t st, size_t* 
         TCK(cudaGetLastError());
         TcScanParams cp{};
         cp.items = m->citems.p; cp.item_count = m->n_items.p + 2; cp.Q = a.Q; cp.qnorm = m->qnorm.p; cp.D = D; cp.KB = KB;
-        cp.xnorm = m->cnorm.p; cp.ids = nullptr; cp.P = 1; cp.partial = nullptr; cp.thr_g = nullptr;
+        cp.xnorm = m->sets[SET_CENTROIDS].xnorm.p; cp.ids = nullptr; cp.P = 1; cp.partial = nullptr; cp.thr_g = nullptr;
         cp.work_counter = m->n_items.p + 3;
         TCK(cudaMemsetAsync(cp.work_counter, 0, 4, st));
         cp.dense_out = m->dense.p; cp.dense_ld = ld;
@@ -2165,7 +2135,7 @@ int tc_ivf_search(TcScratch& s, const TcSearchArgs& a, cudaStream_t st, size_t* 
             m->smem_attr_set_q = true;
         }
         tc_scan_q_kernel<<<std::min<uint32_t>((uint32_t)a.sm_count, n_citems), TC_THREADS,
-                           tc_scan_q_smem_bytes(stages, kbs) + 1024, st>>>(m->tmap_cent, cp);
+                           tc_scan_q_smem_bytes(stages, kbs) + 1024, st>>>(m->sets[SET_CENTROIDS].tmap, cp);
         TCK(cudaGetLastError());
         // candidate set: nprobe + 32 (the proof needs the next approx value to clear the exact
         // nprobe-th by the TF32 bound; centroid distances are dense, so a generous margin)
@@ -2174,7 +2144,7 @@ int tc_ivf_search(TcScratch& s, const TcSearchArgs& a, cudaStream_t st, size_t* 
         TCK(rerank_prepare(m));
         // 8 local entries per thread: P(one thread holds >= 8 of the KC nearest) is negligible
         coarse_select_kernel<8><<<nq, 128, sel_smem, st>>>(m->dense.p, ld, a.centroids, a.Q, m->qnorm.p,
-                                                          m->misc.p + 4, nq, a.nlist, D, np, KC,
+                                                          m->misc.p + 4 * SET_CENTROIDS, nq, a.nlist, D, np, KC,
                                                           m->coarse.p, a.d_fallback_count, a.d_fallback_idx);
         TCK(cudaGetLastError());
         (*launches) += 3;
@@ -2184,10 +2154,9 @@ int tc_ivf_search(TcScratch& s, const TcSearchArgs& a, cudaStream_t st, size_t* 
     if (a.coarse_only) return FVDB_OK;
     TCK(launch_probe_bucketing(coarse_keys, nq, np, a.list_off, a.nlist, tile_q, m->list_cnt.p, m->pair_off.p,
                                m->cursor.p, m->pair_q.p, m->pair_slot.p, m->items.p, m->n_items.p, a.d_scanned_rows, st,
-                               (m->list_order_n == a.nlist && !getenv("FVDB_TC_NO_ORDER")) ? m->list_order.p : nullptr,
-                               getenv("FVDB_TC_ORDER_NEAR") != nullptr, rows_cap, wide_min, (uint32_t)W_NQ,
-                               use_wide ? m->items_w.p : nullptr, m->n_items.p + 6, getenv("FVDB_TC_W_ORDER") != nullptr,
-                               (m->list_order_n == a.nlist && !getenv("FVDB_TC_NO_ORDER")) ? m->live_ids.p : nullptr, m->n_live));
+                               m->list_order_n == a.nlist ? m->list_order.p : nullptr, rows_cap, wide_min, (uint32_t)W_NQ,
+                               use_wide ? m->items_w.p : nullptr, m->n_items.p + 6,
+                               m->list_order_n == a.nlist ? m->live_ids.p : nullptr, m->n_live));
     (*launches) += 3;
     uint32_t stamp = 0;
     TCK(m->next_stamp(n_pairs * prows, dev_bytes, st, &stamp));
@@ -2195,61 +2164,26 @@ int tc_ivf_search(TcScratch& s, const TcSearchArgs& a, cudaStream_t st, size_t* 
     // ---- the scan ----
     TcScanParams p{};
     p.items = m->items.p; p.item_count = m->n_items.p; p.pair_q = m->pair_q.p; p.pair_slot = m->pair_slot.p;
-    p.Q = a.Q; p.qnorm = m->qnorm.p; p.D = D; p.KB = KB; p.xnorm = m->xnorm.p; p.ids = a.ids;
+    p.Q = a.Q; p.qnorm = m->qnorm.p; p.D = D; p.KB = KB; p.xnorm = m->sets[SET_ARENA].xnorm.p; p.ids = a.ids;
     p.tomb = a.tomb; p.tomb_bits = a.tomb_bits; p.filt = a.filt; p.filt_bits = a.filt_bits;
     p.P = np; p.S = prows; p.partial = m->partial.p; p.thr_g = a.thr_ext ? a.thr_ext : m->thr_g.p;
     p.row_stamp = m->row_stamp.p; p.stamp = stamp;
     p.n_peer = a.thr_ext ? std::min(a.n_peers, TC_MAX_PEERS) : 0u;
     for (uint32_t r = 0; r < p.n_peer; ++r) p.thr_peer[r] = a.thr_peers[r];
-    p.rows_raw = a.rows; p.rows_bytes = a.n_rows * (uint64_t)D * 4;
     p.work_counter = m->n_items.p + 1;
-    {
-        const char* dbg = getenv("FVDB_TC_DEBUG");
-        p.debug = dbg ? (uint32_t)atoi(dbg) : 0u;
-    }
-    const bool wide_first_env = [] { const char* oe = getenv("FVDB_TC_ORDER"); return oe && oe[0] == 'W'; }();
-    // opt-in experiment (FVDB_TC_FORK=1): measured 0.4045 -> 0.391 ms for the two scan kernels, but 0.468 -> 0.476 ms
-    // per pipelined batch — the gaps kernel W now fills were where the neighbouring batches' small kernels ran
-    const bool fork_wide = use_wide && !wide_first_env && !(p.debug & 128u) && getenv("FVDB_TC_FORK") != nullptr;
-    if (fork_wide && !m->side) {
-        TCK(cudaStreamCreateWithFlags(&m->side, cudaStreamNonBlocking));
-        TCK(cudaEventCreateWithFlags(&m->ev_fork, cudaEventDisableTiming));
-        TCK(cudaEventCreateWithFlags(&m->ev_join, cudaEventDisableTiming));
-    }
+    p.debug = debug;
     p.scan_sms = a.scan_sms;
     TCK(cudaMemsetAsync(p.work_counter, 0, 4, st));
     if (use_wide) TCK(cudaMemsetAsync(m->n_items.p + 7, 0, 4, st));   // kernel W's work counter
     if (a.wait_before_scan) TCK(cudaStreamWaitEvent(st, a.wait_before_scan, 0));
     if (a.ev_scan0) TCK(cudaEventRecord(a.ev_scan0, st));
-    if (fork_wide) TCK(cudaEventRecord(m->ev_fork, st));
-    auto run_wide = [&]() -> int {
-    if (use_wide) {
-        TcScanParams pw = p;
-        pw.items = m->items_w.p; pw.item_count = m->n_items.p + 6; pw.work_counter = m->n_items.p + 7;
-        if (fork_wide) {
-            // `st` holds kernel R by now (launched just before): kernel W goes to the side stream, ordered
-            // behind everything R itself was ordered behind
-            TCK(cudaStreamWaitEvent(m->side, m->ev_fork, 0));
-            TCK(launch_wide(m, m->tmap_w, pw, KB, a.sm_count, dev_bytes, m->side, nullptr));
-            TCK(cudaEventRecord(m->ev_join, m->side));
-            TCK(cudaStreamWaitEvent(st, m->ev_join, 0));
-        } else {
-            TCK(launch_wide(m, m->tmap_w, pw, KB, a.sm_count, dev_bytes, st, nullptr));
-        }
-        (*launches)++;
-    }
-    return FVDB_OK;
-    };
-    auto run_narrow = [&]() -> int {
+    // Order: the sparsely probed lists first (kernel R), then the hub lists (kernel W).  Every query probes
+    // mostly sparse lists; after their scan its bound is already close to final, so the hub items — where a
+    // candidate is the expensive thing (one thread per query) — start warm.
     {
         size_t smem = 0;
-        uint32_t stages = r2_pick_stages(D, &smem);
+        p.stages = r2_pick_stages(D, &smem);
         if (!smem) { if (err) *err = "TC scan does not fit shared memory for this dim"; return FVDB_ERR_INVALID_CONFIG; }
-        if (const char* e = getenv("FVDB_TC_STAGES")) {
-            const uint32_t v = (uint32_t)atoi(e);
-            if (v >= 2 && v < stages) { stages = v; smem = tc_scan_smem_bytes(KB, stages, tile_q) + R2_SLACK; }
-        }
-        p.stages = stages;
         uint32_t grid = (uint32_t)std::min<size_t>((size_t)a.sm_count, max_items);
         if (p.scan_sms && p.scan_sms < grid) grid = p.scan_sms;
         if (p.debug & 128u) {
@@ -2257,19 +2191,14 @@ int tc_ivf_search(TcScratch& s, const TcSearchArgs& a, cudaStream_t st, size_t* 
             TCK(cudaMemsetAsync(m->prof.p, 0, (size_t)grid * 48 * 8, st));
             p.prof = m->prof.p;
         }
-        TCK(launch_r2(m, m->tmap_arena, p, grid, smem, st));
+        TCK(launch_r2(m, m->sets[SET_ARENA].tmap, p, grid, smem, st));
         if (p.prof) TCK(dump_prof(m->prof.p, grid, st));
     }
-    return FVDB_OK;
-    };
-    // Order: the sparsely probed lists first (kernel R), then the hub lists (kernel W).  Every query probes
-    // mostly sparse lists; after their scan its bound is already close to final, so the hub items — where a
-    // candidate is the expensive thing (one thread per query) — start warm.  FVDB_TC_ORDER=WR reverses it.
-    {
-        const bool wide_first = wide_first_env;
-        if (wide_first) { int r = run_wide(); if (r != FVDB_OK) return r; }
-        { int r = run_narrow(); if (r != FVDB_OK) return r; }
-        if (!wide_first) { int r = run_wide(); if (r != FVDB_OK) return r; }
+    if (use_wide) {
+        TcScanParams pw = p;
+        pw.items = m->items_w.p; pw.item_count = m->n_items.p + 6; pw.work_counter = m->n_items.p + 7;
+        TCK(launch_wide(m, m->sets[SET_ARENA].tmap_w, pw, KB, a.sm_count, dev_bytes, st, nullptr));
+        (*launches)++;
     }
     if (a.ev_scan1) TCK(cudaEventRecord(a.ev_scan1, st));
     if (a.record_after_scan) TCK(cudaEventRecord(a.record_after_scan, st));
@@ -2278,7 +2207,7 @@ int tc_ivf_search(TcScratch& s, const TcSearchArgs& a, cudaStream_t st, size_t* 
     // ---- merge the per-(query, probe) shortlists, exact re-rank, proof ----
     TCK(launch_merge_rows32(m->partial.p, nq, np * prows, m->shortlist.p, st, m->row_stamp.p, stamp));
     TCK(rerank_prepare(m));
-    rerank_kernel<METRIC_L2><<<(nq + 3) / 4, 128, rerank_smem_bytes(D), st>>>(m->shortlist.p, a.rows, a.ids, a.Q, m->qnorm.p, m->misc.p, nq, D, a.k, (uint32_t)TC_KP,
+    rerank_kernel<METRIC_L2><<<(nq + 3) / 4, 128, rerank_smem_bytes(D), st>>>(m->shortlist.p, a.rows, a.ids, a.Q, m->qnorm.p, m->misc.p + 4 * SET_ARENA, nq, D, a.k, (uint32_t)TC_KP,
                                                a.xmax_floor_sq, a.out_keys, a.d_fallback_count, a.d_fallback_idx, a.fin_ids, a.fin_dist, a.fin_count);
     TCK(cudaGetLastError());
     (*launches) += 2;
@@ -2291,39 +2220,19 @@ int tc_flat_search(TcScratch& s, const TcFlatArgs& a, cudaStream_t st, size_t* d
     TcScratchImpl* m = s.impl;
     const uint32_t D = a.D, KB = D / 32, nq = a.nq;
     if (a.n_rows >= 0x7FFFFFFFull) { if (err) *err = "flat tier too large for the TC path"; return FVDB_ERR_INVALID_ARG; }
-    TCK(m->misc.ensure(16, dev_bytes));
-    // ---- per-row-set state: row norms, max norm (misc[8] / misc[12]), TMA descriptor ----
-    TcScratchImpl::RowSet& rs = m->rs[a.state ? 1 : 0];
-    uint32_t* xmax_bits = m->misc.p + (a.state ? 12 : 8);
-    const bool stale = a.state ? (rs.version != a.version) : s.flat_dirty;
-    if (stale || rs.rows != a.rows || rs.n != a.n_rows) {
-        TCK(rs.xnorm.ensure(a.n_rows, dev_bytes));
-        TCK(cudaMemsetAsync(xmax_bits, 0, 4, st));
-        const uint32_t blocks = (uint32_t)std::min<uint64_t>((a.n_rows * 32 + 255) / 256, (uint64_t)a.sm_count * 16);
-        row_norms_kernel<<<blocks, 256, 0, st>>>(a.rows, a.n_rows, D, rs.xnorm.p, xmax_bits);
-        TCK(cudaGetLastError());
-        (*launches)++;
-        EncodeTiledFn enc = get_encode_fn();
-        if (!enc) { if (err) *err = "cuTensorMapEncodeTiled unavailable"; return FVDB_ERR_CUDA; }
-        const cuuint64_t gdim[2] = {D, a.n_rows};
-        const cuuint64_t gstride[1] = {(cuuint64_t)D * 4};
-        const cuuint32_t box[2] = {TC_KB_FLOATS, TC_ROWS};
-        const cuuint32_t estr[2] = {1, 1};
-        CUresult r = enc(&rs.tmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(a.rows), gdim, gstride,
-                         box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                         CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) { if (err) *err = "cuTensorMapEncodeTiled (row set) failed"; return FVDB_ERR_CUDA; }
-        if (encode_rows_tmap(&rs.tmap_w, a.rows, a.n_rows, D, W_NH) != CUDA_SUCCESS) {
-            if (err) *err = "cuTensorMapEncodeTiled (row set, kernel W) failed";
-            return FVDB_ERR_CUDA;
-        }
-        rs.rows = a.rows;
-        rs.n = a.n_rows;
+    TCK(m->misc.ensure(4 * N_ROW_SETS, dev_bytes));
+    const RowSetId id = a.state ? SET_ASSIGN : SET_RECENT;
+    RowSet& rs = m->sets[id];
+    uint32_t* xmax_bits = m->misc.p + 4 * id;
+    {
+        const bool stale = a.state ? (rs.version != a.version) : s.flat_dirty;
+        const int r = refresh_row_set(m, id, a.rows, a.n_rows, D, stale, a.sm_count, st, dev_bytes, launches, err);
+        if (r != FVDB_OK) return r;
         rs.version = a.version;
         if (!a.state) s.flat_dirty = false;
     }
     // ---- work items: every query group (256 queries for kernel W, 64 for kernel R) against every row chunk ----
-    const bool use_wide = tc_kernel_choice(D, a.sm_count) == 'W';
+    const bool use_wide = tc_kernel_choice(D, a.sm_count) != 0;
     if (a.metric != METRIC_L2 && !use_wide) { if (err) *err = "cosine / dot scans need kernel W (dim <= 384)"; return FVDB_ERR_INVALID_CONFIG; }
     const uint32_t tile_q = use_wide ? (uint32_t)W_NQ : r2_tile_q(D);
     const uint32_t tile_rows = use_wide ? (uint32_t)W_N : (uint32_t)TC_ROWS;
@@ -2361,12 +2270,9 @@ int tc_flat_search(TcScratch& s, const TcFlatArgs& a, cudaStream_t st, size_t* d
     p.P = n_chunks; p.S = use_wide ? frows : 0u; p.partial = m->partial.p; p.thr_g = m->thr_g.p;
     p.row_stamp = m->row_stamp.p; p.stamp = stamp;
     p.metric = a.metric; p.xmax_bits = xmax_bits;
-    p.small_list = (a.k == 1 && a.rerank_r && a.rerank_r + 1 <= (uint32_t)W_SMALL_N && !getenv("FVDB_ASSIGN_HEAP")) ? 1u : 0u;
+    p.small_list = (a.k == 1 && a.rerank_r && a.rerank_r + 1 <= (uint32_t)W_SMALL_N) ? 1u : 0u;
     p.work_counter = m->n_items.p + 5;
-    {
-        const char* dbg = getenv("FVDB_TC_DEBUG");
-        p.debug = dbg ? (uint32_t)atoi(dbg) : 0u;
-    }
+    p.debug = tc_debug_bits();
     TCK(cudaMemsetAsync(p.work_counter, 0, 4, st));
     if (a.ev_scan0 && !use_wide) TCK(cudaEventRecord(a.ev_scan0, st));
     if (use_wide) {
@@ -2385,7 +2291,7 @@ int tc_flat_search(TcScratch& s, const TcFlatArgs& a, cudaStream_t st, size_t* d
     rr<<<(nq + 3) / 4, 128, rerank_smem_bytes(D), st>>>(m->shortlist.p, a.rows, a.ids, a.Q, m->qnorm.p, xmax_bits, nq, D, a.k,
                                                         a.rerank_r ? a.rerank_r : (uint32_t)TC_KP, 0.0f, a.out_keys,
                                                         a.d_fallback_count, a.d_fallback_idx, nullptr, nullptr, nullptr,
-                                                        (a.argmin_only && a.k == 1 && !getenv("FVDB_ASSIGN_RERANK_ALL")) ? 1u : 0u);
+                                                        (a.argmin_only && a.k == 1) ? 1u : 0u);
     TCK(cudaGetLastError());
     (*launches) += 3;
     return FVDB_OK;

@@ -607,10 +607,8 @@ def test_hub_list_is_split_into_row_ranges(kernel, monkeypatch):
     item and one shortlist slot each (DESIGN §3.1).  Results — with tombstones and a filter bitmap on —
     must equal the oracle's bit for bit: with kernel R alone, with kernel W alone (every list goes to the
     wide-tile kernel) and with the product's split (the hub list to kernel W, the others to kernel R)."""
-    if kernel == "R":
-        monkeypatch.setenv("FVDB_TC_KERNEL", "R")
-    elif kernel == "W":
-        monkeypatch.setenv("FVDB_TC_WIDE_MIN", "1")
+    if kernel != "hybrid":
+        monkeypatch.setenv("FVDB_TC_KERNEL", kernel)
     rng = np.random.default_rng(77)
     d, nlist, nq, k, nprobe = 128, 12, 150, 10, 6
     cents = rng.standard_normal((nlist, d)).astype(np.float32)

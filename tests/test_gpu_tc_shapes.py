@@ -162,7 +162,7 @@ def _variants(d):
         return [("default", {}, (K_R,), (K_W, K_Q)), ("R", {"FVDB_TC_KERNEL": "R"}, (K_R,), (K_W, K_Q))]
     return [("default", {}, (K_R, K_W, K_Q), ()),       # hub + its neighbours to W, the rest to R
             ("R", {"FVDB_TC_KERNEL": "R"}, (K_R, K_Q), (K_W,)),
-            ("W", {"FVDB_TC_WIDE_MIN": "1"}, (K_W, K_Q), ())]
+            ("W", {"FVDB_TC_KERNEL": "W"}, (K_W, K_Q), ())]
 
 
 @pytest.mark.parametrize("d", DIMS)
@@ -177,8 +177,7 @@ def test_ivf_dimension_sweep(d, monkeypatch):
         want_f = O.hybrid_batch_search(ivf, None, None, q, k, nprobe, tiers=2,
                                        deleted=O.make_bitmap(int(ids.max()) + 1, dele), filter_bits=fbits)
     for name, env, expect, absent in _variants(d):
-        for key in ("FVDB_TC_KERNEL", "FVDB_TC_WIDE_MIN"):
-            monkeypatch.delenv(key, raising=False)
+        monkeypatch.delenv("FVDB_TC_KERNEL", raising=False)
         for key, val in env.items():
             monkeypatch.setenv(key, val)
         got = _run_tc(eng, lambda: eng.search(q, k, nprobe, tiers=L.TIER_HISTORICAL), NQ, expect, absent)
@@ -326,7 +325,7 @@ def _flood_case():
 
 @pytest.mark.parametrize("kernel", ["R", "W"])
 def test_candidate_floods(kernel, monkeypatch):
-    monkeypatch.setenv(*(("FVDB_TC_KERNEL", "R") if kernel == "R" else ("FVDB_TC_WIDE_MIN", "1")))
+    monkeypatch.setenv("FVDB_TC_KERNEL", kernel)
     d, x, ids, q, cents = _flood_case()
     k = 10
     eng = _tc_engine(d)
