@@ -344,6 +344,23 @@ static inline void mark_centroids_dirty(fvdb_index* h) {
     h->scratch.tc.centroids_dirty = true;
     for (auto& sl : h->slots) sl.b.tc.centroids_dirty = true;
 }
+static inline void mark_flat_dirty(fvdb_index* h) {
+    h->scratch.tc.flat_dirty = true;
+    for (auto& sl : h->slots) sl.b.tc.flat_dirty = true;
+}
+// dev_bytes counts the device buffers the handle owns.  A buffer a step fills on the side is not counted until
+// adopt() puts it in place of an owned one (which is then freed with `fresh`); release() frees an owned buffer.
+template <typename T>
+static void adopt(fvdb_index* h, DevBuf<T>& buf, DevBuf<T>& fresh) {
+    h->dev_bytes += fresh.cap * sizeof(T);
+    h->dev_bytes -= buf.cap * sizeof(T);
+    buf.swap(fresh);
+}
+template <typename T>
+static void release(fvdb_index* h, DevBuf<T>& buf) {
+    h->dev_bytes -= buf.cap * sizeof(T);
+    buf.release();
+}
 // Every batch still running in a pipeline slot has to finish before anything it reads may move.
 static inline void quiesce_slots(fvdb_index* h) {
     for (auto& sl : h->slots)
@@ -449,6 +466,73 @@ int scan_all_exact(fvdb_index* h, const float* X, const uint32_t* ids, uint64_t 
     return FVDB_OK;
 }
 
+// ---- regrouping the row tiers --------------------------------------------------------------
+// Seal, vacuum, a list-sharded add, take-unowned and move-to-IVF each reorder a tier the same way: u32 keys, one
+// stable grouping (group_keys), gathers into exact-size buffers (gather), and those buffers adopted in place of
+// the tier's.  The grouping is stable, so the rows of a list stay in insertion order (DESIGN §2).  Nothing is
+// committed to the handle until every allocation of the step has succeeded.
+
+// Stable grouping of n keys into nkeys groups, keys >= nkeys dropped (they follow the groups): the permutation
+// goes to h->s_perm, the nkeys + 2 group offsets to h->s_u32c, and offset words [first, first + count) come back
+// to `out`.
+int group_keys(fvdb_index* h, const uint32_t* keys, uint64_t n, uint32_t nkeys, uint32_t first, uint32_t count,
+               uint32_t* out, cudaStream_t st) {
+    CK(h->s_perm.ensure(n, 0, st, &h->dev_bytes));
+    CK(h->s_group.ensure(stable_group_scratch_bytes(n, nkeys), 0, st, &h->dev_bytes));
+    CK(h->s_u32c.ensure(nkeys + 2, 0, st, &h->dev_bytes));
+    CK(launch_stable_group(keys, n, nkeys, h->s_u32c.p, h->s_perm.p, h->s_group.p, st));
+    CK(cudaMemcpyAsync(out, h->s_u32c.p + first, (size_t)count * 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    return FVDB_OK;
+}
+
+// One row set as a gather reads it: rows [n x D], ids [n] and, in the IVF tier, lists [n].
+struct Rows {
+    const float* x;
+    const uint32_t* ids;
+    const uint32_t* lists;
+};
+Rows arena(const fvdb_index* h) { return {h->ivf_rows.p, h->ivf_ids.p, h->ivf_list.p}; }
+Rows flat_tier(const fvdb_index* h) { return {h->flat_rows.p, h->flat_ids.p, nullptr}; }
+
+// Row i < m of the destination = row perm[i] of `a` (perm[i] < na) or row perm[i] - na of `b`; lists are gathered
+// when `lists` is given.
+int gather(fvdb_index* h, Rows a, uint64_t na, Rows b, const uint32_t* perm, uint64_t m, float* x, uint32_t* ids,
+           uint32_t* lists, cudaStream_t st) {
+    CK(launch_gather_rows(a.x, na, b.x, perm, m, h->dim, x, st));
+    CK(launch_gather_u32(a.ids, na, b.ids, perm, m, ids, st));
+    if (lists) CK(launch_gather_u32(a.lists, na, b.lists, perm, m, lists, st));
+    return FVDB_OK;
+}
+
+// Exact-size buffers of m rows (at least one) that a regrouping fills before they are adopted.
+struct NewRows {
+    DevBuf<float> x;
+    DevBuf<uint32_t> ids, lists;
+};
+int alloc_rows(fvdb_index* h, NewRows& f, uint64_t m, bool lists, cudaStream_t st) {
+    m = std::max<uint64_t>(m, 1);
+    CK(f.x.ensure((size_t)m * h->dim, 0, st, nullptr, true));
+    CK(f.ids.ensure(m, 0, st, nullptr, true));
+    if (lists) CK(f.lists.ensure(m, 0, st, nullptr, true));
+    return FVDB_OK;
+}
+
+// The `kept` gathered rows become the IVF arena.  h->s_u32c holds the grouping that ordered them, with lists
+// 0..nlist-1 as its first groups; list_off takes their offsets and, in word nlist + 1, the end of the arena.
+int adopt_arena(fvdb_index* h, NewRows& f, uint64_t kept, cudaStream_t st) {
+    const uint32_t nl = h->nlist;
+    CK(cudaMemcpyAsync(h->list_off.p, h->s_u32c.p, (size_t)(nl + 1) * 4, cudaMemcpyDeviceToDevice, st));
+    CK(cudaMemcpyAsync(h->list_off.p + nl + 1, h->s_u32c.p + nl, 4, cudaMemcpyDeviceToDevice, st));
+    CK(cudaStreamSynchronize(st));
+    adopt(h, h->ivf_rows, f.x);
+    adopt(h, h->ivf_ids, f.ids);
+    adopt(h, h->ivf_list, f.lists);
+    h->ivf_n = kept;
+    mark_arena_dirty(h);
+    return FVDB_OK;
+}
+
 // Regroup sealed + pending IVF rows so every list is one contiguous row range.
 int seal(fvdb_index* h) {
     if (h->pend_n == 0) return FVDB_OK;
@@ -456,39 +540,23 @@ int seal(fvdb_index* h) {
     cudaStream_t st = h->stream;
     const uint64_t total = h->ivf_n + h->pend_n;
     if (total >= 0xFFFFFFF0ull) return h->fail(FVDB_ERR_INVALID_ARG, "IVF tier exceeds u32 rows");
-    const uint32_t D = h->dim;
     CK(h->s_keys32.ensure(total, 0, st, &h->dev_bytes));
     if (h->ivf_n)
         CK(cudaMemcpyAsync(h->s_keys32.p, h->ivf_list.p, h->ivf_n * 4, cudaMemcpyDeviceToDevice, st));
     CK(cudaMemcpyAsync(h->s_keys32.p + h->ivf_n, h->pend_list.p, h->pend_n * 4,
                        cudaMemcpyDeviceToDevice, st));
-    CK(h->s_perm.ensure(total, 0, st, &h->dev_bytes));
-    CK(h->s_group.ensure(stable_group_scratch_bytes(total, h->nlist), 0, st, &h->dev_bytes));
-    CK(h->list_off.ensure(h->nlist + 2, 0, st, &h->dev_bytes));
-    CK(launch_stable_group(h->s_keys32.p, total, h->nlist, h->list_off.p, h->s_perm.p, h->s_group.p, st));
     uint32_t kept = 0;
-    CK(cudaMemcpyAsync(&kept, h->list_off.p + h->nlist, 4, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    DevBuf<float> nrows;
-    DevBuf<uint32_t> nids, nlist_ids;
-    CK(nrows.ensure((size_t)std::max<uint64_t>(kept, 1) * D, 0, st, &h->dev_bytes, true));
-    CK(nids.ensure(std::max<uint64_t>(kept, 1), 0, st, &h->dev_bytes, true));
-    CK(nlist_ids.ensure(std::max<uint64_t>(kept, 1), 0, st, &h->dev_bytes, true));
-    CK(launch_gather_rows(h->ivf_rows.p, h->ivf_n, h->pend_rows.p, h->s_perm.p, kept, D, nrows.p, st));
-    CK(launch_gather_u32(h->ivf_ids.p, h->ivf_n, h->pend_ids.p, h->s_perm.p, kept, nids.p, st));
-    CK(launch_gather_u32(h->ivf_list.p, h->ivf_n, h->pend_list.p, h->s_perm.p, kept, nlist_ids.p, st));
-    CK(cudaStreamSynchronize(st));
-    h->dev_bytes -= h->ivf_rows.cap * sizeof(float) + (h->ivf_ids.cap + h->ivf_list.cap) * 4;
-    h->dev_bytes -= h->pend_rows.cap * sizeof(float) + (h->pend_ids.cap + h->pend_list.cap) * 4;
-    h->ivf_rows.swap(nrows);
-    h->ivf_ids.swap(nids);
-    h->ivf_list.swap(nlist_ids);
-    h->pend_rows.release();
-    h->pend_ids.release();
-    h->pend_list.release();
-    h->ivf_n = kept;
+    RET(group_keys(h, h->s_keys32.p, total, h->nlist, h->nlist, 1, &kept, st));
+    NewRows f;
+    RET(alloc_rows(h, f, kept, true, st));
+    CK(h->list_off.ensure(h->nlist + 2, 0, st, &h->dev_bytes));
+    const Rows pend{h->pend_rows.p, h->pend_ids.p, h->pend_list.p};
+    RET(gather(h, arena(h), h->ivf_n, pend, h->s_perm.p, kept, f.x.p, f.ids.p, f.lists.p, st));
+    RET(adopt_arena(h, f, kept, st));
+    release(h, h->pend_rows);
+    release(h, h->pend_ids);
+    release(h, h->pend_list);
     h->pend_n = 0;
-    mark_arena_dirty(h);
     return FVDB_OK;
 }
 
@@ -574,9 +642,16 @@ int assign_device(fvdb_index* h, const float* d_x, uint64_t n, uint32_t* d_assig
     return FVDB_OK;
 }
 
-int ivf_add_device_impl(fvdb_index* h, const float* d_x, const uint32_t* d_ids, uint64_t n,
-                        uint32_t mod, uint32_t rem, uint64_t* kept_out, uint32_t* h_out_list,
-                        const uint32_t* d_owner = nullptr) {
+// The rows an IVF add keeps once they are assigned: all of them (no owner table, mod <= 1), those whose list % mod
+// == rank (a list-sharded load), or, given an owner table over the lists, those of the lists `rank` owns.
+struct KeepRule {
+    uint32_t mod, rank;
+    const uint32_t* owner;
+};
+constexpr KeepRule KEEP_ALL{1, 0, nullptr};
+
+int ivf_add_device_impl(fvdb_index* h, const float* d_x, const uint32_t* d_ids, uint64_t n, KeepRule keep,
+                        uint64_t* kept_out, uint32_t* h_out_list) {
     if (!h->trained) return h->fail(FVDB_ERR_NOT_TRAINED, "Index not trained. Call train() before inserting or searching.");
     if (kept_out) *kept_out = 0;
     if (n == 0) return FVDB_OK;
@@ -586,29 +661,23 @@ int ivf_add_device_impl(fvdb_index* h, const float* d_x, const uint32_t* d_ids, 
     CK(h->s_u32a.ensure(n, 0, st, &h->dev_bytes));
     RET(assign_device(h, d_x, n, h->s_u32a.p, nullptr, nullptr, nullptr, st));
     if (h_out_list) RET(d2h(h, h_out_list, h->s_u32a.p, n * 4));
-    if (mod <= 1) {
+    if (!keep.owner && keep.mod <= 1) {
         RET(append_pending(h, d_x, d_ids, h->s_u32a.p, n));
         if (kept_out) *kept_out = n;
         return FVDB_OK;
     }
-    // list-sharded load: keep only rows whose list % mod == rem, compacted (grouped by list)
+    // list-sharded load: the kept rows are keyed by their list, the others by nlist (dropped)
     CK(h->s_u32b.ensure(n, 0, st, &h->dev_bytes));
-    if (d_owner) CK(launch_filter_keys_owner(h->s_u32a.p, n, d_owner, rem, h->nlist, h->s_u32b.p, st));
-    else CK(launch_filter_keys_mod(h->s_u32a.p, n, mod, rem, h->nlist, h->s_u32b.p, st));
-    CK(h->s_perm.ensure(n, 0, st, &h->dev_bytes));
-    CK(h->s_group.ensure(stable_group_scratch_bytes(n, h->nlist), 0, st, &h->dev_bytes));
-    CK(h->s_u32c.ensure(h->nlist + 2, 0, st, &h->dev_bytes));
-    CK(launch_stable_group(h->s_u32b.p, n, h->nlist, h->s_u32c.p, h->s_perm.p, h->s_group.p, st));
+    if (keep.owner) CK(launch_owner_keys(h->s_u32a.p, n, keep.owner, keep.rank, 0, h->nlist, h->s_u32b.p, st));
+    else CK(launch_filter_keys_mod(h->s_u32a.p, n, keep.mod, keep.rank, h->nlist, h->s_u32b.p, st));
     uint32_t kept = 0;
-    CK(cudaMemcpyAsync(&kept, h->s_u32c.p + h->nlist, 4, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
+    RET(group_keys(h, h->s_u32b.p, n, h->nlist, h->nlist, 1, &kept, st));
     if (kept) {
         CK(h->pend_rows.ensure((h->pend_n + kept) * D, h->pend_n * D, st, &h->dev_bytes));
         CK(h->pend_ids.ensure(h->pend_n + kept, h->pend_n, st, &h->dev_bytes));
         CK(h->pend_list.ensure(h->pend_n + kept, h->pend_n, st, &h->dev_bytes));
-        CK(launch_gather_rows(d_x, n, nullptr, h->s_perm.p, kept, D, h->pend_rows.p + h->pend_n * D, st));
-        CK(launch_gather_u32(d_ids, n, nullptr, h->s_perm.p, kept, h->pend_ids.p + h->pend_n, st));
-        CK(launch_gather_u32(h->s_u32b.p, n, nullptr, h->s_perm.p, kept, h->pend_list.p + h->pend_n, st));
+        RET(gather(h, {d_x, d_ids, h->s_u32b.p}, n, {}, h->s_perm.p, kept, h->pend_rows.p + h->pend_n * D,
+                   h->pend_ids.p + h->pend_n, h->pend_list.p + h->pend_n, st));
         CK(cudaStreamSynchronize(st));
         h->pend_n += kept;
     }
@@ -628,7 +697,7 @@ int flat_add_device_impl(fvdb_index* h, const float* d_x, const uint32_t* d_ids,
     CK(cudaMemcpyAsync(h->flat_ids.p + h->flat_n, d_ids, n * 4, cudaMemcpyDeviceToDevice, st));
     CK(cudaStreamSynchronize(st));
     h->flat_n += n;
-    h->scratch.tc.flat_dirty = true;
+    mark_flat_dirty(h);
     return FVDB_OK;
 }
 
@@ -817,14 +886,14 @@ int train_device_impl(fvdb_index* h, const float* d_data, uint64_t n, uint32_t n
     const bool old_trained = h->trained;
     const int r = train_body(h, d_data, n, nlist, max_iterations, d_init, seed, out);
     if (r != FVDB_OK) {
-        h->dev_bytes -= h->centroids.cap * sizeof(float);
-        h->centroids.swap(old_centroids);   // the failed run's table is freed with old_centroids
+        release(h, h->centroids);   // the failed run's table
+        h->centroids.swap(old_centroids);
         h->nlist = old_nlist;
         h->trained = old_trained;
         mark_centroids_dirty(h); ++h->centroids_version;
         return r;
     }
-    h->dev_bytes -= old_centroids.cap * sizeof(float);
+    release(h, old_centroids);
     h->trained = true;
     clear_lists(h);   // src/ivf/core.rs:273-277
     return FVDB_OK;
@@ -851,10 +920,12 @@ int reassign_arena(fvdb_index* h, DevBuf<float>& rows, DevBuf<uint32_t>& ids, ui
     h->ivf_n = 0;
     h->pend_n = 0;
     mark_arena_dirty(h);
-    int r = ivf_add_device_impl(h, rows.p, ids.p, n, 1, 0, nullptr, nullptr);
+    int r = ivf_add_device_impl(h, rows.p, ids.p, n, KEEP_ALL, nullptr, nullptr);
     if (r == FVDB_OK) r = seal(h);
-    if (r == FVDB_OK) h->dev_bytes -= rows.cap * sizeof(float) + ids.cap * sizeof(uint32_t);   // freed on return
-    if (r != FVDB_OK) {
+    if (r == FVDB_OK) {
+        release(h, rows);
+        release(h, ids);
+    } else {
         h->ivf_rows.swap(rows);
         h->ivf_ids.swap(ids);
         h->ivf_n = n;
@@ -1592,48 +1663,24 @@ int fvdb_ivf_take_unowned_device(fvdb_index* h, const uint32_t* d_owner, uint32_
     RET(seal(h));
     cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
     const uint64_t n = h->ivf_n;
-    const uint32_t D = h->dim, nl = h->nlist, nk = nl + world;
+    const uint32_t nl = h->nlist, nk = nl + world;
     std::fill(counts, counts + world, 0);
     if (n == 0) return FVDB_OK;
     // one stable grouping: the kept rows first, by list (their new list offsets), then each rank's rows
     CK(h->s_keys32.ensure(n, 0, st, &h->dev_bytes));
     CK(launch_owner_keys(h->ivf_list.p, n, d_owner, my_rank, world, nl, h->s_keys32.p, st));
-    CK(h->s_perm.ensure(n, 0, st, &h->dev_bytes));
-    CK(h->s_group.ensure(stable_group_scratch_bytes(n, nk), 0, st, &h->dev_bytes));
-    CK(h->s_u32c.ensure(nk + 2, 0, st, &h->dev_bytes));
-    CK(launch_stable_group(h->s_keys32.p, n, nk, h->s_u32c.p, h->s_perm.p, h->s_group.p, st));
     std::vector<uint32_t> off(world + 1);
-    CK(cudaMemcpyAsync(off.data(), h->s_u32c.p + nl, (world + 1) * 4, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
+    RET(group_keys(h, h->s_keys32.p, n, nk, nl, world + 1, off.data(), st));
     if (off[world] != n) return h->fail(FVDB_ERR_INVALID_ARG, "owner table names a rank >= world");
     for (uint32_t r = 0; r < world; ++r) counts[r] = off[r + 1] - off[r];
     const uint64_t kept = off[0], moved = n - kept;
     if (!d_rows_out || moved == 0) return FVDB_OK;
     if (cap < moved) return h->fail(FVDB_ERR_INVALID_ARG, "fvdb_ivf_take_unowned_device: buffers too small");
-    const uint32_t* perm = h->s_perm.p;
-    CK(launch_gather_rows(h->ivf_rows.p, n, nullptr, perm + kept, moved, D, d_rows_out, st));
-    CK(launch_gather_u32(h->ivf_ids.p, n, nullptr, perm + kept, moved, d_ids_out, st));
-    DevBuf<float> nrows;
-    DevBuf<uint32_t> nids, nlists;
-    CK(nrows.ensure((size_t)std::max<uint64_t>(kept, 1) * D, 0, st, &h->dev_bytes, true));
-    CK(nids.ensure(std::max<uint64_t>(kept, 1), 0, st, &h->dev_bytes, true));
-    CK(nlists.ensure(std::max<uint64_t>(kept, 1), 0, st, &h->dev_bytes, true));
-    CK(launch_gather_rows(h->ivf_rows.p, n, nullptr, perm, kept, D, nrows.p, st));
-    CK(launch_gather_u32(h->ivf_ids.p, n, nullptr, perm, kept, nids.p, st));
-    CK(launch_gather_u32(h->ivf_list.p, n, nullptr, perm, kept, nlists.p, st));
-    CK(cudaStreamSynchronize(st));
-    // groups 0..nlist-1 of the grouping are the kept lists: offsets[0..nlist] are the new list offsets, and
-    // list_off[nlist + 1] is one past the arena, as seal() leaves it
-    CK(cudaMemcpyAsync(h->list_off.p, h->s_u32c.p, (size_t)(nl + 1) * 4, cudaMemcpyDeviceToDevice, st));
-    CK(cudaMemcpyAsync(h->list_off.p + nl + 1, h->s_u32c.p + nl, 4, cudaMemcpyDeviceToDevice, st));
-    CK(cudaStreamSynchronize(st));
-    h->dev_bytes -= h->ivf_rows.cap * sizeof(float) + (h->ivf_ids.cap + h->ivf_list.cap) * 4;
-    h->ivf_rows.swap(nrows);
-    h->ivf_ids.swap(nids);
-    h->ivf_list.swap(nlists);
-    h->ivf_n = kept;
-    mark_arena_dirty(h);
-    return FVDB_OK;
+    RET(gather(h, arena(h), n, {}, h->s_perm.p + kept, moved, d_rows_out, d_ids_out, nullptr, st));
+    NewRows f;
+    RET(alloc_rows(h, f, kept, true, st));
+    RET(gather(h, arena(h), n, {}, h->s_perm.p, kept, f.x.p, f.ids.p, f.lists.p, st));
+    return adopt_arena(h, f, kept, st);
 }
 
 int fvdb_ivf_dump_lists(fvdb_index* h, uint32_t* out_row_ids, uint32_t* out_lists, uint64_t cap, uint64_t* n_out) {
@@ -1679,7 +1726,7 @@ int fvdb_ivf_add(fvdb_index* h, const float* x, const uint32_t* row_ids, uint64_
         CK(h->s_out_ids.ensure(c, 0, h->stream, &h->dev_bytes));
         RET(h2d(h, h->s_x.p, x + off * h->dim, c * h->dim * 4));
         RET(h2d(h, h->s_out_ids.p, row_ids + off, c * 4));
-        int r = ivf_add_device_impl(h, h->s_x.p, h->s_out_ids.p, c, 1, 0, nullptr,
+        int r = ivf_add_device_impl(h, h->s_x.p, h->s_out_ids.p, c, KEEP_ALL, nullptr,
                                     out_list ? out_list + off : nullptr);
         if (r != FVDB_OK) {
             if (h->track_ids) for (uint64_t i = off; i < n; ++i) h->id_state[row_ids[i]] = 0;
@@ -1693,7 +1740,7 @@ int fvdb_ivf_add_device(fvdb_index* h, const float* d_x, const uint32_t* d_row_i
                         uint32_t list_filter_mod, uint32_t list_filter_rem, uint64_t* kept) {
     ENTER(h);
     h->track_ids = false;  // ids never visit the host on this path
-    return ivf_add_device_impl(h, d_x, d_row_ids, n, list_filter_mod, list_filter_rem, kept, nullptr);
+    return ivf_add_device_impl(h, d_x, d_row_ids, n, {list_filter_mod, list_filter_rem, nullptr}, kept, nullptr);
 }
 
 int fvdb_ivf_add_device_owned(fvdb_index* h, const float* d_x, const uint32_t* d_row_ids, uint64_t n,
@@ -1701,7 +1748,7 @@ int fvdb_ivf_add_device_owned(fvdb_index* h, const float* d_x, const uint32_t* d
     ENTER(h);
     if (!d_owner) return h->fail(FVDB_ERR_INVALID_ARG, "owner table is NULL");
     h->track_ids = false;
-    return ivf_add_device_impl(h, d_x, d_row_ids, n, 2, my_rank, kept, nullptr, d_owner);
+    return ivf_add_device_impl(h, d_x, d_row_ids, n, {0, my_rank, d_owner}, kept, nullptr);
 }
 
 int fvdb_assign_device(fvdb_index* h, const float* d_x, uint64_t n, uint32_t* d_out_list, void* stream) {
@@ -1773,60 +1820,35 @@ int fvdb_vacuum(fvdb_index* h, uint64_t* removed) {
     RET(seal(h));
     if (h->deleted_count == 0 || h->tomb_bits == 0) return FVDB_OK;
     cudaStream_t st = h->stream;
-    const uint32_t D = h->dim;
     uint64_t gone = 0;
-    if (h->ivf_n) {
-        const uint64_t n = h->ivf_n;
+    // each tier keeps the rows whose id is not tombstoned, in their order: the IVF arena keyed by list (tombstoned
+    // rows by nlist, dropped), the flat tier as one group (tombstoned rows by 1)
+    if (const uint64_t n = h->ivf_n) {
         CK(h->s_keys32.ensure(n, 0, st, &h->dev_bytes));
         CK(launch_keys_from_bitmap(h->ivf_ids.p, n, h->tomb.p, h->tomb_bits, h->nlist, h->ivf_list.p, 0,
                                    h->s_keys32.p, st));
-        CK(h->s_perm.ensure(n, 0, st, &h->dev_bytes));
-        CK(h->s_group.ensure(stable_group_scratch_bytes(n, h->nlist), 0, st, &h->dev_bytes));
-        CK(launch_stable_group(h->s_keys32.p, n, h->nlist, h->list_off.p, h->s_perm.p, h->s_group.p, st));
         uint32_t kept = 0;
-        CK(cudaMemcpyAsync(&kept, h->list_off.p + h->nlist, 4, cudaMemcpyDeviceToHost, st));
-        CK(cudaStreamSynchronize(st));
-        DevBuf<float> nrows;
-        DevBuf<uint32_t> nids, nl;
-        CK(nrows.ensure((size_t)std::max<uint64_t>(kept, 1) * D, 0, st, &h->dev_bytes, true));
-        CK(nids.ensure(std::max<uint64_t>(kept, 1), 0, st, &h->dev_bytes, true));
-        CK(nl.ensure(std::max<uint64_t>(kept, 1), 0, st, &h->dev_bytes, true));
-        CK(launch_gather_rows(h->ivf_rows.p, n, nullptr, h->s_perm.p, kept, D, nrows.p, st));
-        CK(launch_gather_u32(h->ivf_ids.p, n, nullptr, h->s_perm.p, kept, nids.p, st));
-        CK(launch_gather_u32(h->ivf_list.p, n, nullptr, h->s_perm.p, kept, nl.p, st));
-        CK(cudaStreamSynchronize(st));
-        h->dev_bytes -= h->ivf_rows.cap * 4 + (h->ivf_ids.cap + h->ivf_list.cap) * 4;
-        h->ivf_rows.swap(nrows);
-        h->ivf_ids.swap(nids);
-        h->ivf_list.swap(nl);
+        RET(group_keys(h, h->s_keys32.p, n, h->nlist, h->nlist, 1, &kept, st));
+        NewRows f;
+        RET(alloc_rows(h, f, kept, true, st));
+        RET(gather(h, arena(h), n, {}, h->s_perm.p, kept, f.x.p, f.ids.p, f.lists.p, st));
+        RET(adopt_arena(h, f, kept, st));
         gone += n - kept;
-        h->ivf_n = kept;
-        mark_arena_dirty(h);
     }
-    if (h->flat_n) {
-        const uint64_t n = h->flat_n;
+    if (const uint64_t n = h->flat_n) {
         CK(h->s_keys32.ensure(n, 0, st, &h->dev_bytes));
         CK(launch_keys_from_bitmap(h->flat_ids.p, n, h->tomb.p, h->tomb_bits, 1, nullptr, 0, h->s_keys32.p, st));
-        CK(h->s_perm.ensure(n, 0, st, &h->dev_bytes));
-        CK(h->s_group.ensure(stable_group_scratch_bytes(n, 1), 0, st, &h->dev_bytes));
-        CK(h->s_u32c.ensure(8, 0, st, &h->dev_bytes));
-        CK(launch_stable_group(h->s_keys32.p, n, 1, h->s_u32c.p, h->s_perm.p, h->s_group.p, st));
         uint32_t kept = 0;
-        CK(cudaMemcpyAsync(&kept, h->s_u32c.p + 1, 4, cudaMemcpyDeviceToHost, st));
+        RET(group_keys(h, h->s_keys32.p, n, 1, 1, 1, &kept, st));
+        NewRows f;
+        RET(alloc_rows(h, f, kept, false, st));
+        RET(gather(h, flat_tier(h), n, {}, h->s_perm.p, kept, f.x.p, f.ids.p, nullptr, st));
         CK(cudaStreamSynchronize(st));
-        DevBuf<float> nrows;
-        DevBuf<uint32_t> nids;
-        CK(nrows.ensure((size_t)std::max<uint64_t>(kept, 1) * D, 0, st, &h->dev_bytes, true));
-        CK(nids.ensure(std::max<uint64_t>(kept, 1), 0, st, &h->dev_bytes, true));
-        CK(launch_gather_rows(h->flat_rows.p, n, nullptr, h->s_perm.p, kept, D, nrows.p, st));
-        CK(launch_gather_u32(h->flat_ids.p, n, nullptr, h->s_perm.p, kept, nids.p, st));
-        CK(cudaStreamSynchronize(st));
-        h->dev_bytes -= h->flat_rows.cap * 4 + h->flat_ids.cap * 4;
-        h->flat_rows.swap(nrows);
-        h->flat_ids.swap(nids);
-        gone += n - kept;
+        adopt(h, h->flat_rows, f.x);
+        adopt(h, h->flat_ids, f.ids);
         h->flat_n = kept;
-        h->scratch.tc.flat_dirty = true;
+        mark_flat_dirty(h);
+        gone += n - kept;
     }
     CK(cudaMemsetAsync(h->tomb.p, 0, (h->tomb_bits + 63) / 64 * 8, st));
     CK(cudaStreamSynchronize(st));
@@ -1853,39 +1875,25 @@ int fvdb_move_flat_to_ivf(fvdb_index* h, const uint32_t* row_ids, uint64_t n, ui
     CK(h->s_out_ids.ensure(n, 0, st, &h->dev_bytes));
     RET(h2d(h, h->s_out_ids.p, row_ids, n * 4));
     CK(launch_set_bits(h->s_tmpbits.p, nbits, h->s_out_ids.p, n, 1, st));
+    // the flat tier in two groups, the staying rows then the moving ones, each in flat-tier order
     const uint64_t fn = h->flat_n;
     CK(h->s_keys32.ensure(fn, 0, st, &h->dev_bytes));
     CK(launch_keys_from_bitmap(h->flat_ids.p, fn, h->s_tmpbits.p, nbits, 1, nullptr, 0, h->s_keys32.p, st));
-    CK(h->s_perm.ensure(fn, 0, st, &h->dev_bytes));
-    CK(h->s_group.ensure(stable_group_scratch_bytes(fn, 2), 0, st, &h->dev_bytes));
-    CK(h->s_u32c.ensure(8, 0, st, &h->dev_bytes));
-    CK(launch_stable_group(h->s_keys32.p, fn, 2, h->s_u32c.p, h->s_perm.p, h->s_group.p, st));
-    uint32_t offs[4] = {0, 0, 0, 0};
-    CK(cudaMemcpyAsync(offs, h->s_u32c.p, 16, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    const uint64_t stay = offs[1], mv = offs[2] - offs[1];
+    uint32_t offs[2] = {0, 0};
+    RET(group_keys(h, h->s_keys32.p, fn, 2, 1, 2, offs, st));
+    const uint64_t stay = offs[0], mv = offs[1] - offs[0];
     if (mv == 0) return FVDB_OK;
-    DevBuf<float> nrows;
-    DevBuf<uint32_t> nids;
-    CK(nrows.ensure((size_t)fn * D, 0, st, &h->dev_bytes, true));
-    CK(nids.ensure(fn, 0, st, &h->dev_bytes, true));
-    CK(launch_gather_rows(h->flat_rows.p, fn, nullptr, h->s_perm.p, fn, D, nrows.p, st));
-    CK(launch_gather_u32(h->flat_ids.p, fn, nullptr, h->s_perm.p, fn, nids.p, st));
+    NewRows f;
+    RET(alloc_rows(h, f, fn, false, st));
+    RET(gather(h, flat_tier(h), fn, {}, h->s_perm.p, fn, f.x.p, f.ids.p, nullptr, st));
     CK(cudaStreamSynchronize(st));
     // append the moved rows to the IVF tier FIRST (assignment or allocation may fail); only then does
     // the compacted array replace the flat tier — a failure leaves both tiers as they were
-    {
-        const int r = ivf_add_device_impl(h, nrows.p + stay * D, nids.p + stay, mv, 1, 0, nullptr, nullptr);
-        if (r != FVDB_OK) {
-            h->dev_bytes -= nrows.cap * 4 + nids.cap * 4;
-            return r;
-        }
-    }
-    h->dev_bytes -= h->flat_rows.cap * 4 + h->flat_ids.cap * 4;
-    h->flat_rows.swap(nrows);
-    h->flat_ids.swap(nids);
+    RET(ivf_add_device_impl(h, f.x.p + stay * D, f.ids.p + stay, mv, KEEP_ALL, nullptr, nullptr));
+    adopt(h, h->flat_rows, f.x);
+    adopt(h, h->flat_ids, f.ids);
     h->flat_n = stay;
-    h->scratch.tc.flat_dirty = true;
+    mark_flat_dirty(h);
     if (h->track_ids)
         for (uint64_t i = 0; i < n; ++i)
             if (row_ids[i] < h->id_state.size() && (h->id_state[row_ids[i]] & 3) == 1)

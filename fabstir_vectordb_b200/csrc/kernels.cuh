@@ -99,15 +99,12 @@ cudaError_t launch_set_bits(uint64_t* bits, uint64_t nbits, const uint32_t* ids,
 // keys_out[i] = (keys[i] % mod == rem) ? keys[i] : drop
 cudaError_t launch_filter_keys_mod(const uint32_t* keys, uint64_t n, uint32_t mod, uint32_t rem,
                                    uint32_t drop, uint32_t* keys_out, cudaStream_t stream);
-// keys_out[i] = (owner[keys[i]] == rank) ? keys[i] : drop   (owner: device table over the `drop` lists)
-cudaError_t launch_filter_keys_owner(const uint32_t* keys, uint64_t n, const uint32_t* owner, uint32_t rank,
-                                     uint32_t drop, uint32_t* keys_out, cudaStream_t stream);
 // keys[i] = owner[lists[i]] == rank ? lists[i] : nlist + owner[lists[i]]  (nlist + world when the owner is
 // >= world): launch_stable_group over nlist + world keys then puts the kept rows first, grouped by list, and
-// the rows of every other rank after them, rank by rank
+// the rows of every other rank after them, rank by rank.  With world = 0 those rows all get nlist, the drop group
+// of a grouping over nlist keys: the owned IVF add keeps the rows of its own lists that way.
 cudaError_t launch_owner_keys(const uint32_t* lists, uint64_t n, const uint32_t* owner, uint32_t rank,
                               uint32_t world, uint32_t nlist, uint32_t* keys, cudaStream_t stream);
-cudaError_t launch_iota_u32(uint32_t* p, uint64_t n, uint32_t start, cudaStream_t stream);
 cudaError_t launch_extract_assign(const uint64_t* keys, uint64_t n, uint32_t* assign, float* dist,
                                   const uint32_t* prev_assign, uint32_t* changed, cudaStream_t stream);
 

@@ -180,18 +180,6 @@ __global__ void filter_keys_mod_kernel(const uint32_t* __restrict__ keys, uint64
     }
 }
 
-// list -> GPU placement table (size-balanced list sharding): keep a row when its list's owner is `rank`
-__global__ void filter_keys_owner_kernel(const uint32_t* __restrict__ keys, uint64_t n,
-                                         const uint32_t* __restrict__ owner, uint32_t rank, uint32_t drop,
-                                         uint32_t* __restrict__ out) {
-    uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
-    for (; i < n; i += stride) {
-        const uint32_t k = keys[i];
-        out[i] = (k < drop && __ldg(owner + k) == rank) ? k : drop;
-    }
-}
-
 // re-placement after a sharded retrain: a row of a list this rank owns keeps its list as key (group l), a
 // row of another rank's list gets nlist + that rank; an owner >= world goes to the drop group
 __global__ void owner_keys_kernel(const uint32_t* __restrict__ lists, uint64_t n,
@@ -204,12 +192,6 @@ __global__ void owner_keys_kernel(const uint32_t* __restrict__ lists, uint64_t n
         const uint32_t o = __ldg(owner + l);
         keys[i] = o == rank ? l : (o < world ? nlist + o : nlist + world);
     }
-}
-
-__global__ void iota_kernel(uint32_t* __restrict__ p, uint64_t n, uint32_t start) {
-    uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
-    for (; i < n; i += stride) p[i] = start + (uint32_t)i;
 }
 
 __global__ void extract_assign_kernel(const uint64_t* __restrict__ keys, uint64_t n,
@@ -295,23 +277,10 @@ cudaError_t launch_filter_keys_mod(const uint32_t* keys, uint64_t n, uint32_t mo
     return cudaGetLastError();
 }
 
-cudaError_t launch_filter_keys_owner(const uint32_t* keys, uint64_t n, const uint32_t* owner, uint32_t rank,
-                                     uint32_t drop, uint32_t* keys_out, cudaStream_t stream) {
-    if (n == 0) return cudaSuccess;
-    filter_keys_owner_kernel<<<grid_for(n), 256, 0, stream>>>(keys, n, owner, rank, drop, keys_out);
-    return cudaGetLastError();
-}
-
 cudaError_t launch_owner_keys(const uint32_t* lists, uint64_t n, const uint32_t* owner, uint32_t rank,
                               uint32_t world, uint32_t nlist, uint32_t* keys, cudaStream_t stream) {
     if (n == 0) return cudaSuccess;
     owner_keys_kernel<<<grid_for(n), 256, 0, stream>>>(lists, n, owner, rank, world, nlist, keys);
-    return cudaGetLastError();
-}
-
-cudaError_t launch_iota_u32(uint32_t* p, uint64_t n, uint32_t start, cudaStream_t stream) {
-    if (n == 0) return cudaSuccess;
-    iota_kernel<<<grid_for(n), 256, 0, stream>>>(p, n, start);
     return cudaGetLastError();
 }
 
